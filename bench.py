@@ -59,7 +59,36 @@ def parse():
     ap.add_argument("--view-chunk", type=int, default=8, help="views per decoder pass (capped by the views a rank renders)")
     ap.add_argument("--view-streams", type=int, default=1, help="CUDA streams the view chunks are spread over")
     ap.add_argument("--ref-cuda-worker", default="", help=argparse.SUPPRESS)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the images the last timed step returned to DIR/image.npy (float32 [1, V, R, R, 3]); "
+                         "when they exceed 64 MB, a fixed seeded sample of their pixels to DIR/image_sample.npy instead")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 64_000_000
+DUMP_SEED = 0
+
+
+def dump_images(img: torch.Tensor, out_dir: str) -> str:
+    """Write the images of one job as float32 .npy under out_dir; returns the file written.  Above DUMP_BYTES the
+    file holds the RGB values of a sample of pixels instead: positions drawn without replacement from all views
+    with numpy's default_rng(DUMP_SEED), in increasing flat order, so the same job always yields the same sample."""
+    import numpy as np
+    arr = img.detach().float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    if arr.nbytes + 4096 <= DUMP_BYTES:
+        path = os.path.join(out_dir, "image.npy")
+    else:
+        pixels = arr.reshape(-1, arr.shape[-1])
+        n = (DUMP_BYTES - 4096) // pixels[0].nbytes
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(pixels.shape[0], size=n, replace=False))
+        arr = pixels[idx]
+        path = os.path.join(out_dir, "image_sample.npy")
+    np.save(path, arr)
+    return path
 
 
 def load_peaks():
@@ -382,6 +411,7 @@ def main():
     graphs = not args.no_cuda_graphs
 
     pending = [None]  # image gather of the previous job, still travelling while this job's scene stage runs
+    last = [None]  # rank 0: the images of the newest job of step_device (for --dump-outputs)
 
     def flush():
         """Wait for the outstanding image gather; returns the gathered images on rank 0."""
@@ -389,6 +419,8 @@ def main():
         if pending[0] is not None:
             out = pending[0].wait()
             pending[0] = None
+            if out is not None:
+                last[0] = out[None]
         return out
 
     def step_device(inp, dst=0):
@@ -396,8 +428,9 @@ def main():
         job k is enqueued asynchronously and waited for right after job k+1 has been launched (and before the timed
         region closes), so it overlaps the next scene stage; dst=None returns this rank's own views."""
         if world == 1:
-            return pipe.render(inp["triangles"], inp["texture"], inp["mask"], inp["vn"], inp["c2w"], inp["fov"],
-                               resolution=R, torch_dtype=torch.bfloat16)
+            last[0] = pipe.render(inp["triangles"], inp["texture"], inp["mask"], inp["vn"], inp["c2w"], inp["fov"],
+                                  resolution=R, torch_dtype=torch.bfloat16)
+            return last[0]
         h = render_sharded(pipe, inp["triangles"], inp["texture"], inp["mask"], inp["vn"], inp["c2w"], inp["fov"],
                            resolution=R, dst=dst, torch_dtype=torch.bfloat16, async_gather=dst is not None)
         if dst is None:
@@ -436,6 +469,11 @@ def main():
     launches = (lib.launch_count() + pipe.replayed_launches - launches0)
     clocks = sampler.stop() if sampler else None
     value = V / (ms_step * 1e-3)
+    if args.dump_outputs:  # before the steps below render the job again
+        if rank == 0:
+            print(f"bench: images of the last timed step -> {dump_images(last[0], args.dump_outputs)}", file=sys.stderr)
+        if world > 1:
+            dist.barrier()  # the other ranks wait here rather than spin in the next render's in-graph barrier
 
     # ---- N > 1 correctness, outside the timed region: the gathered images of the sharded job must be
     # bit-identical to rank 0's own single-GPU render of the same views

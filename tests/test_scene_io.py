@@ -8,7 +8,10 @@ import os
 import numpy as np
 import pytest
 
+from oracle.reference_loader import find_reference
 from renderformer_b200 import scene_io as sio
+
+REF = find_reference() or ""  # a source tree of the unmodified reference, when one is at hand (RFB_REFERENCE)
 
 CUBE = """# unit cube, quads
 v -1 -1 -1
@@ -148,8 +151,8 @@ def test_cbox_fixture(golden_dir):
     room = s["triangles"][:-1].reshape(-1, 3)
     assert np.abs(room).max() <= 0.5 + 1e-6  # the box itself spans [-0.5, 0.5]^3
     np.testing.assert_allclose(s["fov"], [37.5])
-    if os.path.exists("/root/reference/examples/cbox.json"):  # regenerate and compare where the source exists
-        again = sio.load_scene("/root/reference/examples/cbox.json")
+    if os.path.exists(os.path.join(REF, "examples", "cbox.json")):  # regenerate and compare where the source exists
+        again = sio.load_scene(os.path.join(REF, "examples", "cbox.json"))
         for k in s:
             np.testing.assert_array_equal(again[k], s[k])
 
@@ -212,13 +215,13 @@ EXAMPLE_TRIANGLES = {  # triangle counts of the reference's example scenes as co
 }
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/examples"), reason="reference examples only exist in the build container")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "examples")), reason="no reference source tree with examples/ (set RFB_REFERENCE)")
 @pytest.mark.parametrize("name", sorted(EXAMPLE_TRIANGLES))
 def test_every_reference_example_scene_converts(name):
     """All 16 scene descriptions the reference ships (examples/*.json: templates, nested transforms, smooth and flat
     shading, random diffuse, multiple materials) go through the numpy-only converter: finite geometry, unit normals,
     textures inside their documented ranges, one look-at camera each."""
-    sc = sio.load_scene(f"/root/reference/examples/{name}.json")
+    sc = sio.load_scene(os.path.join(REF, "examples", f"{name}.json"))
     n = sc["triangles"].shape[0]
     assert n == EXAMPLE_TRIANGLES[name] and n <= 12288
     assert sc["vn"].shape == (n, 3, 3) and sc["tex13"].shape == (n, 13)

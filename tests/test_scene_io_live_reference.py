@@ -15,8 +15,10 @@ import sys
 import numpy as np
 import pytest
 
+from oracle.reference_loader import find_reference
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = find_reference() or ""  # a source tree of the unmodified reference (RFB_REFERENCE), with examples/
 
 WORKER = r"""
 import json, os, sys, types
@@ -58,7 +60,7 @@ np.savez(out_npz, **captured)
 """
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "scene_processor")), reason="the reference only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "scene_processor")), reason="no reference source tree with scene_processor/ (set RFB_REFERENCE)")
 @pytest.mark.parametrize("scene", ["cbox", "room", "crystals"])
 def test_to_h5_half_of_the_converter_equals_the_reference(scene, tmp_path):
     from renderformer_b200 import scene_io as sio
@@ -103,7 +105,7 @@ np.save(sys.argv[2], normalize_to_unit_sphere(mesh).vertices)
 """
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "scene_processor")), reason="the reference only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "scene_processor")), reason="no reference source tree with scene_processor/ (set RFB_REFERENCE)")
 def test_normalisation_equals_the_reference(tmp_path):
     """scene_mesh.py:12-18 run live on the vertices of a shipped OBJ: centre on the vertex mean, scale so that the
     farthest vertex sits at radius 0.5."""
@@ -144,7 +146,7 @@ np.savez(sys.argv[3], **{k: v.numpy() for k, v in item.items() if hasattr(v, "nu
 """
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "scene_processor")), reason="the reference only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "scene_processor")), reason="no reference source tree with scene_processor/ (set RFB_REFERENCE)")
 @pytest.mark.parametrize("pad", [None, 48])
 def test_scene_loading_and_padding_equal_the_reference_dataset(tmp_path, pad):
     """batch_infer.py:17-58 (`TriangleRenderH5Dataset.__getitem__`, incl. `--padding_length`) run live on a scene file

@@ -3,12 +3,9 @@ the 4096 ray tokens of a 512 x 512 view, DPT 128 / [96, 192, 384, 768]) on the c
 (5633 triangles), one view, against the golden frame of the unmodified reference (tests/golden/base_cbox_512.npz,
 oracle == reference to 0.0 when it was made).
 
-This case was written in a session that had NO GPU minutes left: its first run is the driver's round-end run.  The
-V1-Base architecture is parity-green at 256 triangles / 64 x 64 (`base_small` in tests/test_parity_gpu.py); what is
-new here are the full-size shapes of its full-attention decoder.  Therefore (1) it runs in a subprocess, so that
-whatever happens cannot disturb the other GPU tests, (2) it comes last (file name), and (3) it is marked
-xfail(strict=False): a pass shows up as XPASS, a miss as XFAIL with the measured numbers in the report -- either way
-the rest of the suite is unaffected."""
+The V1-Base architecture is also checked at 256 triangles / 64 x 64 (`base_small` in tests/test_parity_gpu.py); this
+case adds the full-size shapes of its full-attention decoder.  It runs in a subprocess, so that whatever happens cannot
+disturb the other GPU tests, and comes last (file name)."""
 import json
 import os
 import subprocess
@@ -47,7 +44,6 @@ print("BASE_JSON " + json.dumps(out))
 """
 
 
-@pytest.mark.xfail(strict=False, reason="first run of V1-Base at full size happens here (written without GPU access)")
 def test_v1_base_cbox_512_against_reference_golden():
     from renderformer_b200.metrics import PSNR_MIN, REL_TOL
     r = subprocess.run([sys.executable, "-c", WORKER % {"root": ROOT}], capture_output=True, text=True, timeout=600, cwd=ROOT)

@@ -1,7 +1,7 @@
 """GPU, boxes with 4 or 8 devices: the sharded render equals the single-GPU render bit for bit at 4 and 8 ranks too
 (tests/test_dist_gpu.py runs the same worker at 2 ranks; `bench.py` re-checks bit-identity at whatever N it runs on --
-measured true at N = 2 and N = 8).  N = 4 was never run on hardware before the round ended, so these cases are
-xfail(strict=False) like the other tests/test_zz_* files; the worker runs under torchrun in its own processes."""
+measured true at N = 2 and N = 8).  This worker has not been run on hardware at 4 or 8 ranks yet, so both cases are
+xfail(strict=False); the worker runs under torchrun in its own processes."""
 import os
 import socket
 import subprocess
@@ -14,7 +14,7 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-@pytest.mark.xfail(strict=False, reason="first run at this rank count happens here (written without GPU access)")
+@pytest.mark.xfail(strict=False, reason="this worker has not yet run on hardware at this rank count")
 @pytest.mark.parametrize("n", [4, 8])
 def test_sharded_render_equals_single_gpu_more_ranks(n):
     if torch.cuda.device_count() < n:

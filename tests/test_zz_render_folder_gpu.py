@@ -3,10 +3,9 @@ through `render_stream` + `frame_io.FrameWriter`, and the EXR / PNG / MP4 files 
 fp32 oracle on the same scene files (the unchanged reference CLI on the same package is covered by
 tests/test_reference_clis_gpu.py; this is the overlapped replacement of its loop).
 
-Written in a session that had NO GPU minutes left, so the first run is the driver's: the tool runs in a
-subprocess, the file sorts last, and the cases are xfail(strict=False) -- XPASS = verified on hardware, XFAIL = the
-report shows why; neither touches the rest of the suite.  The file encoders themselves are verified on CPU
-(tests/test_frame_io.py, against OpenCV and Pillow)."""
+The tool runs in a subprocess and the file sorts last.  The two-rank case has not been run on hardware yet and is
+xfail(strict=False) until it has.  The file encoders themselves are verified on CPU (tests/test_frame_io.py, against
+OpenCV and Pillow)."""
 import os
 import subprocess
 import sys
@@ -23,7 +22,7 @@ from renderformer_b200.synth import init_state_dict, make_scene
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-NOT_YET = pytest.mark.xfail(strict=False, reason="first run on hardware happens here (written without GPU access)")
+NOT_YET = pytest.mark.xfail(strict=False, reason="not yet run on hardware with two GPUs")
 
 
 def _write_scenes(folder, counts, views):
@@ -68,7 +67,6 @@ def _run(cmd, timeout=600):
     return r.stdout
 
 
-@NOT_YET
 @pytest.mark.parametrize("extra", [["--padding_length", "64", "--save_video"], ["--constant_texture"]],
                          ids=["padded-one-graph-video", "constant-texture-eager"])
 def test_render_folder_tool_against_oracle(tmp_path, extra):

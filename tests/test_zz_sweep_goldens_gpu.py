@@ -2,9 +2,8 @@
 frames of the unmodified reference -- V1.1-swin-Large at (512 triangles, 256^2), (2048 triangles, 2 views, 512^2) and
 (4096 triangles, 1024^2).  tests/test_parity_gpu.py already holds (4096, 512^2), (1024, 1024^2) and (8192, 256^2).
 
-Same rendering code path as the verified parity tests; only the tolerances at these sizes have never been observed on
-hardware (the fixtures were generated in a session without GPU minutes).  So the cases run in ONE subprocess (one model
-initialisation), sort last and are xfail(strict=False): their first run, the driver's, cannot stop the verified suite."""
+Same rendering code path as the parity tests, held to the same tolerances.  The cases run in ONE subprocess (one model
+initialisation) and sort last."""
 import json
 import os
 import subprocess
@@ -63,7 +62,6 @@ def _results():
     return _RESULT
 
 
-@pytest.mark.xfail(strict=False, reason="tolerances at these sweep corners are first observed here (fixtures made without GPU access)")
 @pytest.mark.parametrize("name", NAMES)
 def test_sweep_corner_against_reference_golden(name):
     from renderformer_b200.metrics import PSNR_MIN, REL_TOL
