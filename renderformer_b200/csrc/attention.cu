@@ -3,9 +3,10 @@
 //   O = softmax(scale * Q K^T + mask) V        per (batch, head, 128-query tile)
 //
 // The kernels live in attention2.cu (two query tiles per CTA), attention3.cu (one query tile per CTA, Q in
-// TMEM) and attention_swin.cu (block-diagonal shifted-window mode); this file builds the TMA descriptors
-// and picks the kernel.  Operands are bf16 or fp16 (`dtype`), V is consumed transposed ([head_dim, keys],
-// keys contiguous) so every operand is K-major.
+// TMEM) and attention_swin.cu (block-diagonal shifted-window mode); the arithmetic they share is in
+// attention_common.cuh.  This file builds the TMA descriptors and the dense kernels' parameters, picks the
+// kernel and merges key-split partial results.  Operands are bf16 or fp16 (`dtype`), V is consumed
+// transposed ([head_dim, keys], keys contiguous) so every operand is K-major.
 //
 // mode 0: every query tile visits all key tiles; keys are masked by a packed bit mask
 //         (the key-padding mask of layers/attention.py:145-161, True = attend).
@@ -14,23 +15,9 @@
 //         same shifted-window region id (layers/attention.py:238-271,327-358).
 #include <stdlib.h>
 
-#include <atomic>
-
-#include "host_util.h"
-#include "ptx.cuh"
+#include "attention_common.cuh"
 
 namespace rfb {
-
-extern std::atomic<long long> g_launch_count;
-
-int launch_attention_swin(const CUtensorMap& tmQ, const CUtensorMap& tmK, const CUtensorMap& tmV,
-                          const rfb_attn_args* a, int k_batched, int v_batched, cudaStream_t stream);
-int launch_attention3(const CUtensorMap& tmK, const CUtensorMap& tmV, const rfb_attn_args* a, int k_batched,
-                      int v_batched, int split_tiles, int n_splits, float* part_o, float* part_ml,
-                      cudaStream_t stream);
-int launch_attention2(const CUtensorMap& tmQ, const CUtensorMap& tmK, const CUtensorMap& tmV,
-                      const rfb_attn_args* a, int k_batched, int v_batched, int split_tiles, int n_splits,
-                      float* part_o, float* part_ml, cudaStream_t stream);
 
 // Key-split attention, second pass: one warp per (batch, head, query row) merges the chunks' partial results
 // IN CHUNK ORDER (deterministic; a row's result does not depend on the grid that produced the chunks):
@@ -70,6 +57,28 @@ __global__ void __launch_bounds__(256)
   uint2 u;
   u.x = pack16<F16>(acc.x * inv, acc.y * inv), u.y = pack16<F16>(acc.z * inv, acc.w * inv);
   *reinterpret_cast<uint2*>(O + (long long)b * o_batch_stride + (long long)q * ldo + h * 128 + lane * 4) = u;
+}
+
+// Parameters of the dense kernels (mode 0).  With n_splits > 1 the key chunks leave their results in part_o /
+// part_ml (null otherwise).
+static DenseAttnParams dense_attn_params(const rfb_attn_args* a, int k_batched, int v_batched, int n_splits,
+                                         float* part_o, float* part_ml) {
+  DenseAttnParams p{};
+  p.B = a->B, p.split_tiles = n_splits > 1 ? a->kv_split_tiles : 0;
+  p.part_o = part_o, p.part_ml = part_ml;
+  p.Nq = a->Nq, p.Nk = a->Nk;
+  p.n_kv_tiles = (a->Nk + 127) / 128;
+  p.k_batched = k_batched, p.v_batched = v_batched;
+  p.Q = static_cast<const uint16_t*>(a->Q), p.ldq = a->ldq;
+  p.q_batch_stride = a->B > 1 ? a->q_batch_stride : 0;
+  p.mask_bits = a->key_mask_bits;
+  p.mask_stride_words = a->mask_batch_stride_words;
+  p.O = a->O, p.ldo = a->ldo, p.o_batch_stride = a->o_batch_stride;
+  p.scale_log2 = a->scale * 1.4426950408889634f;
+  p.q_sumsq = a->q_sumsq, p.sumsq_ld = a->sumsq_ld > 0 ? a->sumsq_ld : 1;
+  p.sumsq_parts = a->sumsq_parts > 0 ? a->sumsq_parts : 1;
+  p.inv_norm_dim = a->norm_dim > 0 ? 1.0f / (float)a->norm_dim : 0.f, p.norm_eps = a->norm_eps;
+  return p;
 }
 
 }  // namespace rfb
@@ -148,9 +157,8 @@ extern "C" int rfb_attention(const rfb_attn_args* a, rfb_stream_t stream_) {
       const double e3 = (double)n3 / (double)(((n3 + sms - 1) / sms) * sms);
       gen = (e3 > e2 + 0.02) ? 3 : 2;
     }
-    rc = gen == 3 ? launch_attention3(tmK, tmV, a, k_batched, v_batched, a->kv_split_tiles, n_splits, part_o, part_ml, stream)
-                  : launch_attention2(tmQ, tmK, tmV, a, k_batched, v_batched, a->kv_split_tiles, n_splits, part_o, part_ml,
-                                      stream);
+    const DenseAttnParams p = dense_attn_params(a, k_batched, v_batched, n_splits, part_o, part_ml);
+    rc = (gen == 3 ? launch_attention3 : launch_attention2)(tmQ, tmK, tmV, a, p, stream);
     if (rc != RFB_OK || n_splits <= 1) return rc;
     const long long rows = (long long)a->B * a->H * a->Nq;
     const unsigned blocks = (unsigned)((rows + 7) / 8);

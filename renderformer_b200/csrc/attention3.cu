@@ -17,65 +17,28 @@
 // previous P V retired; the (rare) rescale waits on an explicit pv_done barrier first.
 //
 // Used for mode 0 (encoder self-attention, decoder cross-attention, key-padding mask, fused query
-// RMSNorm).  Reference call sites: include/rfb200.h.
-#include <atomic>
-
-#include "host_util.h"
-#include "ptx.cuh"
+// RMSNorm), like attn2_tc_kernel (attention2.cu), which must give bit-identical results: the softmax
+// steps, the epilogues and the key-tile range of a CTA are shared with it in attention_common.cuh;
+// this file holds the Q copy into TMEM, the TMA producer, the MMA issuer and the barrier protocol
+// around the softmax.  Reference call sites: include/rfb200.h.
+#include "attention_common.cuh"
 
 namespace rfb {
 
-extern std::atomic<long long> g_launch_count;
-
-struct Attn3Params {
-  int Nq, Nk, n_kv_tiles;
-  int k_batched, v_batched;
-  const uint16_t* Q;
-  long long ldq, q_batch_stride;
-  const uint32_t* mask_bits;
-  long long mask_stride_words;
-  void* O;
-  long long ldo, o_batch_stride;
-  float scale_log2;
-  const float* q_sumsq;
-  int sumsq_ld, sumsq_parts;
-  float inv_norm_dim, norm_eps;
-  // key splitting, as in attention2.cu (the two kernels leave bit-identical partial results)
-  int B, split_tiles;
-  float* part_o;
-  float* part_ml;
-};
-
-constexpr uint32_t kT3 = 128 * 128 * 2;  // 128 x 128 bf16 tile
-constexpr uint32_t kH3 = 128 * 64 * 2;   // one 64-column swizzle half
 constexpr int kStg3 = 3;
 constexpr int kAttn3Threads = 64 + 128;
-constexpr uint32_t kAttn3Smem = kT3 * 2 * kStg3 + 1024 + 256;
-constexpr int kPoly3 = 4;  // every 4th pair of exponentials on the FMA pipe
-
-__device__ __forceinline__ void exp2_poly2_3(uint64_t t2, float& p0, float& p1) {
-  const float ta = fmaxf(lo2f(t2), -126.0f), tb = fmaxf(hi2f(t2), -126.0f);
-  const uint64_t t = pack2f(ta, tb);
-  const uint64_t r = fadd2(t, pack2f(12582912.0f, 12582912.0f));
-  const uint64_t n = fadd2(r, pack2f(-12582912.0f, -12582912.0f));
-  const uint64_t f = ffma2(n, pack2f(-1.0f, -1.0f), t);
-  uint64_t p = ffma2(f, pack2f(0.0551716685f, 0.0551716685f), pack2f(0.2426111251f, 0.2426111251f));
-  p = ffma2(p, f, pack2f(0.6932609677f, 0.6932609677f));
-  p = ffma2(p, f, pack2f(0.9999280572f, 0.9999280572f));
-  p0 = __uint_as_float(__float_as_uint(lo2f(p)) + (__float_as_uint(lo2f(r)) << 23));
-  p1 = __uint_as_float(__float_as_uint(hi2f(p)) + (__float_as_uint(hi2f(r)) << 23));
-}
+constexpr uint32_t kAttn3Smem = kAttnTile * 2 * kStg3 + 1024 + 256;
 
 template <bool F16>
 __global__ void __launch_bounds__(kAttn3Threads, 1)
     attn3_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_constant__ CUtensorMap tmV,
-                    const Attn3Params p) {
+                    const DenseAttnParams p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_addr = smem_u32(smem_raw);
   uint8_t* smem = smem_raw + ((1024u - (raw_addr & 1023u)) & 1023u);
-  uint8_t* sK = smem;                  // kStg3 tiles
-  uint8_t* sV = sK + kStg3 * kT3;      // kStg3 tiles
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sV + kStg3 * kT3);
+  uint8_t* sK = smem;                       // kStg3 tiles
+  uint8_t* sV = sK + kStg3 * kAttnTile;     // kStg3 tiles
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sV + kStg3 * kAttnTile);
   uint64_t* k_full = bars;              // kStg3
   uint64_t* k_empty = k_full + kStg3;   // kStg3
   uint64_t* v_full = k_empty + kStg3;   // kStg3
@@ -89,10 +52,10 @@ __global__ void __launch_bounds__(kAttn3Threads, 1)
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int h = blockIdx.y;
-  const int split = p.split_tiles > 0 ? blockIdx.z / p.B : 0;
+  const DenseTiles tiles = dense_tiles(p);
+  const int split = tiles.split, j_begin = tiles.j_begin, n_tiles = tiles.n_tiles, tail_local = tiles.tail_local;
   const int b = blockIdx.z - split * p.B;
   const int q0 = blockIdx.x * 128;
-  const int j_begin = split * p.split_tiles;  // first key tile of this CTA
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < kStg3; ++i) {
@@ -114,12 +77,6 @@ __global__ void __launch_bounds__(kAttn3Threads, 1)
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const uint32_t tO = tmem_base + 256, tQ = tmem_base + 384;
-  const int n_tiles = p.split_tiles > 0 ? min(p.split_tiles, p.n_kv_tiles - j_begin) : p.n_kv_tiles;
-  // Short tail: when the LAST key tile of the sequence holds <= 32 keys (16 register tokens + a multiple of 128
-  // triangles is the common case) its products run 32 keys wide -- S = Q K^T with N = 32, P V with two K = 16 steps --
-  // and the softmax touches one 32-column chunk instead of four.  The skipped columns are masked keys, whose
-  // probabilities are exactly 0: the result is bit-identical to the full-width tile.
-  const int tail_local = (p.Nk - (p.n_kv_tiles - 1) * 128 <= 32) ? p.n_kv_tiles - 1 - j_begin : -1;  // local index or never
   const int kb = p.k_batched ? b : 0;
   const int vb = p.v_batched ? b : 0;
 
@@ -129,14 +86,14 @@ __global__ void __launch_bounds__(kAttn3Threads, 1)
         const int s = j % kStg3;
         const uint32_t ph = (j / kStg3) & 1;
         mbar_wait(&k_empty[s], ph ^ 1);
-        mbar_expect_tx(&k_full[s], kT3);
+        mbar_expect_tx(&k_full[s], kAttnTile);
         const int key0 = (j_begin + j) * 128;
-        tma_load_3d(sK + s * kT3, &tmK, &k_full[s], h * 128, key0, kb);
-        tma_load_3d(sK + s * kT3 + kH3, &tmK, &k_full[s], h * 128 + 64, key0, kb);
+        tma_load_3d(sK + s * kAttnTile, &tmK, &k_full[s], h * 128, key0, kb);
+        tma_load_3d(sK + s * kAttnTile + kAttnHalf, &tmK, &k_full[s], h * 128 + 64, key0, kb);
         mbar_wait(&v_empty[s], ph ^ 1);
-        mbar_expect_tx(&v_full[s], kT3);
-        tma_load_3d(sV + s * kT3, &tmV, &v_full[s], key0, h * 128, vb);
-        tma_load_3d(sV + s * kT3 + kH3, &tmV, &v_full[s], key0 + 64, h * 128, vb);
+        mbar_expect_tx(&v_full[s], kAttnTile);
+        tma_load_3d(sV + s * kAttnTile, &tmV, &v_full[s], key0, h * 128, vb);
+        tma_load_3d(sV + s * kAttnTile + kAttnHalf, &tmV, &v_full[s], key0 + 64, h * 128, vb);
       }
     }
   } else if (warp == 1) {
@@ -147,13 +104,10 @@ __global__ void __launch_bounds__(kAttn3Threads, 1)
         const int s = j % kStg3;
         mbar_wait(&k_full[s], (j / kStg3) & 1);
         tc_fence_after();
-        const uint64_t bd = umma_desc_sw128(smem_u32(sK + s * kT3));
+        const uint64_t bd = umma_desc_sw128(smem_u32(sK + s * kAttnTile));
         const uint32_t id = (j == tail_local) ? idesc_tail : idesc;
 #pragma unroll
-        for (int k = 0; k < 8; ++k) {
-          const uint32_t off = (k >> 2) * (kH3 >> 4) + (k & 3) * 2;
-          umma_f16_ts(tmem_base + (j & 1) * 128, tQ + k * 8, bd + off, id, k != 0);
-        }
+        for (int k = 0; k < 8; ++k) umma_f16_ts(tmem_base + (j & 1) * 128, tQ + k * 8, bd + sw128_kstep(k), id, k != 0);
         umma_commit(&k_empty[s]);
         umma_commit(&s_full[j & 1]);
       };
@@ -162,13 +116,11 @@ __global__ void __launch_bounds__(kAttn3Threads, 1)
         mbar_wait(&v_full[s], (j / kStg3) & 1);
         mbar_wait(&p_full[j & 1], (j >> 1) & 1);
         tc_fence_after();
-        const uint64_t bd = umma_desc_sw128(smem_u32(sV + s * kT3));
+        const uint64_t bd = umma_desc_sw128(smem_u32(sV + s * kAttnTile));
         const int ksteps = (j == tail_local) ? 2 : 8;  // short tail: 32 keys = two K = 16 steps
 #pragma unroll
-        for (int k = 0; k < 8; ++k) {
-          const uint32_t off = (k >> 2) * (kH3 >> 4) + (k & 3) * 2;
-          if (k < ksteps) umma_f16_ts(tO, tmem_base + (j & 1) * 128 + k * 8, bd + off, idesc, (j | k) != 0);
-        }
+        for (int k = 0; k < 8; ++k)
+          if (k < ksteps) umma_f16_ts(tO, tmem_base + (j & 1) * 128 + k * 8, bd + sw128_kstep(k), idesc, (j | k) != 0);
         umma_commit(&v_empty[s]);
         umma_commit(pv_done);
       };
@@ -208,106 +160,26 @@ __global__ void __launch_bounds__(kAttn3Threads, 1)
       if (lane == 0) mbar_arrive(q_ready);
     }
 
-    float sl2 = p.scale_log2;
-    if (p.q_sumsq && row_ok) {  // fused q RMSNorm: per-row 1/rms folded into the scale
-      const float* sp = p.q_sumsq + (static_cast<long long>(b) * p.Nq + qrow) * p.sumsq_ld;
-      float ss = 0.f;
-      for (int j = 0; j < p.sumsq_parts; ++j) ss += sp[j];
-      sl2 *= rsqrtf(ss * p.inv_norm_dim + p.norm_eps);
-    }
+    const float sl2 = dense_scale_log2(p, b, qrow);
     float m_run = -INFINITY, l_run = 0.f;
     const uint32_t tOl = tO + lane_addr;
 
     for (int j = 0; j < n_tiles; ++j) {
       uint32_t mw[4];
-      if (p.mask_bits) {
-        const uint4 u = __ldg(reinterpret_cast<const uint4*>(p.mask_bits + static_cast<long long>(b) * p.mask_stride_words + (j_begin + j) * 4));
-        mw[0] = u.x, mw[1] = u.y, mw[2] = u.z, mw[3] = u.w;
-      } else {
-        const int rem = p.Nk - (j_begin + j) * 128;
-#pragma unroll
-        for (int w = 0; w < 4; ++w) {
-          const int lo = w * 32;
-          mw[w] = rem <= lo ? 0u : (rem - lo >= 32 ? 0xffffffffu : ((1u << (rem - lo)) - 1u));
-        }
-      }
-      const bool all_valid = (mw[0] & mw[1] & mw[2] & mw[3]) == 0xffffffffu;
+      key_mask_words(p, b, j_begin + j, mw);
       const uint32_t tS = tmem_base + (j & 1) * 128 + lane_addr;
-
       mbar_wait(&s_full[j & 1], (j >> 1) & 1);
       tc_fence_after();
       const int nc = (j == tail_local) ? 1 : 4;  // 32-column chunks of S that exist (short tail: one)
       uint32_t v[4][32];
-      tmem_ld32(tS, v[0]);
-      if (nc == 4) {
-        tmem_ld32(tS + 32, v[1]);
-        tmem_ld32(tS + 64, v[2]);
-        tmem_ld32(tS + 96, v[3]);
-      }
-      tmem_wait_ld();
-
-      if (!all_valid) {
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          if (c < nc) {
-            const uint32_t bits = mw[c];
-#pragma unroll
-            for (int i = 0; i < 32; ++i)
-              if (!((bits >> i) & 1u)) v[c][i] = 0xff800000u;  // -inf
-          }
-        }
-      }
-      float mx4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-#pragma unroll
-      for (int c = 0; c < 4; ++c)
-        if (c < nc) {
-#pragma unroll
-          for (int i = 0; i < 32; ++i) mx4[i & 3] = fmaxf(mx4[i & 3], __uint_as_float(v[c][i]));
-        }
-      const float mx = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
-      const float m_new = fmaxf(m_run, mx);
-      const float m_use = (m_new == -INFINITY) ? 0.f : m_new;
-      const float alpha = (m_run == -INFINITY) ? 0.f : ex2_f((m_run - m_use) * sl2);
-      const float neg_ms = -m_use * sl2;
-
-      if (j > 0 && __any_sync(0xffffffffu, alpha != 1.0f)) {
+      const SoftmaxMax sm = softmax_max(tS, nc, mw, m_run, sl2, v);
+      if (j > 0 && __any_sync(0xffffffffu, sm.alpha != 1.0f)) {
         mbar_wait(pv_done, (j - 1) & 1);  // P_{j-1} V_{j-1} retired: O is stable
         tc_fence_after();
-#pragma unroll 1
-        for (int c = 0; c < 4; ++c) {
-          uint32_t o[32];
-          tmem_ld32(tOl + c * 32, o);
-          tmem_wait_ld();
-#pragma unroll
-          for (int i = 0; i < 32; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
-          tmem_st32(tOl + c * 32, o);
-        }
+        rescale_o(tOl, sm.alpha);
       }
-
-      // P = exp2(s*sl2 - m*sl2) -> bf16 pairs -> columns [0,64) of S[j&1]
-      const uint64_t sl2_2 = pack2f(sl2, sl2), nms_2 = pack2f(neg_ms, neg_ms);
-      uint64_t rs2[4] = {0ull, 0ull, 0ull, 0ull};
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        if (c >= nc) continue;
-        uint32_t pk[16];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-          const uint64_t t2 = ffma2(pack2f(__uint_as_float(v[c][2 * i]), __uint_as_float(v[c][2 * i + 1])), sl2_2, nms_2);
-          float p0, p1;
-          if (kPoly3 > 0 && (i % (kPoly3 > 0 ? kPoly3 : 1)) == kPoly3 - 1) {
-            exp2_poly2_3(t2, p0, p1);
-          } else {
-            p0 = ex2_f(lo2f(t2)), p1 = ex2_f(hi2f(t2));
-          }
-          rs2[i & 3] = fadd2(rs2[i & 3], pack2f(p0, p1));
-          pk[i] = pack16<F16>(p0, p1);
-        }
-        tmem_st16(tS + c * 16, pk);
-      }
-      const uint64_t rsum = fadd2(fadd2(rs2[0], rs2[1]), fadd2(rs2[2], rs2[3]));
-      l_run = l_run * alpha + (lo2f(rsum) + hi2f(rsum));
-      m_run = m_new;
+      l_run = fmaf(l_run, sm.alpha, softmax_exp<F16>(v, tS, nc, sl2, sm.neg_ms));
+      m_run = sm.m_new;
 
       tmem_wait_st();
       tc_fence_before();
@@ -322,49 +194,9 @@ __global__ void __launch_bounds__(kAttn3Threads, 1)
       if (lane == 0) mbar_arrive(&p_full[j & 1]);
     }
 
-    // epilogue: O / l -> bf16 -> global
     mbar_wait(pv_done, (n_tiles - 1) & 1);
     tc_fence_after();
-    if (p.part_o) {  // key split: un-normalised O (relative to m_run), (m_run in log2 units, l_run)
-      const long long prow = ((static_cast<long long>(split) * p.B + b) * gridDim.y + h) * p.Nq + qrow;
-      if (row_ok) {
-        float2* ml = reinterpret_cast<float2*>(p.part_ml) + prow;
-        *ml = make_float2(m_run * sl2, l_run);
-      }
-      float* po = p.part_o + prow * 128;
-#pragma unroll 1
-      for (int c = 0; c < 4; ++c) {
-        uint32_t o[32];
-        tmem_ld32(tOl + c * 32, o);
-        tmem_wait_ld();
-        if (row_ok) {
-#pragma unroll
-          for (int i = 0; i < 8; ++i)
-            *reinterpret_cast<uint4*>(po + c * 32 + i * 4) = make_uint4(o[i * 4], o[i * 4 + 1], o[i * 4 + 2], o[i * 4 + 3]);
-        }
-      }
-    } else {
-    const float inv_l = (l_run > 0.f) ? 1.0f / l_run : 0.f;
-    uint16_t* orow = static_cast<uint16_t*>(p.O) + static_cast<long long>(b) * p.o_batch_stride +
-                     static_cast<long long>(qrow) * p.ldo + h * 128;
-#pragma unroll 1
-    for (int c = 0; c < 4; ++c) {
-      uint32_t o[32];
-      tmem_ld32(tOl + c * 32, o);
-      tmem_wait_ld();
-      if (row_ok) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          uint4 u;
-          u.x = pack16<F16>(__uint_as_float(o[i * 8 + 0]) * inv_l, __uint_as_float(o[i * 8 + 1]) * inv_l);
-          u.y = pack16<F16>(__uint_as_float(o[i * 8 + 2]) * inv_l, __uint_as_float(o[i * 8 + 3]) * inv_l);
-          u.z = pack16<F16>(__uint_as_float(o[i * 8 + 4]) * inv_l, __uint_as_float(o[i * 8 + 5]) * inv_l);
-          u.w = pack16<F16>(__uint_as_float(o[i * 8 + 6]) * inv_l, __uint_as_float(o[i * 8 + 7]) * inv_l);
-          *reinterpret_cast<uint4*>(orow + c * 32 + i * 8) = u;
-        }
-      }
-    }
-    }
+    dense_store_row<F16>(p, tOl, split, b, h, qrow, m_run, l_run, sl2);
   }
 
   tc_fence_before();
@@ -375,39 +207,14 @@ __global__ void __launch_bounds__(kAttn3Threads, 1)
   }
 }
 
-// called by rfb_attention (attention.cu) for mode 0
-int launch_attention3(const CUtensorMap& tmK, const CUtensorMap& tmV, const rfb_attn_args* a, int k_batched,
-                      int v_batched, int split_tiles, int n_splits, float* part_o, float* part_ml,
-                      cudaStream_t stream) {
+int launch_attention3(const CUtensorMap&, const CUtensorMap& tmK, const CUtensorMap& tmV, const rfb_attn_args* a,
+                      const DenseAttnParams& p, cudaStream_t stream) {
   if (a->ldq % 8 || (reinterpret_cast<uintptr_t>(a->Q) & 15) || (a->B > 1 && a->q_batch_stride % 8)) return RFB_ERR_ALIGN;
-  Attn3Params p{};
-  p.B = a->B, p.split_tiles = n_splits > 1 ? split_tiles : 0;
-  p.part_o = n_splits > 1 ? part_o : nullptr, p.part_ml = n_splits > 1 ? part_ml : nullptr;
-  p.Nq = a->Nq, p.Nk = a->Nk;
-  p.n_kv_tiles = (a->Nk + 127) / 128;
-  p.k_batched = k_batched, p.v_batched = v_batched;
-  p.Q = static_cast<const uint16_t*>(a->Q), p.ldq = a->ldq;
-  p.q_batch_stride = a->B > 1 ? a->q_batch_stride : 0;
-  p.mask_bits = a->key_mask_bits;
-  p.mask_stride_words = a->mask_batch_stride_words;
-  p.O = a->O, p.ldo = a->ldo, p.o_batch_stride = a->o_batch_stride;
-  p.scale_log2 = a->scale * 1.4426950408889634f;
-  p.q_sumsq = a->q_sumsq, p.sumsq_ld = a->sumsq_ld > 0 ? a->sumsq_ld : 1;
-  p.sumsq_parts = a->sumsq_parts > 0 ? a->sumsq_parts : 1;
-  p.inv_norm_dim = a->norm_dim > 0 ? 1.0f / (float)a->norm_dim : 0.f, p.norm_eps = a->norm_eps;
   const bool f16 = a->dtype == RFB_F16;
-  auto kern = f16 ? attn3_tc_kernel<true> : attn3_tc_kernel<false>;
   static PerDeviceFlag attr_flags[2];
-  bool& attr_set = attr_flags[f16].get();
-  if (!attr_set) {
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kAttn3Smem) != cudaSuccess)
-      return RFB_ERR_LAUNCH;
-    attr_set = true;
-  }
-  dim3 grid((a->Nq + 127) / 128, a->H, a->B * (n_splits > 1 ? n_splits : 1));
-  kern<<<grid, kAttn3Threads, kAttn3Smem, stream>>>(tmK, tmV, p);
-  g_launch_count++;
-  return check_launch("attn3_tc_kernel");
+  const dim3 grid((a->Nq + 127) / 128, a->H, a->B * p.n_splits());
+  return launch_attn_kernel(f16 ? attn3_tc_kernel<true> : attn3_tc_kernel<false>, "attn3_tc_kernel",
+                            attr_flags[f16].get(), kAttn3Smem, grid, kAttn3Threads, stream, tmK, tmV, p);
 }
 
 }  // namespace rfb

@@ -16,14 +16,9 @@
 //
 // Replaces the per-window SDPA of SwinSelfAttention.forward, layers/attention.py:349-358, incl.
 // window_partition / get_swin_attn_mask (:205-271).
-#include <atomic>
-
-#include "host_util.h"
-#include "ptx.cuh"
+#include "attention_common.cuh"
 
 namespace rfb {
-
-extern std::atomic<long long> g_launch_count;
 
 struct SwinParams {
   int N, H;
@@ -39,19 +34,9 @@ struct SwinParams {
   float inv_norm_dim, norm_eps;
 };
 
-constexpr uint32_t kSwTile = 128 * 128 * 2;  // one 128 x 128 bf16 operand tile (two SW128 halves)
-constexpr uint32_t kSwHalf = 128 * 64 * 2;
-constexpr uint32_t kSwStage = 3 * kSwTile;   // Q, K, V^T of one head
+constexpr uint32_t kSwStage = 3 * kAttnTile;  // Q, K, V^T of one head
 constexpr int kSwThreads = 64 + 128;
 constexpr uint32_t kSwSmem = 2 * kSwStage + 1024 + 1024;
-
-__device__ __forceinline__ float sw_rms_factor(const float* sumsq, long long row, int ld, int parts, float inv_dim,
-                                               float eps) {
-  const float* sp = sumsq + row * ld;
-  float ss = 0.f;
-  for (int j = 0; j < parts; ++j) ss += sp[j];
-  return rsqrtf(ss * inv_dim + eps);
-}
 
 template <bool F16>
 __global__ void __launch_bounds__(kSwThreads, 1)
@@ -93,8 +78,8 @@ __global__ void __launch_bounds__(kSwThreads, 1)
     s_gid[i] = p.group_id[(q0 + i) % p.group_period];
     float rk = 1.0f;
     if (p.k_sumsq && q0 + i < p.N)
-      rk = sw_rms_factor(p.k_sumsq, static_cast<long long>(b) * p.N + q0 + i, p.sumsq_ld, p.sumsq_parts,
-                         p.inv_norm_dim, p.norm_eps);
+      rk = rms_factor(p.k_sumsq, static_cast<long long>(b) * p.N + q0 + i, p.sumsq_ld, p.sumsq_parts, p.inv_norm_dim,
+                      p.norm_eps);
     s_rk[i] = rk;
   }
   tc_fence_before();
@@ -112,11 +97,11 @@ __global__ void __launch_bounds__(kSwThreads, 1)
         mbar_wait(&empty[s], ((h >> 1) & 1) ^ 1);
         mbar_expect_tx(&full[s], kSwStage);
         tma_load_3d(st, &tmQ, &full[s], h * 128, q0, b);
-        tma_load_3d(st + kSwHalf, &tmQ, &full[s], h * 128 + 64, q0, b);
-        tma_load_3d(st + kSwTile, &tmK, &full[s], h * 128, q0, kb);
-        tma_load_3d(st + kSwTile + kSwHalf, &tmK, &full[s], h * 128 + 64, q0, kb);
-        tma_load_3d(st + 2 * kSwTile, &tmV, &full[s], q0, h * 128, vb);
-        tma_load_3d(st + 2 * kSwTile + kSwHalf, &tmV, &full[s], q0 + 64, h * 128, vb);
+        tma_load_3d(st + kAttnHalf, &tmQ, &full[s], h * 128 + 64, q0, b);
+        tma_load_3d(st + kAttnTile, &tmK, &full[s], h * 128, q0, kb);
+        tma_load_3d(st + kAttnTile + kAttnHalf, &tmK, &full[s], h * 128 + 64, q0, kb);
+        tma_load_3d(st + 2 * kAttnTile, &tmV, &full[s], q0, h * 128, vb);
+        tma_load_3d(st + 2 * kAttnTile + kAttnHalf, &tmV, &full[s], q0 + 64, h * 128, vb);
       }
     }
   } else if (warp == 1) {
@@ -127,12 +112,9 @@ __global__ void __launch_bounds__(kSwThreads, 1)
         mbar_wait(&full[s], (h >> 1) & 1);
         tc_fence_after();
         const uint64_t ad = umma_desc_sw128(smem_u32(smem + s * kSwStage));
-        const uint64_t bd = umma_desc_sw128(smem_u32(smem + s * kSwStage + kSwTile));
+        const uint64_t bd = umma_desc_sw128(smem_u32(smem + s * kSwStage + kAttnTile));
 #pragma unroll
-        for (int k = 0; k < 8; ++k) {
-          const uint32_t off = (k >> 2) * (kSwHalf >> 4) + (k & 3) * 2;
-          umma_f16(tmem_base + s * 128, ad + off, bd + off, idesc, k != 0);
-        }
+        for (int k = 0; k < 8; ++k) umma_f16(tmem_base + s * 128, ad + sw128_kstep(k), bd + sw128_kstep(k), idesc, k != 0);
         umma_commit(&s_full[s]);
       };
       auto issue_pv = [&](int h) {  // O[h&1] = P_h V_h  (A operand: packed bf16 P in S[h&1] columns [0,64))
@@ -140,12 +122,10 @@ __global__ void __launch_bounds__(kSwThreads, 1)
         mbar_wait(&p_full[s], (h >> 1) & 1);
         mbar_wait(&o_empty[s], ((h >> 1) & 1) ^ 1);
         tc_fence_after();
-        const uint64_t bd = umma_desc_sw128(smem_u32(smem + s * kSwStage + 2 * kSwTile));
+        const uint64_t bd = umma_desc_sw128(smem_u32(smem + s * kSwStage + 2 * kAttnTile));
 #pragma unroll
-        for (int k = 0; k < 8; ++k) {
-          const uint32_t off = (k >> 2) * (kSwHalf >> 4) + (k & 3) * 2;
-          umma_f16_ts(tmem_base + 256 + s * 128, tmem_base + s * 128 + k * 8, bd + off, idesc, k != 0);
-        }
+        for (int k = 0; k < 8; ++k)
+          umma_f16_ts(tmem_base + 256 + s * 128, tmem_base + s * 128 + k * 8, bd + sw128_kstep(k), idesc, k != 0);
         umma_commit(&o_full[s]);
         umma_commit(&empty[s]);
       };
@@ -164,8 +144,8 @@ __global__ void __launch_bounds__(kSwThreads, 1)
     const bool row_ok = q0 + r < p.N;
     float sl2 = p.scale_log2;
     if (p.q_sumsq && row_ok)
-      sl2 *= sw_rms_factor(p.q_sumsq, static_cast<long long>(b) * p.N + q0 + r, p.sumsq_ld, p.sumsq_parts,
-                           p.inv_norm_dim, p.norm_eps);
+      sl2 *= rms_factor(p.q_sumsq, static_cast<long long>(b) * p.N + q0 + r, p.sumsq_ld, p.sumsq_parts, p.inv_norm_dim,
+                        p.norm_eps);
     // keys of the own window this row may attend: same region id, inside the sequence
     uint32_t mw[2];
     {
@@ -195,24 +175,7 @@ __global__ void __launch_bounds__(kSwThreads, 1)
       const int s = g & 1;
       mbar_wait(&o_full[s], (g >> 1) & 1);
       tc_fence_after();
-      uint16_t* orow = obase + g * 128;
-#pragma unroll 1
-      for (int c = 0; c < 4; ++c) {
-        uint32_t o[32];
-        tmem_ld32(tmem_base + 256 + s * 128 + lane_addr + c * 32, o);
-        tmem_wait_ld();
-        if (row_ok) {
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            uint4 u;
-            u.x = pack16<F16>(__uint_as_float(o[i * 8 + 0]) * inv_l, __uint_as_float(o[i * 8 + 1]) * inv_l);
-            u.y = pack16<F16>(__uint_as_float(o[i * 8 + 2]) * inv_l, __uint_as_float(o[i * 8 + 3]) * inv_l);
-            u.z = pack16<F16>(__uint_as_float(o[i * 8 + 4]) * inv_l, __uint_as_float(o[i * 8 + 5]) * inv_l);
-            u.w = pack16<F16>(__uint_as_float(o[i * 8 + 6]) * inv_l, __uint_as_float(o[i * 8 + 7]) * inv_l);
-            *reinterpret_cast<uint4*>(orow + c * 32 + i * 8) = u;
-          }
-        }
-      }
+      store_o_row<F16>(tmem_base + 256 + s * 128 + lane_addr, obase + g * 128, row_ok, inv_l);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&o_empty[s]);
@@ -300,18 +263,10 @@ int launch_attention_swin(const CUtensorMap& tmQ, const CUtensorMap& tmK, const 
   p.sumsq_ld = a->sumsq_ld > 0 ? a->sumsq_ld : 1, p.sumsq_parts = a->sumsq_parts > 0 ? a->sumsq_parts : 1;
   p.inv_norm_dim = a->norm_dim > 0 ? 1.0f / (float)a->norm_dim : 0.f, p.norm_eps = a->norm_eps;
   const bool f16 = a->dtype == RFB_F16;
-  auto kern = f16 ? attn_swin_kernel<true> : attn_swin_kernel<false>;
   static PerDeviceFlag attr_flags[2];
-  bool& attr_set = attr_flags[f16].get();
-  if (!attr_set) {
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSwSmem) != cudaSuccess)
-      return RFB_ERR_LAUNCH;
-    attr_set = true;
-  }
-  dim3 grid((a->Nq + 127) / 128, a->B);
-  kern<<<grid, kSwThreads, kSwSmem, stream>>>(tmQ, tmK, tmV, p);
-  g_launch_count++;
-  return check_launch("attn_swin_kernel");
+  const dim3 grid((a->Nq + 127) / 128, a->B);
+  return launch_attn_kernel(f16 ? attn_swin_kernel<true> : attn_swin_kernel<false>, "attn_swin_kernel",
+                            attr_flags[f16].get(), kSwSmem, grid, kSwThreads, stream, tmQ, tmK, tmV, p);
 }
 
 }  // namespace rfb

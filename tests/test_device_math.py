@@ -2,7 +2,7 @@
 (fused multiply-adds evaluated in float64 and rounded once, as the hardware does), checked against libm:
 
 * the degree-3 exp2 polynomial the attention softmax runs on the FMA pipe for a quarter of the exponentials
-  (attention2.cu `exp2_poly2`, attention3.cu `exp2_poly2_3`) -- claimed relative error 7.5e-5, far below the
+  (attention_common.cuh `exp2_poly2`) -- claimed relative error 7.5e-5, far below the
   resolution of the 16-bit P operand (bf16: 3.9e-3, fp16: 4.9e-4);
 * the two-constant Cody-Waite reduction in front of `__sincosf` for the RoPE angles (rowops.cu `fast_sincos`);
 * the LDR quantisation rule of `rfb_ldr_quantize` mode 0 (dpt.cu) against the reference CLIs' numpy expression.
@@ -52,27 +52,27 @@ def _exp2_poly(t, magic, coef, clamp):
 
 
 def test_softmax_exp2_polynomial_accuracy():
-    for name, fn in (("attention2.cu", "void exp2_poly2("), ("attention3.cu", "void exp2_poly2_3(")):
-        magic, coef, clamp = _poly_constants(_src(name), fn)
-        assert magic == f32(12582912.0) and len(coef) == 4 and clamp == f32(-126.0), name
-        t = np.concatenate([np.linspace(-126.0, 0.0, 2_000_001), -np.arange(0.0, 127.0), [-0.5, -1.5, -125.5]]).astype(f32)
-        got = _exp2_poly(t, magic, coef, clamp).astype(np.float64)
-        want = np.exp2(t.astype(np.float64))
-        rel = np.abs(got - want) / want
-        # below 2^-125 the polynomial's value (< 1) times 2^n leaves the normal range: the exponent-field trick then
-        # yields a denormal-coded number of the right magnitude only (1e-38: a probability that is zero in any sum)
-        normal = t >= f32(-125.0)
-        assert rel[normal].max() <= 1.0e-4, (name, rel[normal].max())   # claimed 7.5e-5 (+ fp32 rounding)
-        assert rel[normal].max() < 0.25 * 2.0 ** -11                      # well under half an ulp of fp16, 16x under bf16's
-        assert (got[~normal] >= 0).all() and (got[~normal] <= 2.0 ** -125).all()
-        assert (got <= 1.0 + 1e-4).all() and (got > 0).all()   # probabilities stay in (0, 1]
-        # inputs below the clamp (masked keys arrive as -inf) give the smallest normal, never NaN / negative
-        low = _exp2_poly(np.array([-1e4, -np.inf], dtype=f32), magic, coef, clamp)
-        assert np.isfinite(low).all() and (low >= 0).all() and (low <= 1.2e-38).all()
-        # monotone on a fine grid around every integer boundary (the n / f split must not tear the curve)
-        edge = (np.arange(-125, 0)[:, None] + np.linspace(-0.5, 0.5, 2001)[None, :]).astype(f32).reshape(-1)
-        y = _exp2_poly(np.sort(edge), magic, coef, clamp)
-        assert (np.diff(y.astype(np.float64)) >= -1e-4 * y[1:]).all()
+    name = "attention_common.cuh"
+    magic, coef, clamp = _poly_constants(_src(name), "void exp2_poly2(")
+    assert magic == f32(12582912.0) and len(coef) == 4 and clamp == f32(-126.0), name
+    t = np.concatenate([np.linspace(-126.0, 0.0, 2_000_001), -np.arange(0.0, 127.0), [-0.5, -1.5, -125.5]]).astype(f32)
+    got = _exp2_poly(t, magic, coef, clamp).astype(np.float64)
+    want = np.exp2(t.astype(np.float64))
+    rel = np.abs(got - want) / want
+    # below 2^-125 the polynomial's value (< 1) times 2^n leaves the normal range: the exponent-field trick then
+    # yields a denormal-coded number of the right magnitude only (1e-38: a probability that is zero in any sum)
+    normal = t >= f32(-125.0)
+    assert rel[normal].max() <= 1.0e-4, (name, rel[normal].max())   # claimed 7.5e-5 (+ fp32 rounding)
+    assert rel[normal].max() < 0.25 * 2.0 ** -11                      # well under half an ulp of fp16, 16x under bf16's
+    assert (got[~normal] >= 0).all() and (got[~normal] <= 2.0 ** -125).all()
+    assert (got <= 1.0 + 1e-4).all() and (got > 0).all()   # probabilities stay in (0, 1]
+    # inputs below the clamp (masked keys arrive as -inf) give the smallest normal, never NaN / negative
+    low = _exp2_poly(np.array([-1e4, -np.inf], dtype=f32), magic, coef, clamp)
+    assert np.isfinite(low).all() and (low >= 0).all() and (low <= 1.2e-38).all()
+    # monotone on a fine grid around every integer boundary (the n / f split must not tear the curve)
+    edge = (np.arange(-125, 0)[:, None] + np.linspace(-0.5, 0.5, 2001)[None, :]).astype(f32).reshape(-1)
+    y = _exp2_poly(np.sort(edge), magic, coef, clamp)
+    assert (np.diff(y.astype(np.float64)) >= -1e-4 * y[1:]).all()
 
 
 def test_rope_angle_reduction_constants():

@@ -37,6 +37,23 @@ def test_kernel_selftests(binary, env):
     assert "[FAIL]" not in r.stdout
 
 
+@pytest.mark.parametrize("f16", ["0", "1"])
+def test_dense_attention_kernels_bit_identical(f16):
+    """attn2_tc_kernel and attn3_tc_kernel produce the same output bytes for every selftest_attn case: the
+    kernel is picked from the grid shape, so a sharded render may run a row on the other kernel than a
+    single-GPU render of the same job."""
+    exe = os.path.join(ROOT, "renderformer_b200", "selftest_attn")
+    assert os.path.exists(exe), f"{exe} missing: run __graft_entry__.build()"
+    hashes = {}
+    for gen in ("2", "3"):
+        r = subprocess.run([exe, "check"], capture_output=True, text=True, timeout=600,
+                           env={**os.environ, "RFB_TEST_F16": f16, "RFB_ATTN_GEN": gen})
+        assert r.returncode == 0, "\n".join(r.stdout.splitlines()[-15:]) + r.stderr[-2000:]
+        hashes[gen] = [line for line in r.stdout.splitlines() if line.startswith("[HASH] ")]
+    assert hashes["2"], "selftest_attn printed no [HASH] lines"
+    assert hashes["2"] == hashes["3"]
+
+
 def _pipe(cfg, seed):
     from renderformer_b200.model import RenderFormer, RenderFormerRenderingPipeline
     model = RenderFormer(cfg)
