@@ -234,16 +234,25 @@ int rfb_texture_const_prep(const float* tex, void* out, long long n_tris, int ch
 /* NeRF encoding of vertex normals [n,9] -> f16 [n, ld] (encodings/nerf_encoding.py:63-84). */
 int rfb_vn_encode(const float* vn, void* out, int n, int nfreq, int ld, rfb_stream_t stream);
 
-/* camera-space ray bundles -> patch tokens f16 [V, (R/8)^2, 192] (utils/ray_generator.py:13-50,
- * models/view_transformer.py:104-107); fov in degrees. */
+/* Ray kernels of an H x W image (height, width multiples of 8 where patch tokens are produced).  Camera: pinhole,
+ * square pixels, principal point at the image centre, pixel centres at +0.5, fov spanning the LONGER side:
+ * f = max(H, W) / 2 / tan(fov / 2), d = ((px + 0.5 - W/2) / f, -(py + 0.5 - H/2) / f, -1).  Patch tokens are
+ * f16 [V, (H/8)*(W/8), 192] in row-major patch-grid order (token = h1 * (W/8) + w1, feature = c*64 + p1*8 + p2,
+ * models/view_transformer.py:104-107).  The `resolution` forms are the square case H = W = resolution. */
+
+/* camera-space ray bundles -> patch tokens (utils/ray_generator.py:13-50 with identity c2w); fov in degrees. */
+int rfb_ray_tokens_hw(const float* fov_deg, void* out, int n_views, int height, int width, rfb_stream_t stream);
 int rfb_ray_tokens(const float* fov_deg, void* out, int n_views, int resolution, rfb_stream_t stream);
 
 /* RayGenerator.forward (utils/ray_generator.py:13-50) for callers that want the ray map itself: c2w [V,4,4],
- * fov in RADIANS [V] -> rays_d fp32 [V, R, R, 3] (rotated by R(c2w), L2-normalised). */
+ * fov in RADIANS [V] -> rays_d fp32 [V, H, W, 3] (rotated by R(c2w), L2-normalised). */
+int rfb_ray_map_hw(const float* c2w, const float* fov_rad, float* rays_d, int n_views, int height, int width,
+                   rfb_stream_t stream);
 int rfb_ray_map(const float* c2w, const float* fov_rad, float* rays_d, int n_views, int resolution, rfb_stream_t stream);
 
-/* explicit ray map fp32 [V, R, R, 3] -> patch tokens f16 [V, (R/8)^2, 192] (models/view_transformer.py:104-107):
- * the model-level entry RenderFormer.forward(..., rays_d, tri_vpos_view_tf) hands rays in instead of cameras. */
+/* explicit ray map fp32 [V, H, W, 3] -> patch tokens (models/view_transformer.py:104-107): the model-level entry
+ * RenderFormer.forward(..., rays_d, tri_vpos_view_tf) hands rays in instead of cameras. */
+int rfb_ray_map_tokens_hw(const float* rays_d, void* out, int n_views, int height, int width, rfb_stream_t stream);
 int rfb_ray_map_tokens(const float* rays_d, void* out, int n_views, int resolution, rfb_stream_t stream);
 
 /* RoPE positions [V, rows_out, 9]: register rows = masked centroid, then T_v^-1 * triangle

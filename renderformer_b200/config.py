@@ -7,9 +7,10 @@ Field names and defaults mirror the reference's flat config.json contract
 from __future__ import annotations
 
 import json
+import numbers
 import os
 from dataclasses import asdict, dataclass, field, fields
-from typing import List, Optional
+from typing import List, Optional, Tuple
 
 _CONFIG_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "configs")
 
@@ -139,3 +140,25 @@ class RenderFormerConfig:
             bad.append("dpt_out_channels must be multiples of 32")
         if bad:
             raise NotImplementedError("unsupported RenderFormerConfig options: " + ", ".join(bad))
+
+
+def view_grid(cfg: RenderFormerConfig, resolution) -> Tuple[int, int]:
+    """(height, width) in pixels of the images `resolution` asks for: an int is a square image, a pair is
+    (height, width).  Sides must be multiples of 64 for the swin decoder (8x8 windows of 8x8-pixel patches, the
+    reference's own constraint, SURVEY §8b) and multiples of the 8-pixel patch for full attention.  Raises
+    ValueError before anything is launched."""
+    if isinstance(resolution, (tuple, list)):
+        if len(resolution) != 2:
+            raise ValueError(f"resolution must be an int or a (height, width) pair, got {resolution!r}")
+        hw = tuple(resolution)
+    else:
+        hw = (resolution, resolution)
+    if not all(isinstance(s, numbers.Integral) and not isinstance(s, bool) and s > 0 for s in hw):
+        raise ValueError(f"resolution must be a positive int or a (height, width) pair of positive ints, got {resolution!r}")
+    H, W = int(hw[0]), int(hw[1])
+    if cfg.view_transformer_use_swin_attn and (H % 64 or W % 64):
+        raise ValueError(f"image height and width must be multiples of 64 for swin attention, got {H}x{W}")
+    if H % cfg.patch_size or W % cfg.patch_size:
+        raise ValueError(f"image height and width must be multiples of the {cfg.patch_size}-pixel patch size, "
+                         f"got {H}x{W}")
+    return H, W

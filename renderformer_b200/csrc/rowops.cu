@@ -462,58 +462,66 @@ __global__ void vn_encode_kernel(const float* __restrict__ vn, uint16_t* __restr
   out[t] = *reinterpret_cast<uint16_t*>(&h);
 }
 
+// Pinhole camera of an H x W image: square pixels, principal point at the image centre, the field of view
+// spanning the LONGER side (Blender's "Auto" sensor fit), so f = max(H, W) / 2 / tan(fov / 2); pixel centres at
+// +0.5.  For H == W this is utils/ray_generator.py:13-50, evaluated in the same float order.
+__device__ __forceinline__ float pinhole_focal(int H, int W, float fov_rad) {
+  return (max(H, W) * 0.5f) / tanf(0.5f * fov_rad);
+}
+
 // Ray-bundle patch tokens for V pinhole cameras in camera space:
 //   utils/ray_generator.py:13-50 (c2w = identity) + models/view_transformer.py:104-107.
-// out [V, (R/8)^2, 192] f16, feature = c*64 + p1*8 + p2, token = h1*(R/8) + w1.
-__global__ void ray_tokens_kernel(const float* __restrict__ fov_deg, uint16_t* __restrict__ out, int V,
-                                  int R) {
-  const int P = 8, T = R / P;
+// out [V, (H/8)*(W/8), 192] f16, feature = c*64 + p1*8 + p2, token = h1*(W/8) + w1 (row-major patch grid).
+__global__ void ray_tokens_kernel(const float* __restrict__ fov_deg, uint16_t* __restrict__ out, int V, int H,
+                                  int W) {
+  const int P = 8, Tw = W / P;
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const long long per_view = (long long)T * T * 192;
+  const long long per_view = (long long)(H / P) * Tw * 192;
   if (t >= V * per_view) return;
   const int v = t / per_view;
   const int rem = t % per_view;
   const int tok = rem / 192, f = rem % 192;
   const int c = f >> 6, p1 = (f >> 3) & 7, p2 = f & 7;
-  const int py = (tok / T) * P + p1, px = (tok % T) * P + p2;
+  const int py = (tok / Tw) * P + p1, px = (tok % Tw) * P + p2;
   const float fov = fov_deg[v] / 180.f * 3.14159265358979323846f;
-  const float fl = (R * 0.5f) / tanf(0.5f * fov);
-  const float dx = ((px + 0.5f) - R * 0.5f) / fl;
-  const float dy = -((py + 0.5f) - R * 0.5f) / fl;
+  const float fl = pinhole_focal(H, W, fov);
+  const float dx = ((px + 0.5f) - W * 0.5f) / fl;
+  const float dy = -((py + 0.5f) - H * 0.5f) / fl;
   const float inv = 1.0f / fmaxf(sqrtf(dx * dx + dy * dy + 1.f), 1e-12f);
   const float val = (c == 0 ? dx : (c == 1 ? dy : -1.f)) * inv;
   __half h = __float2half(val);
   out[t] = *reinterpret_cast<uint16_t*>(&h);
 }
 
-// explicit ray map [V, R, R, 3] fp32 -> patch tokens (same layout as ray_tokens_kernel): the model-level
+// explicit ray map [V, H, W, 3] fp32 -> patch tokens (same layout as ray_tokens_kernel): the model-level
 // entry RenderFormer.forward(..., rays_d, ...) (models/renderformer.py:171-206) hands the rays in
-__global__ void ray_map_tokens_kernel(const float* __restrict__ rays, uint16_t* __restrict__ out, int V, int R) {
-  const int P = 8, T = R / P;
+__global__ void ray_map_tokens_kernel(const float* __restrict__ rays, uint16_t* __restrict__ out, int V, int H,
+                                      int W) {
+  const int P = 8, Tw = W / P;
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const long long per_view = (long long)T * T * 192;
+  const long long per_view = (long long)(H / P) * Tw * 192;
   if (t >= V * per_view) return;
   const int v = t / per_view;
   const int rem = t % per_view;
   const int tok = rem / 192, f = rem % 192;
   const int c = f >> 6, p1 = (f >> 3) & 7, p2 = f & 7;
-  const int py = (tok / T) * P + p1, px = (tok % T) * P + p2;
-  __half h = __float2half(rays[(((long long)v * R + py) * R + px) * 3 + c]);
+  const int py = (tok / Tw) * P + p1, px = (tok % Tw) * P + p2;
+  __half h = __float2half(rays[(((long long)v * H + py) * W + px) * 3 + c]);
   out[t] = *reinterpret_cast<uint16_t*>(&h);
 }
 
-// Pinhole ray map of V cameras: rays_d [V, R, R, 3] fp32 = normalize(R_v * ((x - cx) / f, -(y - cy) / f, -1)),
-// pixel centres, f = R / 2 / tan(fov / 2), fov in RADIANS as RayGenerator.forward takes it
-// (utils/ray_generator.py:13-50).  One thread per pixel, 12-byte stores.
+// Pinhole ray map of V cameras: rays_d [V, H, W, 3] fp32 = normalize(R_v * ((x - cx) / f, -(y - cy) / f, -1)),
+// the camera of pinhole_focal, fov in RADIANS as RayGenerator.forward takes it (utils/ray_generator.py:13-50).
+// One thread per pixel, 12-byte stores.
 __global__ void ray_map_kernel(const float* __restrict__ c2w, const float* __restrict__ fov_rad, float* __restrict__ out,
-                               int V, int R) {
+                               int V, int H, int W) {
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= (long long)V * R * R) return;
-  const int v = t / ((long long)R * R);
-  const int rem = t % ((long long)R * R);
-  const int py = rem / R, px = rem % R;
-  const float fl = (R * 0.5f) / tanf(0.5f * fov_rad[v]);
-  const float d[3] = {((px + 0.5f) - R * 0.5f) / fl, -((py + 0.5f) - R * 0.5f) / fl, -1.0f};
+  if (t >= (long long)V * H * W) return;
+  const int v = t / ((long long)H * W);
+  const int rem = t % ((long long)H * W);
+  const int py = rem / W, px = rem % W;
+  const float fl = pinhole_focal(H, W, fov_rad[v]);
+  const float d[3] = {((px + 0.5f) - W * 0.5f) / fl, -((py + 0.5f) - H * 0.5f) / fl, -1.0f};
   const float* m = c2w + (long long)v * 16;
   float r[3];
 #pragma unroll
@@ -761,30 +769,45 @@ extern "C" int rfb_vn_encode(const float* vn, void* out, int n, int nfreq, int l
   RFB_LAUNCHED("vn_encode_kernel");
 }
 
+extern "C" int rfb_ray_tokens_hw(const float* fov_deg, void* out, int n_views, int height, int width,
+                                 rfb_stream_t stream) {
+  if (!fov_deg || !out || n_views <= 0 || height <= 0 || width <= 0 || height % 8 || width % 8) return RFB_ERR_ARG;
+  const long long total = (long long)n_views * (height / 8) * (width / 8) * 192;
+  ray_tokens_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(fov_deg, (uint16_t*)out,
+                                                                                       n_views, height, width);
+  RFB_LAUNCHED("ray_tokens_kernel");
+}
+
 extern "C" int rfb_ray_tokens(const float* fov_deg, void* out, int n_views, int resolution,
                               rfb_stream_t stream) {
-  if (!fov_deg || !out || n_views <= 0 || resolution % 8) return RFB_ERR_ARG;
-  const long long total = (long long)n_views * (resolution / 8) * (resolution / 8) * 192;
-  ray_tokens_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(fov_deg, (uint16_t*)out,
-                                                                                       n_views, resolution);
-  RFB_LAUNCHED("ray_tokens_kernel");
+  return rfb_ray_tokens_hw(fov_deg, out, n_views, resolution, resolution, stream);
+}
+
+extern "C" int rfb_ray_map_hw(const float* c2w, const float* fov_rad, float* rays_d, int n_views, int height, int width,
+                              rfb_stream_t stream) {
+  if (!c2w || !fov_rad || !rays_d || n_views <= 0 || height <= 0 || width <= 0) return RFB_ERR_ARG;
+  const long long total = (long long)n_views * height * width;
+  ray_map_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(c2w, fov_rad, rays_d, n_views,
+                                                                                    height, width);
+  RFB_LAUNCHED("ray_map_kernel");
 }
 
 extern "C" int rfb_ray_map(const float* c2w, const float* fov_rad, float* rays_d, int n_views, int resolution,
                            rfb_stream_t stream) {
-  if (!c2w || !fov_rad || !rays_d || n_views <= 0 || resolution <= 0) return RFB_ERR_ARG;
-  const long long total = (long long)n_views * resolution * resolution;
-  ray_map_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(c2w, fov_rad, rays_d, n_views,
-                                                                                    resolution);
-  RFB_LAUNCHED("ray_map_kernel");
+  return rfb_ray_map_hw(c2w, fov_rad, rays_d, n_views, resolution, resolution, stream);
+}
+
+extern "C" int rfb_ray_map_tokens_hw(const float* rays_d, void* out, int n_views, int height, int width,
+                                     rfb_stream_t stream) {
+  if (!rays_d || !out || n_views <= 0 || height <= 0 || width <= 0 || height % 8 || width % 8) return RFB_ERR_ARG;
+  const long long total = (long long)n_views * (height / 8) * (width / 8) * 192;
+  ray_map_tokens_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(rays_d, (uint16_t*)out,
+                                                                                           n_views, height, width);
+  RFB_LAUNCHED("ray_map_tokens_kernel");
 }
 
 extern "C" int rfb_ray_map_tokens(const float* rays_d, void* out, int n_views, int resolution, rfb_stream_t stream) {
-  if (!rays_d || !out || n_views <= 0 || resolution % 8) return RFB_ERR_ARG;
-  const long long total = (long long)n_views * (resolution / 8) * (resolution / 8) * 192;
-  ray_map_tokens_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(rays_d, (uint16_t*)out,
-                                                                                           n_views, resolution);
-  RFB_LAUNCHED("ray_map_tokens_kernel");
+  return rfb_ray_map_tokens_hw(rays_d, out, n_views, resolution, resolution, stream);
 }
 
 extern "C" int rfb_positions(const float* tri, const uint8_t* mask, const float* c2w, float* pos, int n,

@@ -24,6 +24,7 @@ import sys
 import torch
 import torch.distributed as dist
 
+from .config import view_grid
 from .engine import RowShard, SceneState
 
 
@@ -194,7 +195,7 @@ def gather_images(img: torch.Tensor, dst: int = 0, sizes: Optional[List[int]] = 
 
 
 @torch.no_grad()
-def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov, resolution: int = 512, dst: Optional[int] = 0,
+def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov, resolution=512, dst: Optional[int] = 0,
                    texture_own_rows: bool = False, torch_dtype: torch.dtype = torch.float16, async_gather: bool = False):
     """`RenderFormerRenderingPipeline.render` on all ranks of the process group: every rank passes the
     SAME scene and the full camera list c2w [B,V,4,4] / fov [B,V,1]; the scene stage is row-sharded, each
@@ -204,7 +205,8 @@ def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov, resolution: int
     CUDA-graph replay.  `async_gather` (one scene per call): the image gather is only enqueued and a
     GatherHandle is returned on every rank -- a caller rendering job after job lets the gather of job k
     travel over NVLink while the scene stage of job k+1 runs, and calls `handle.wait()` before using the
-    images (at the latest before the job after next)."""
+    images (at the latest before the job after next).  `resolution`: an int or (H, W), as in `render`."""
+    resolution = view_grid(pipe.config, resolution)
     world, rank = _world()
     V = c2w.shape[1]
     mine = view_slice(V, world, rank)
@@ -239,7 +241,7 @@ def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov, resolution: int
 
 
 @torch.no_grad()
-def render_stream_sharded(pipe, scenes, resolution: int = 512, ldr: Optional[str] = None,
+def render_stream_sharded(pipe, scenes, resolution=512, ldr: Optional[str] = None,
                           torch_dtype: torch.dtype = torch.float16):
     """Multi-GPU counterpart of `RenderFormerRenderingPipeline.render_stream`: every rank iterates the SAME
     sequence of host scene dicts (keys of `render`).  Each rank uploads the geometry and only ITS OWN
@@ -248,7 +250,8 @@ def render_stream_sharded(pipe, scenes, resolution: int = 512, ldr: Optional[str
     frames).  Uploads of scene i+1 and downloads of scene i overlap the kernels of the neighbouring scene.
 
     Yields (view_slice, pinned host tensor [B, V_rank, H, W, 3]) per scene; the buffer belongs to a ring of
-    three."""
+    three.  `resolution`: an int or (H, W), as in `render`."""
+    resolution = view_grid(pipe.config, resolution)
     dev = pipe.device
     world, rank = _world()
     main = torch.cuda.current_stream(dev)

@@ -21,7 +21,7 @@ import torch
 
 from . import lib as L
 from . import ops
-from .config import RenderFormerConfig
+from .config import RenderFormerConfig, view_grid
 
 EPS = 1e-6  # reference: layers/attention.py:16
 
@@ -602,29 +602,29 @@ class Engine:
 
     @torch.no_grad()
     def render_views(self, st: SceneState, b: int, c2w: Optional[torch.Tensor], fov_deg: Optional[torch.Tensor],
-                     resolution: int, taps: Optional[dict] = None, rays_d: Optional[torch.Tensor] = None,
+                     resolution, taps: Optional[dict] = None, rays_d: Optional[torch.Tensor] = None,
                      tri_cam: Optional[torch.Tensor] = None, pos_cam: Optional[torch.Tensor] = None,
                      raw_log: bool = False, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """Render V views of scene `b` -> HDR fp32 [V,R,R,3].  Either cameras (c2w [V,4,4], fov_deg [V] or
-        [V,1]; rays and camera-space triangles are derived on the device) or, for the model-level entry
-        (models/renderformer.py:171-206), an explicit camera-space ray map `rays_d` [V,R,R,3] together
+        """Render V views of scene `b` -> HDR fp32 [V,H,W,3]; `resolution` is an int (square) or (H, W)
+        (config.view_grid).  Either cameras (c2w [V,4,4], fov_deg [V] or [V,1]; rays and camera-space triangles
+        are derived on the device, fov spanning the longer image side) or, for the model-level entry
+        (models/renderformer.py:171-206), an explicit camera-space ray map `rays_d` [V,H,W,3] together
         with the camera-space triangles `tri_cam` [V,N,9] -- or the ready RoPE positions `pos_cam`
         [V,Nt,9] (register centroids included) as ViewTransformer.forward receives them
-        (models/view_transformer.py:88).  `raw_log`: return the head's pre-ELU output [V,R,R,3] instead
-        (DPTHead.forward, layers/dpt.py:242-273).  `out`: contiguous fp32 [V,R,R,3] buffer the last kernel
+        (models/view_transformer.py:88).  `raw_log`: return the head's pre-ELU output [V,H,W,3] instead
+        (DPTHead.forward, layers/dpt.py:242-273).  `out`: contiguous fp32 [V,H,W,3] buffer the last kernel
         writes the image into (a slice of the caller's result tensor: no concatenation afterwards)."""
         cfg, dev = self.cfg, self.device
         explicit = rays_d is not None
         if explicit and tri_cam is None and pos_cam is None:
             raise ValueError("rays_d needs tri_cam (camera-space triangle vertices) or pos_cam")
-        V, R = (rays_d.shape[0] if explicit else c2w.shape[0]), resolution
-        if R % 64 != 0 and cfg.view_transformer_use_swin_attn:
-            raise ValueError("resolution must be a multiple of 64 for swin attention")  # SURVEY §8b
-        if R % 8 != 0:
-            raise ValueError("resolution must be a multiple of the 8-pixel patch size")
-        Hp = Wp = R // 8
+        V = rays_d.shape[0] if explicit else c2w.shape[0]
+        H, W = view_grid(cfg, resolution)
+        Hp, Wp = H // 8, W // 8
         Ntp, N = st.Ntp, st.N
         if explicit:
+            if tuple(rays_d.shape[1:]) != (H, W, 3):
+                raise ValueError(f"rays_d must be [V, {H}, {W}, 3], got {tuple(rays_d.shape)}")
             rays = rays_d.to(dev, torch.float32).contiguous()
             if pos_cam is not None:
                 pos = torch.zeros((V, Ntp, 9), dtype=torch.float32, device=dev)
@@ -635,27 +635,28 @@ class Engine:
                 for vi in range(V):  # centroid registers + vertices, already in camera space
                     ops.positions(tc[vi], st.mask_u8[b], None, pos[vi], n=N, n_reg=cfg.num_register_tokens,
                                   rows_out=Ntp, n_views=1)
-            x = self.ray_tokens(V, R, rays=rays)
+            x = self.ray_tokens(V, H, W, rays=rays)
         else:
             c2w = c2w.to(dev, torch.float32).contiguous()
             fov = fov_deg.reshape(-1).to(dev, torch.float32).contiguous()
             pos = ops.positions(st.tri[b], st.mask_u8[b], c2w, self._e((V, Ntp, 9), torch.float32), n=N,
                                 n_reg=cfg.num_register_tokens, rows_out=Ntp, n_views=V)
-            x = self.ray_tokens(V, R, fov=fov)
+            x = self.ray_tokens(V, H, W, fov=fov)
         feats = self.decoder_layers(st, b, x, pos, V, Hp, Wp, taps)
         return self._dpt(feats, V, Hp, Wp, raw_out=raw_log, out=out)
 
-    def ray_tokens(self, V: int, R: int, fov=None, rays=None):
-        """Ray-bundle patch tokens x fp32 [V*(R/8)^2, dv]: pinhole rays (utils/ray_generator.py:13-50) or an
-        explicit ray map -> 8x8 patches -> ray_map_patch_token + RMSNorm(Linear)  (view_transformer.py:104-108)."""
+    def ray_tokens(self, V: int, H: int, W: int, fov=None, rays=None):
+        """Ray-bundle patch tokens x fp32 [V*(H/8)*(W/8), dv], row-major patch grid: pinhole rays
+        (utils/ray_generator.py:13-50) or an explicit ray map -> 8x8 patches -> ray_map_patch_token +
+        RMSNorm(Linear)  (view_transformer.py:104-108)."""
         w = self.w
         dv = self.cfg.view_transformer_latent_dim
-        rows = V * (R // 8) ** 2
+        rows = V * (H // 8) * (W // 8)
         rt = self._e((rows, 192), torch.float16)
         if rays is not None:
-            ops.ray_map_tokens(rays, rt, n_views=V, resolution=R)
+            ops.ray_map_tokens(rays, rt, n_views=V, height=H, width=W)
         else:
-            ops.ray_tokens(fov, rt, n_views=V, resolution=R)
+            ops.ray_tokens(fov, rt, n_views=V, height=H, width=W)
         lin = ops.gemm(rt, w["ray.w"], bias=w["ray.b"], out_dtype=torch.float32)
         x = self._e((rows, dv), torch.float32)
         ops.token_assemble(lin, w["ray.norm"], None, None, w["ray.token"], None, x, n_prefix=0, rows_in=rows,

@@ -7,6 +7,12 @@ from __future__ import annotations
 from .config import RenderFormerConfig
 
 
+def _patch_grid(resolution):
+    """(H/8, W/8) of an int (square) or (H, W) resolution."""
+    h, w = tuple(resolution) if isinstance(resolution, (tuple, list)) else (resolution, resolution)
+    return h // 8, w // 8
+
+
 def scene_flops(cfg: RenderFormerConfig, n_tris: int) -> float:
     d, f, L = cfg.latent_dim, cfg.dim_feedforward, cfg.num_layers
     nt = n_tris + cfg.num_register_tokens
@@ -18,11 +24,11 @@ def scene_flops(cfg: RenderFormerConfig, n_tris: int) -> float:
     return tokens + L * layer + hoisted_kv
 
 
-def dpt_flops(cfg: RenderFormerConfig, resolution: int) -> float:
+def dpt_flops(cfg: RenderFormerConfig, resolution) -> float:
     dv, F = cfg.view_transformer_latent_dim, cfg.dpt_features
     C = cfg.dpt_out_channels
-    hp = resolution // 8
-    p = hp * hp
+    hp, wp = _patch_grid(resolution)
+    p = hp * wp
     fl = sum(2.0 * p * dv * c for c in C)                      # 1x1 projects
     fl += 2.0 * p * C[0] * C[0] * 16 + 2.0 * p * C[1] * C[1] * 4   # ConvT k4s4, k2s2
     fl += 2.0 * (p / 4) * 9 * C[3] * C[3]                          # 3x3 stride 2
@@ -37,14 +43,16 @@ def dpt_flops(cfg: RenderFormerConfig, resolution: int) -> float:
     return fl
 
 
-def view_flops(cfg: RenderFormerConfig, n_tris: int, resolution: int) -> float:
+def view_flops(cfg: RenderFormerConfig, n_tris: int, resolution) -> float:
+    """`resolution`: an int (square) or (H, W)."""
     dv, fv, Lv = cfg.view_transformer_latent_dim, cfg.view_transformer_ffn_hidden_dim, cfg.view_transformer_n_layers
     nt = n_tris + cfg.num_register_tokens
-    nr = (resolution // 8) ** 2
+    hp, wp = _patch_grid(resolution)
+    nr = hp * wp
     self_keys = 64 if cfg.view_transformer_use_swin_attn else nr
     layer = 12.0 * nr * dv * dv + 4.0 * nr * nt * dv + 4.0 * nr * self_keys * dv + 6.0 * nr * dv * fv
     return 2.0 * nr * 192 * dv + Lv * layer + dpt_flops(cfg, resolution)
 
 
-def job_flops(cfg: RenderFormerConfig, n_tris: int, resolution: int, n_scenes: int, n_views: int) -> float:
+def job_flops(cfg: RenderFormerConfig, n_tris: int, resolution, n_scenes: int, n_views: int) -> float:
     return n_scenes * (scene_flops(cfg, n_tris) + n_views * view_flops(cfg, n_tris, resolution))

@@ -452,7 +452,7 @@ def prefetch(iterable: Iterable, depth: int = 2):
         t.join(timeout=5)
 
 
-def render_to_files(pipeline, scenes: Iterable[dict], names: Sequence[str], out_dir: str, resolution: int = 512,
+def render_to_files(pipeline, scenes: Iterable[dict], names: Sequence[str], out_dir: str, resolution=512,
                     torch_dtype=None, tone_mapper: str = "none", pad_to: Optional[int] = None,
                     save_video: bool = False, workers: int = 4, fps: int = 24, sharded: bool = False) -> List[str]:
     """The batch_infer.py loop (batch_infer.py:122-172) with nothing serialised behind the renderer: `scenes`
@@ -460,7 +460,7 @@ def render_to_files(pipeline, scenes: Iterable[dict], names: Sequence[str], out_
     of image i-1 overlap the kernels of scene i) and every frame is handed to a `FrameWriter`.  Files are
     named like the reference's: `{name}_view_{v}.exr`, `{name}_view_{v}.png`, `video.mp4`.  `names[i]` belongs
     to the i-th scene (a scene dict holding B > 1 scenes takes B consecutive names).  Returns the frame paths
-    (without extension) this process wrote, in order.
+    (without extension) this process wrote, in order.  `resolution` is an int or (H, W), as in `render`.
 
     `sharded=True` (one process per GPU, `torch.distributed` initialised): every rank iterates the SAME scenes
     through `dist.render_stream_sharded` -- scene stage row-sharded, each rank renders and WRITES its own slice

@@ -69,7 +69,8 @@ class AttnArgs(C.Structure):
 # every symbol include/rfb200.h declares (tests/test_abi.py checks the built library exports them)
 SYMBOLS = [
     "rfb_version", "rfb_launch_count", "rfb_gemm", "rfb_attention", "rfb_attention_ws_bytes", "rfb_rmsnorm", "rfb_rowstat", "rfb_qknorm_rope", "rfb_qknorm_rope_table", "rfb_qkv_post",
-    "rfb_token_assemble", "rfb_texture_prep", "rfb_texture_const_prep", "rfb_vn_encode", "rfb_ray_tokens", "rfb_ray_map_tokens", "rfb_ray_map", "rfb_positions",
+    "rfb_token_assemble", "rfb_texture_prep", "rfb_texture_const_prep", "rfb_vn_encode", "rfb_ray_tokens", "rfb_ray_map_tokens", "rfb_ray_map", "rfb_ray_tokens_hw",
+    "rfb_ray_map_tokens_hw", "rfb_ray_map_hw", "rfb_positions",
     "rfb_pack_mask", "rfb_cast", "rfb_transpose16", "rfb_pixel_shuffle", "rfb_im2col_s2", "rfb_upsample_bilinear", "rfb_ldr_quantize",
 ]
 
@@ -104,6 +105,9 @@ def load() -> C.CDLL:
         "rfb_ray_map": [p, p, p, i, i, p],
         "rfb_vn_encode": [p, p, i, i, i, p],
         "rfb_ray_tokens": [p, p, i, i, p],
+        "rfb_ray_map_tokens_hw": [p, p, i, i, i, p],
+        "rfb_ray_map_hw": [p, p, p, i, i, i, p],
+        "rfb_ray_tokens_hw": [p, p, i, i, i, p],
         "rfb_positions": [p, p, p, p, i, i, i, i, p],
         "rfb_pack_mask": [p, p, i, i, i, i, p],
         "rfb_cast": [p, p, i, ll, p],

@@ -14,7 +14,7 @@ from typing import Dict, Optional
 import torch
 from torch import nn
 
-from .config import RenderFormerConfig
+from .config import RenderFormerConfig, view_grid
 from . import lib as L
 from .engine import Engine, SceneState
 
@@ -137,9 +137,10 @@ class RenderFormer(nn.Module):
         texture_patch_list [B,N,13,P,P] with the emission channels ALREADY log-encoded (the pipeline does
         that before calling the model, rendering_pipeline.py:67-68), valid_mask [B,N], vns [B,N,9],
         rays_o [B,V,3] (must be 0: the origin of camera-space rays; anything else raises), rays_d [B,V,H,W,3] camera-space ray
-        map, tri_vpos_view_tf [B,V,N,9] camera-space vertices.  Returns log-encoded images
-        [B, V, 3, H, W] like the reference.  Alternatively pass cameras as keywords (`c2w` [B,V,4,4],
-        `fov` [B,V,1] degrees, `resolution`) and leave rays_d / tri_vpos_view_tf None.  `tf32_view_tf`
+        map (H != W allowed, within the size rules of config.view_grid), tri_vpos_view_tf [B,V,N,9] camera-space
+        vertices.  Returns log-encoded images [B, V, 3, H, W] like the reference.  Alternatively pass cameras as
+        keywords (`c2w` [B,V,4,4], `fov` [B,V,1] degrees, `resolution` an int or (H, W), fov spanning the longer
+        side as in `RenderFormerRenderingPipeline.render`) and leave rays_d / tri_vpos_view_tf None.  `tf32_view_tf`
         is accepted and ignored; the operand format follows the ambient `torch.autocast("cuda", dtype)` like
         the reference's (fp16 outside an autocast region).  The pipeline calls the engine
         directly and skips the log round trip."""
@@ -150,9 +151,8 @@ class RenderFormer(nn.Module):
         eng = self.engine(operand_dtype(torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else torch.float16))
         st = eng.encode_scene(tri_vpos_list, texture_patch_list, valid_mask, vns, texture_is_log=True)
         if rays_d is not None and tri_vpos_view_tf is not None:
-            B, V, R = rays_d.shape[0], rays_d.shape[1], rays_d.shape[2]
-            assert rays_d.shape[3] == R, "square images only"
-            out = [eng.render_views(st, b, None, None, R, rays_d=rays_d[b], tri_cam=tri_vpos_view_tf[b])
+            B, H, W = rays_d.shape[0], rays_d.shape[2], rays_d.shape[3]
+            out = [eng.render_views(st, b, None, None, (H, W), rays_d=rays_d[b], tri_cam=tri_vpos_view_tf[b])
                    for b in range(B)]
         elif c2w is not None and fov is not None and resolution is not None:
             out = [eng.render_views(st, b, c2w[b], fov[b], resolution) for b in range(c2w.shape[0])]
@@ -299,18 +299,20 @@ class RenderFormerRenderingPipeline:
         return eng.encode_scene(triangles, texture, mask, vn, **kw)
 
     @torch.no_grad()
-    def render_views(self, state: SceneState, c2w, fov, resolution: int = 512, _eager: bool = False) -> torch.Tensor:
+    def render_views(self, state: SceneState, c2w, fov, resolution=512, _eager: bool = False) -> torch.Tensor:
+        """View-dependent stage of `render` on an encoded scene -> HDR [B,V,H,W,3]; `resolution` as in `render`."""
         eng = self.model.engine(state.v_all.dtype)  # the operand format the scene state was built in
+        resolution = view_grid(self.config, resolution)
         if self.cuda_graphs and not _eager and getattr(state, "static", False) and c2w.is_cuda and fov.is_cuda:
             # the graph reads the persistent state in place (no copy of the 300 MB of hoisted K / V)
             return self._graph_entry(("views", id(eng), id(state), resolution, self.view_chunk) + self._sig((c2w, fov)),
                                      (c2w, fov), lambda a, b: self.render_views(state, a, b, resolution, _eager=True))
         B, V = c2w.shape[:2]
         if V == 0:  # a rank whose view slice is empty (fewer views than ranks)
-            return torch.empty((B, 0, resolution, resolution, 3), dtype=torch.float32, device=self.device)
+            return torch.empty((B, 0, *resolution, 3), dtype=torch.float32, device=self.device)
         jobs = [(b, v0) for b in range(B) for v0 in range(0, V, self.view_chunk)]
         # every decoder pass writes its images straight into its slice of the result (no torch.cat afterwards)
-        result = torch.empty((B, V, resolution, resolution, 3), dtype=torch.float32, device=self.device)
+        result = torch.empty((B, V, *resolution, 3), dtype=torch.float32, device=self.device)
         n_str = min(self.view_streams, len(jobs))
         if n_str <= 1:
             for b, v0 in jobs:
@@ -337,10 +339,15 @@ class RenderFormerRenderingPipeline:
         return result
 
     @torch.no_grad()
-    def render(self, triangles, texture, mask, vn, c2w, fov, resolution: int = 512,
+    def render(self, triangles, texture, mask, vn, c2w, fov, resolution=512,
                torch_dtype: torch.dtype = torch.float16):
         """triangles [B,N,3,3], texture [B,N,13,32,32], mask [B,N] bool, vn [B,N,3,3], c2w [B,V,4,4],
         fov [B,V,1] degrees -> HDR [B,V,H,W,3] fp32.
+
+        `resolution` is an int (square H = W) or a (height, width) pair; sides must be multiples of 64 for the
+        swin models and of 8 for full attention (config.view_grid, checked before any launch).  Camera: pinhole,
+        square pixels, principal point at the image centre, `fov` spanning the LONGER image side (Blender's
+        "Auto" sensor fit), i.e. f = max(H, W) / 2 / tan(fov / 2); for H = W this is the reference's camera.
 
         `texture` may also be [B,N,13]: per-triangle constants (what scene_processor/to_h5.py:37-66
         expands to the 32x32 texel grid with a fixed triangular mask).  The texture projection then
@@ -353,6 +360,7 @@ class RenderFormerRenderingPipeline:
         softmax, norms and the residual stream are fp32 in every mode and the result is always fp32.
         Unlike the reference (:68) the caller's `texture` is not modified."""
         op = operand_dtype(torch_dtype)
+        resolution = view_grid(self.config, resolution)
         if self.cuda_graphs and all(t.is_cuda for t in (triangles, texture, mask, vn, c2w, fov)):
             out = self._render_graphed((triangles, texture, mask, vn, c2w, fov), resolution, op)
             return out if self.graph_static_outputs else out.clone()
@@ -391,7 +399,7 @@ class RenderFormerRenderingPipeline:
     def _sig(tensors):
         return tuple((tuple(t.shape), t.dtype) for t in tensors)
 
-    def _render_graphed(self, inputs, resolution: int, op: torch.dtype = torch.bfloat16) -> torch.Tensor:
+    def _render_graphed(self, inputs, resolution, op: torch.dtype = torch.bfloat16) -> torch.Tensor:
         eng = self.model.engine(op)
 
         def run(tri, tex, mask, vn, c2w, fov):
@@ -421,12 +429,12 @@ class RenderFormerRenderingPipeline:
         return ops.ldr_quantize(hdr, tone_mapper)
 
     @torch.no_grad()
-    def render_stream(self, scenes, resolution: int = 512, torch_dtype: torch.dtype = torch.float16,
+    def render_stream(self, scenes, resolution=512, torch_dtype: torch.dtype = torch.float16,
                       ldr: Optional[str] = None, pad_to: Optional[int] = None):
         """Render a sequence of scenes given as HOST tensors (the batch_infer.py use case,
         batch_infer.py:103-143): generator over dicts with the keys of `render` ('triangles', 'texture',
         'mask', 'vn', 'c2w', 'fov'), yielding one pinned-host fp32 HDR tensor [B,V,H,W,3] per scene,
-        in order.
+        in order.  `resolution` is an int or (H, W) as in `render`.
 
         The host->device copy of scene i+1 (218 MB of texture for 4096 triangles) runs on a copy
         stream while scene i is being rendered, and the device->host copy of image i overlaps scene

@@ -188,17 +188,19 @@ class TriangleRotaryEmbedding(nn.Module):
 
 # =============================================================================================== utils
 class RayGenerator(nn.Module):
-    """utils/ray_generator.py:6-50 on rfb_ray_map: pinhole pixel-centre rays rotated by R(c2w), normalised."""
+    """utils/ray_generator.py:6-50 on rfb_ray_map_hw: pinhole pixel-centre rays rotated by R(c2w), normalised.
+    `img_res` is an int (square, as in the reference) or (height, width); the fov spans the longer side."""
 
-    def forward(self, c2w, fov, img_res: int = 256):
+    def forward(self, c2w, fov, img_res=256):
         batch_shape = c2w.shape[:-2]
         if not c2w.is_cuda:
             raise L.RfbError("RayGenerator.forward needs CUDA tensors (no CPU fallback)")
+        H, W = tuple(img_res) if isinstance(img_res, (tuple, list)) else (img_res, img_res)
         c = c2w.reshape(-1, 4, 4).to(torch.float32).contiguous()
         f = fov.reshape(-1).to(torch.float32).contiguous()
-        out = torch.empty((c.shape[0], img_res, img_res, 3), dtype=torch.float32, device=c.device)
-        ops.ray_map(c, f, out, n_views=c.shape[0], resolution=img_res)
-        return c2w[..., :3, 3], out.view(*batch_shape, img_res, img_res, 3)
+        out = torch.empty((c.shape[0], H, W, 3), dtype=torch.float32, device=c.device)
+        ops.ray_map(c, f, out, n_views=c.shape[0], height=H, width=W)
+        return c2w[..., :3, 3], out.view(*batch_shape, H, W, 3)
 
 
 @torch.no_grad()
@@ -737,7 +739,8 @@ class DPTHead(nn.Module, _EngineBacked):
 class ViewTransformer(nn.Module, _EngineBacked):
     """models/view_transformer.py:12-127: ray map -> 8x8 patch tokens -> decoder (cross-attention to the
     triangle tokens, swin / full self-attention, SwiGLU) -> DPT head -> ELU; returns the log-encoded image
-    [B, 3, H, W].  One Engine call per batch element (Engine.render_views with an explicit ray map)."""
+    [B, 3, H, W] (H != W within the size rules of config.view_grid).  One Engine call per batch element
+    (Engine.render_views with an explicit ray map)."""
     _parts, _prefix = ("ray", "decoder", "dpt"), "view_transformer."
 
     def __init__(self, config: RenderFormerConfig):
@@ -766,10 +769,9 @@ class ViewTransformer(nn.Module, _EngineBacked):
         if bool((camera_o != 0).any()):
             raise NotImplementedError("view-stage kernels: camera_o must be 0 (camera-space rays)")
         eng = self._engine()
-        B, R = ray_map.shape[0], ray_map.shape[1]
-        if ray_map.shape[2] != R:
-            raise NotImplementedError("square images only")
+        B, H, W = ray_map.shape[0], ray_map.shape[1], ray_map.shape[2]
         st = eng.scene_state_from_tokens(tri_tokens, None, valid_mask)
-        imgs = [eng.render_views(st, b, None, None, R, rays_d=ray_map[b:b + 1], pos_cam=tri_pos[b:b + 1]) for b in range(B)]
-        hdr = torch.cat(imgs, dim=0)                      # [B, R, R, 3] = 10^elu(head) - 1
+        imgs = [eng.render_views(st, b, None, None, (H, W), rays_d=ray_map[b:b + 1], pos_cam=tri_pos[b:b + 1])
+                for b in range(B)]
+        hdr = torch.cat(imgs, dim=0)                      # [B, H, W, 3] = 10^elu(head) - 1
         return torch.log10(hdr + 1.0).permute(0, 3, 1, 2)  # back to what the reference returns (elu(head))

@@ -256,23 +256,41 @@ def vn_encode(vn, out, *, n, nfreq, ld):
     return out
 
 
-def ray_tokens(fov_deg, out, *, n_views, resolution):
+def _image_hw(resolution, height, width):
+    """(height, width) of a ray-kernel call: `height=` / `width=`, or the square `resolution=`."""
+    if height is None and width is None:
+        if resolution is None:
+            raise ValueError("pass resolution= or height= and width=")
+        return resolution, resolution
+    if height is None or width is None or resolution is not None:
+        raise ValueError("pass resolution= or both height= and width=, not a mix")
+    return height, width
+
+
+def ray_tokens(fov_deg, out, *, n_views, resolution=None, height=None, width=None):
+    """Pinhole ray-bundle patch tokens f16 [V, (H/8)*(W/8), 192] from fov in degrees [V] (rfb_ray_tokens_hw)."""
     _need_cuda(fov_deg, out)
-    L.check(_timed("ray_tokens", 0.0, lambda: L.load().rfb_ray_tokens(fov_deg.data_ptr(), out.data_ptr(), n_views, resolution, _stream())), "rfb_ray_tokens")
+    H, W = _image_hw(resolution, height, width)
+    L.check(_timed("ray_tokens", 0.0, lambda: L.load().rfb_ray_tokens_hw(fov_deg.data_ptr(), out.data_ptr(), n_views, H, W,
+                                                                          _stream())), "rfb_ray_tokens_hw")
     return out
 
 
-def ray_map_tokens(rays_d, out, *, n_views, resolution):
+def ray_map_tokens(rays_d, out, *, n_views, resolution=None, height=None, width=None):
+    """Explicit ray map fp32 [V, H, W, 3] -> patch tokens f16 [V, (H/8)*(W/8), 192] (rfb_ray_map_tokens_hw)."""
     _need_cuda(rays_d, out)
-    L.check(_timed("ray_map_tokens", 0.0, lambda: L.load().rfb_ray_map_tokens(rays_d.data_ptr(), out.data_ptr(), n_views,
-                                                                              resolution, _stream())), "rfb_ray_map_tokens")
+    H, W = _image_hw(resolution, height, width)
+    L.check(_timed("ray_map_tokens", 0.0, lambda: L.load().rfb_ray_map_tokens_hw(rays_d.data_ptr(), out.data_ptr(), n_views,
+                                                                                 H, W, _stream())), "rfb_ray_map_tokens_hw")
     return out
 
 
-def ray_map(c2w, fov_rad, out, *, n_views, resolution):
+def ray_map(c2w, fov_rad, out, *, n_views, resolution=None, height=None, width=None):
+    """Pinhole ray map fp32 [V, H, W, 3] from c2w [V,4,4] and fov in radians [V] (rfb_ray_map_hw)."""
     _need_cuda(c2w, fov_rad, out)
-    L.check(_timed("ray_map", 0.0, lambda: L.load().rfb_ray_map(c2w.data_ptr(), fov_rad.data_ptr(), out.data_ptr(), n_views,
-                                                                resolution, _stream())), "rfb_ray_map")
+    H, W = _image_hw(resolution, height, width)
+    L.check(_timed("ray_map", 0.0, lambda: L.load().rfb_ray_map_hw(c2w.data_ptr(), fov_rad.data_ptr(), out.data_ptr(), n_views,
+                                                                   H, W, _stream())), "rfb_ray_map_hw")
     return out
 
 

@@ -6,14 +6,17 @@ converter's `.h5` files (when h5py is installed); frames are named like the refe
 `<scene>_view_<v>.exr`, `<scene>_view_<v>.png`, `video.mp4`.
 
 usage: python tools/render_folder.py --scene_folder scenes/ --model_id /path/to/checkpoint_dir \
-           [--precision fp16|bf16|fp32] [--resolution 512] [--padding_length N] [--constant_texture]
+           [--precision fp16|bf16|fp32] [--resolution 512] [--height H] [--width W] [--padding_length N] [--constant_texture]
            [--tone_mapper none|pbr_neutral] [--save_video] [--output_dir out/] [--workers 4]
 
 Multi-GPU: launch with torchrun (`python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1
 tools/render_folder.py ...`): the scene stage is row-sharded, every rank renders and writes its own views.
 
 `--model_id` is a local directory with config.json + model.safetensors (there is no hub access here);
-`--random_init NAME` renders with seeded random weights of a named architecture instead (smoke runs)."""
+`--random_init NAME` renders with seeded random weights of a named architecture instead (smoke runs).
+
+`--height` / `--width` render H x W frames (e.g. 576 x 1024 for 16:9 video); either one replaces the matching side of
+the square `--resolution`.  The field of view of a scene spans the longer side."""
 import argparse
 import glob
 import os
@@ -37,6 +40,8 @@ def main(argv=None, _pipeline=None) -> int:
     ap.add_argument("--random_init", default=None, help="architecture name (e.g. v1_1_swin_large, tiny_swin) for seeded random weights")
     ap.add_argument("--precision", choices=["bf16", "fp16", "fp32"], default="fp16")
     ap.add_argument("--resolution", type=int, default=512)
+    ap.add_argument("--height", type=int, default=None, help="image height in pixels (overrides --resolution)")
+    ap.add_argument("--width", type=int, default=None, help="image width in pixels (overrides --resolution)")
     ap.add_argument("--padding_length", type=int, default=None, help="pad every scene to this many triangles on the device: one CUDA graph for all scenes")
     ap.add_argument("--constant_texture", action="store_true", help="upload 13 constants per triangle instead of the 32x32 texel grid")
     ap.add_argument("--tone_mapper", choices=["none", "pbr_neutral"], default="none")
@@ -44,6 +49,9 @@ def main(argv=None, _pipeline=None) -> int:
     ap.add_argument("--output_dir", default=None)
     ap.add_argument("--workers", type=int, default=4)
     args = ap.parse_args(argv)
+    resolution = args.resolution
+    if args.height is not None or args.width is not None:
+        resolution = (args.height or args.resolution, args.width or args.resolution)
 
     import torch
     from renderformer_b200 import frame_io, scene_io
@@ -89,7 +97,7 @@ def main(argv=None, _pipeline=None) -> int:
     names = [os.path.splitext(os.path.basename(p))[0] for p in files]
     t0 = time.time()
     # scene files are read / expanded / pinned two scenes ahead on a background thread
-    paths = frame_io.render_to_files(pipe, frame_io.prefetch(scenes(), depth=2), names, out_dir, resolution=args.resolution, torch_dtype=dtype,
+    paths = frame_io.render_to_files(pipe, frame_io.prefetch(scenes(), depth=2), names, out_dir, resolution=resolution, torch_dtype=dtype,
                                      tone_mapper=args.tone_mapper, pad_to=args.padding_length if world == 1 else None,
                                      save_video=args.save_video, workers=args.workers, sharded=world > 1)
     dt = time.time() - t0
