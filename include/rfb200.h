@@ -110,6 +110,11 @@ typedef struct {
   int vt_rows_per_batch;
   long long vt_ld;
   long long vt_batch_stride;
+  /* ---- output crop (conv A with RFB_EPI_FINAL / RFB_EPI_FINAL_RAW; all zero = none): only the pixels of the
+   * window [crop_top, crop_top + crop_h) x [crop_left, crop_left + crop_w) of the H x Wd image are stored, pixel
+   * (b, y, x) to row (b * crop_h + y - crop_top) * crop_w + (x - crop_left) of out [B, crop_h, crop_w, ldo].
+   * The window must lie inside the image; the rest of the image is computed and discarded (overscan). */
+  int crop_h, crop_w, crop_top, crop_left;
 } rfb_gemm_args;
 
 int rfb_gemm(const rfb_gemm_args* a, rfb_stream_t stream);
@@ -243,6 +248,12 @@ int rfb_vn_encode(const float* vn, void* out, int n, int nfreq, int ld, rfb_stre
 /* camera-space ray bundles -> patch tokens (utils/ray_generator.py:13-50 with identity c2w); fov in degrees. */
 int rfb_ray_tokens_hw(const float* fov_deg, void* out, int n_views, int height, int width, rfb_stream_t stream);
 int rfb_ray_tokens(const float* fov_deg, void* out, int n_views, int resolution, rfb_stream_t stream);
+/* the same over a canvas_h x canvas_w canvas (sides multiples of 8) that holds the height x width image at canvas
+ * pixel (top, left): tokens [V, (canvas_h/8)*(canvas_w/8), 192]; the camera is the image's (f from max(height,
+ * width)), with the principal point at the window's centre (left + width/2, top + height/2).  rfb_ray_tokens_hw
+ * is the case canvas == image, top = left = 0. */
+int rfb_ray_tokens_canvas(const float* fov_deg, void* out, int n_views, int canvas_h, int canvas_w, int height,
+                          int width, int top, int left, rfb_stream_t stream);
 
 /* RayGenerator.forward (utils/ray_generator.py:13-50) for callers that want the ray map itself: c2w [V,4,4],
  * fov in RADIANS [V] -> rays_d fp32 [V, H, W, 3] (rotated by R(c2w), L2-normalised). */

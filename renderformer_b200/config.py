@@ -142,11 +142,8 @@ class RenderFormerConfig:
             raise NotImplementedError("unsupported RenderFormerConfig options: " + ", ".join(bad))
 
 
-def view_grid(cfg: RenderFormerConfig, resolution) -> Tuple[int, int]:
-    """(height, width) in pixels of the images `resolution` asks for: an int is a square image, a pair is
-    (height, width).  Sides must be multiples of 64 for the swin decoder (8x8 windows of 8x8-pixel patches, the
-    reference's own constraint, SURVEY §8b) and multiples of the 8-pixel patch for full attention.  Raises
-    ValueError before anything is launched."""
+def _size_pair(resolution) -> Tuple[int, int]:
+    """(height, width) of an int (square) or a (height, width) pair of positive ints; ValueError otherwise."""
     if isinstance(resolution, (tuple, list)):
         if len(resolution) != 2:
             raise ValueError(f"resolution must be an int or a (height, width) pair, got {resolution!r}")
@@ -155,10 +152,33 @@ def view_grid(cfg: RenderFormerConfig, resolution) -> Tuple[int, int]:
         hw = (resolution, resolution)
     if not all(isinstance(s, numbers.Integral) and not isinstance(s, bool) and s > 0 for s in hw):
         raise ValueError(f"resolution must be a positive int or a (height, width) pair of positive ints, got {resolution!r}")
-    H, W = int(hw[0]), int(hw[1])
+    return int(hw[0]), int(hw[1])
+
+
+def view_grid(cfg: RenderFormerConfig, resolution) -> Tuple[int, int]:
+    """(height, width) in pixels of the images `resolution` asks for: an int is a square image, a pair is
+    (height, width).  Sides must be multiples of 64 for the swin decoder (8x8 windows of 8x8-pixel patches, the
+    reference's own constraint, SURVEY §8b) and multiples of the 8-pixel patch for full attention.  Raises
+    ValueError before anything is launched."""
+    H, W = _size_pair(resolution)
     if cfg.view_transformer_use_swin_attn and (H % 64 or W % 64):
         raise ValueError(f"image height and width must be multiples of 64 for swin attention, got {H}x{W}")
     if H % cfg.patch_size or W % cfg.patch_size:
         raise ValueError(f"image height and width must be multiples of the {cfg.patch_size}-pixel patch size, "
                          f"got {H}x{W}")
     return H, W
+
+
+def overscan_grid(cfg: RenderFormerConfig, resolution) -> Tuple[Tuple[int, int], Tuple[int, int], Tuple[int, int]]:
+    """Overscan geometry of an image of ANY positive size: ((H, W), (Hc, Wc), (top, left)).
+
+    The model runs on a canvas Hc x Wc whose sides are H, W rounded up to the grid of `view_grid` (64 for swin,
+    the 8-pixel patch for full attention); the requested H x W window sits at canvas pixel (top, left) =
+    ((Hc - H) // 2, (Wc - W) // 2).  The camera is the one of the requested image (f from max(H, W), principal
+    point at the window's centre), so every returned pixel is the model's output for a real H x W pinhole image;
+    only the window is stored.  A size already on the grid is its own canvas.  Validates like `view_grid` and
+    raises ValueError before anything is launched."""
+    H, W = _size_pair(resolution)
+    m = 64 if cfg.view_transformer_use_swin_attn else cfg.patch_size
+    Hc, Wc = -(-H // m) * m, -(-W // m) * m
+    return (H, W), (Hc, Wc), ((Hc - H) // 2, (Wc - W) // 2)

@@ -61,7 +61,22 @@ struct GemmKParams {
   void* vt_out;
   int vt_dtype, vt_split, vt_rows_per_batch;
   long long vt_ld, vt_batch_stride;
+  // conv output crop (final epilogue only; crop_w == 0: none): only pixels of the window [crop_top, +crop_h) x
+  // [crop_left, +crop_w) are stored, to row (b * crop_h + y - crop_top) * crop_w + x - crop_left
+  int crop_h, crop_w, crop_top, crop_left;
 };
+
+// output row of conv pixel (b, y, x); false when the pixel lies outside the image or outside the crop window
+__device__ __forceinline__ bool conv_out_row(const GemmKParams& p, int b, int y, int x, long long& orow) {
+  if (p.crop_w) {
+    y -= p.crop_top, x -= p.crop_left;
+    orow = (static_cast<long long>(b) * p.crop_h + y) * p.crop_w + x;
+    return static_cast<unsigned>(y) < static_cast<unsigned>(p.crop_h) &&
+           static_cast<unsigned>(x) < static_cast<unsigned>(p.crop_w);
+  }
+  orow = (static_cast<long long>(b) * p.H + y) * p.Wd + x;
+  return (y < p.H) && (x < p.Wd);
+}
 
 constexpr int kBM = 128;
 constexpr int kBK = 64;
@@ -738,8 +753,7 @@ __global__ void __launch_bounds__(ek_resid(EK) ? kGemmThreadsWG : kGemmThreads, 
         const int rr = mt % per_img;
         const int y = (rr / p.tiles_x) * p.th + r / p.tw;
         const int x = (rr % p.tiles_x) * p.tw + r % p.tw;
-        valid = (y < p.H) && (x < p.Wd);
-        orow = (static_cast<long long>(bi) * p.H + y) * p.Wd + x;
+        valid = conv_out_row(p, bi, y, x, orow);
       }
       // fused-norm inputs of this thread's row: aux row index and 1/rms factor
       int orow_mine = valid ? static_cast<int>(orow) : -1;
@@ -989,8 +1003,8 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
 #pragma unroll 1
       for (int t = 0; t < 2; ++t) {
         const int x = (rr % p.tiles_x) * 16 + t * 8 + (r & 7);
-        const bool valid = (y < p.H) && (x < p.Wd);
-        const long long orow = (static_cast<long long>(bi) * p.H + y) * p.Wd + x;
+        long long orow;
+        const bool valid = conv_out_row(p, bi, y, x, orow);
         const int orow_mine = valid ? static_cast<int>(orow) : -1;
         const uint32_t taddr0 = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + as * 2 * BN + t * BN;
         if (p.epi == RFB_EPI_STORE) {
@@ -1079,6 +1093,12 @@ extern "C" int rfb_gemm(const rfb_gemm_args* a, rfb_stream_t stream_) {
   if (a->out_rscale && !a->in_sumsq) return RFB_ERR_ARG;
   const bool epi_final = a->epi == RFB_EPI_FINAL || a->epi == RFB_EPI_FINAL_RAW;
   if (fused_any && epi_final) return RFB_ERR_ARG;
+  if (a->crop_h || a->crop_w || a->crop_top || a->crop_left) {  // the window must lie inside the conv image
+    if (a->a_mode != RFB_A_CONV3X3 || !epi_final || a->crop_h <= 0 || a->crop_w <= 0 || a->crop_top < 0 ||
+        a->crop_left < 0 || a->crop_h > a->H - a->crop_top || a->crop_w > a->Wd - a->crop_left)
+      return RFB_ERR_ARG;
+    p.crop_h = a->crop_h, p.crop_w = a->crop_w, p.crop_top = a->crop_top, p.crop_left = a->crop_left;
+  }
   if (a->epi == RFB_EPI_SWIGLU && (a->out_rscale || a->out_sumsq || a->out16 || a->col_mul ||
                                    (a->in_rscale && a->scale_dim != 0)))
     return RFB_ERR_ARG;

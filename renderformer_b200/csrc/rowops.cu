@@ -471,12 +471,15 @@ __device__ __forceinline__ float pinhole_focal(int H, int W, float fov_rad) {
 
 // Ray-bundle patch tokens for V pinhole cameras in camera space:
 //   utils/ray_generator.py:13-50 (c2w = identity) + models/view_transformer.py:104-107.
-// out [V, (H/8)*(W/8), 192] f16, feature = c*64 + p1*8 + p2, token = h1*(W/8) + w1 (row-major patch grid).
-__global__ void ray_tokens_kernel(const float* __restrict__ fov_deg, uint16_t* __restrict__ out, int V, int H,
-                                  int W) {
-  const int P = 8, Tw = W / P;
+// out [V, (Hc/8)*(Wc/8), 192] f16 over an Hc x Wc canvas, feature = c*64 + p1*8 + p2, token = h1*(Wc/8) + w1
+// (row-major patch grid).  The camera is the one of the H x W image the canvas holds at (top, left): f from
+// max(H, W), principal point (cx, cy) = (left + W/2, top + H/2) in canvas pixels.  Canvas == image is the plain
+// H x W camera (cx = W * 0.5 is the same exact float the subtraction used before).
+__global__ void ray_tokens_kernel(const float* __restrict__ fov_deg, uint16_t* __restrict__ out, int V, int Hc,
+                                  int Wc, int H, int W, float cx, float cy) {
+  const int P = 8, Tw = Wc / P;
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const long long per_view = (long long)(H / P) * Tw * 192;
+  const long long per_view = (long long)(Hc / P) * Tw * 192;
   if (t >= V * per_view) return;
   const int v = t / per_view;
   const int rem = t % per_view;
@@ -485,8 +488,8 @@ __global__ void ray_tokens_kernel(const float* __restrict__ fov_deg, uint16_t* _
   const int py = (tok / Tw) * P + p1, px = (tok % Tw) * P + p2;
   const float fov = fov_deg[v] / 180.f * 3.14159265358979323846f;
   const float fl = pinhole_focal(H, W, fov);
-  const float dx = ((px + 0.5f) - W * 0.5f) / fl;
-  const float dy = -((py + 0.5f) - H * 0.5f) / fl;
+  const float dx = ((px + 0.5f) - cx) / fl;
+  const float dy = -((py + 0.5f) - cy) / fl;
   const float inv = 1.0f / fmaxf(sqrtf(dx * dx + dy * dy + 1.f), 1e-12f);
   const float val = (c == 0 ? dx : (c == 1 ? dy : -1.f)) * inv;
   __half h = __float2half(val);
@@ -769,13 +772,22 @@ extern "C" int rfb_vn_encode(const float* vn, void* out, int n, int nfreq, int l
   RFB_LAUNCHED("vn_encode_kernel");
 }
 
+extern "C" int rfb_ray_tokens_canvas(const float* fov_deg, void* out, int n_views, int canvas_h, int canvas_w,
+                                     int height, int width, int top, int left, rfb_stream_t stream) {
+  if (!fov_deg || !out || n_views <= 0 || canvas_h <= 0 || canvas_w <= 0 || canvas_h % 8 || canvas_w % 8 ||
+      height <= 0 || width <= 0 || top < 0 || left < 0 || height > canvas_h - top || width > canvas_w - left)
+    return RFB_ERR_ARG;
+  // principal point of the window in canvas pixels: integers + halves, exact in fp32 for any image size here
+  const float cx = (float)left + (float)width * 0.5f, cy = (float)top + (float)height * 0.5f;
+  const long long total = (long long)n_views * (canvas_h / 8) * (canvas_w / 8) * 192;
+  ray_tokens_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      fov_deg, (uint16_t*)out, n_views, canvas_h, canvas_w, height, width, cx, cy);
+  RFB_LAUNCHED("ray_tokens_kernel");
+}
+
 extern "C" int rfb_ray_tokens_hw(const float* fov_deg, void* out, int n_views, int height, int width,
                                  rfb_stream_t stream) {
-  if (!fov_deg || !out || n_views <= 0 || height <= 0 || width <= 0 || height % 8 || width % 8) return RFB_ERR_ARG;
-  const long long total = (long long)n_views * (height / 8) * (width / 8) * 192;
-  ray_tokens_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(fov_deg, (uint16_t*)out,
-                                                                                       n_views, height, width);
-  RFB_LAUNCHED("ray_tokens_kernel");
+  return rfb_ray_tokens_canvas(fov_deg, out, n_views, height, width, height, width, 0, 0, stream);
 }
 
 extern "C" int rfb_ray_tokens(const float* fov_deg, void* out, int n_views, int resolution,

@@ -24,7 +24,6 @@ import sys
 import torch
 import torch.distributed as dist
 
-from .config import view_grid
 from .engine import RowShard, SceneState
 
 
@@ -196,7 +195,8 @@ def gather_images(img: torch.Tensor, dst: int = 0, sizes: Optional[List[int]] = 
 
 @torch.no_grad()
 def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov, resolution=512, dst: Optional[int] = 0,
-                   texture_own_rows: bool = False, torch_dtype: torch.dtype = torch.float16, async_gather: bool = False):
+                   texture_own_rows: bool = False, torch_dtype: torch.dtype = torch.float16, async_gather: bool = False,
+                   overscan: bool = False):
     """`RenderFormerRenderingPipeline.render` on all ranks of the process group: every rank passes the
     SAME scene and the full camera list c2w [B,V,4,4] / fov [B,V,1]; the scene stage is row-sharded, each
     rank renders `view_slice(V)`, and the images are gathered on `dst` (returns [B,V,H,W,3] there and
@@ -205,15 +205,17 @@ def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov, resolution=512,
     CUDA-graph replay.  `async_gather` (one scene per call): the image gather is only enqueued and a
     GatherHandle is returned on every rank -- a caller rendering job after job lets the gather of job k
     travel over NVLink while the scene stage of job k+1 runs, and calls `handle.wait()` before using the
-    images (at the latest before the job after next).  `resolution`: an int or (H, W), as in `render`."""
-    resolution = view_grid(pipe.config, resolution)
+    images (at the latest before the job after next).  `resolution`: an int or (H, W), and `overscan`, as in
+    `render`."""
+    canvas, window, _ = pipe.view_geometry(resolution, overscan)
     world, rank = _world()
     V = c2w.shape[1]
     mine = view_slice(V, world, rank)
     c2w_l, fov_l = c2w[:, mine].contiguous(), fov[:, mine].contiguous()
     sh = row_shard()
     if world == 1:
-        img = pipe.render(triangles, texture, mask, vn, c2w_l, fov_l, resolution=resolution, torch_dtype=torch_dtype)
+        img = pipe.render(triangles, texture, mask, vn, c2w_l, fov_l, resolution=resolution, torch_dtype=torch_dtype,
+                          overscan=overscan)
     else:
         from .model import operand_dtype
         eng = pipe.model.engine(operand_dtype(torch_dtype))
@@ -221,9 +223,10 @@ def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov, resolution=512,
 
         def run(tri, tex, msk, vnn, cw, fv):
             st = eng.encode_scene(tri, tex, msk, vnn, shard=sh, texture_own_rows=texture_own_rows)
-            return pipe.render_views(st, cw, fv, resolution, _eager=True)
+            return pipe.render_views(st, cw, fv, resolution, overscan, _eager=True)
         if pipe.cuda_graphs and all(t.is_cuda for t in inputs) and mine.stop > mine.start:
-            key = ("render_sharded", id(eng), rank, world, resolution, pipe.view_chunk, texture_own_rows) + pipe._sig(inputs)
+            key = (("render_sharded", id(eng), rank, world, canvas, window, pipe.view_chunk, texture_own_rows) +
+                   pipe._sig(inputs))
             img = pipe._graph_entry(key, inputs, run)
         else:
             img = run(*inputs)
@@ -242,7 +245,7 @@ def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov, resolution=512,
 
 @torch.no_grad()
 def render_stream_sharded(pipe, scenes, resolution=512, ldr: Optional[str] = None,
-                          torch_dtype: torch.dtype = torch.float16):
+                          torch_dtype: torch.dtype = torch.float16, overscan: bool = False):
     """Multi-GPU counterpart of `RenderFormerRenderingPipeline.render_stream`: every rank iterates the SAME
     sequence of host scene dicts (keys of `render`).  Each rank uploads the geometry and only ITS OWN
     rows of the texture (1/world of the 218 MB), the scene stage runs row-sharded, each rank renders its
@@ -250,8 +253,8 @@ def render_stream_sharded(pipe, scenes, resolution=512, ldr: Optional[str] = Non
     frames).  Uploads of scene i+1 and downloads of scene i overlap the kernels of the neighbouring scene.
 
     Yields (view_slice, pinned host tensor [B, V_rank, H, W, 3]) per scene; the buffer belongs to a ring of
-    three.  `resolution`: an int or (H, W), as in `render`."""
-    resolution = view_grid(pipe.config, resolution)
+    three.  `resolution`: an int or (H, W), and `overscan`, as in `render`."""
+    canvas, window, _ = pipe.view_geometry(resolution, overscan)
     dev = pipe.device
     world, rank = _world()
     main = torch.cuda.current_stream(dev)
@@ -288,16 +291,16 @@ def render_stream_sharded(pipe, scenes, resolution=512, ldr: Optional[str] = Non
         main.wait_event(ev)
         if sh is None:
             img = pipe.render(d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], d["fov"], resolution=resolution,
-                              torch_dtype=torch_dtype)
+                              torch_dtype=torch_dtype, overscan=overscan)
         else:
             # full camera list is not needed here: the slice was taken on the host
             inputs = (d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], d["fov"])
 
             def run(tri, tex, msk, vnn, cw, fv):
                 st = eng.encode_scene(tri, tex, msk, vnn, shard=sh, texture_own_rows=True)
-                return pipe.render_views(st, cw, fv, resolution, _eager=True)
+                return pipe.render_views(st, cw, fv, resolution, overscan, _eager=True)
             if pipe.cuda_graphs and mine.stop > mine.start:
-                key = ("stream_sharded", id(eng), rank, world, resolution, pipe.view_chunk) + pipe._sig(inputs)
+                key = ("stream_sharded", id(eng), rank, world, canvas, window, pipe.view_chunk) + pipe._sig(inputs)
                 img = pipe._graph_entry(key, inputs, run)
             else:
                 img = run(*inputs)

@@ -604,7 +604,8 @@ class Engine:
     def render_views(self, st: SceneState, b: int, c2w: Optional[torch.Tensor], fov_deg: Optional[torch.Tensor],
                      resolution, taps: Optional[dict] = None, rays_d: Optional[torch.Tensor] = None,
                      tri_cam: Optional[torch.Tensor] = None, pos_cam: Optional[torch.Tensor] = None,
-                     raw_log: bool = False, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+                     raw_log: bool = False, out: Optional[torch.Tensor] = None,
+                     window: Optional[tuple] = None) -> torch.Tensor:
         """Render V views of scene `b` -> HDR fp32 [V,H,W,3]; `resolution` is an int (square) or (H, W)
         (config.view_grid).  Either cameras (c2w [V,4,4], fov_deg [V] or [V,1]; rays and camera-space triangles
         are derived on the device, fov spanning the longer image side) or, for the model-level entry
@@ -613,11 +614,16 @@ class Engine:
         [V,Nt,9] (register centroids included) as ViewTransformer.forward receives them
         (models/view_transformer.py:88).  `raw_log`: return the head's pre-ELU output [V,H,W,3] instead
         (DPTHead.forward, layers/dpt.py:242-273).  `out`: contiguous fp32 [V,H,W,3] buffer the last kernel
-        writes the image into (a slice of the caller's result tensor: no concatenation afterwards)."""
+        writes the image into (a slice of the caller's result tensor: no concatenation afterwards).
+        `window=(h, w, top, left)` (cameras only, config.overscan_grid): `resolution` is the canvas the model runs
+        on, the cameras are those of the h x w image it holds at canvas pixel (top, left), and only that window is
+        stored: the result (and `out`) is [V, h, w, 3]."""
         cfg, dev = self.cfg, self.device
         explicit = rays_d is not None
         if explicit and tri_cam is None and pos_cam is None:
             raise ValueError("rays_d needs tri_cam (camera-space triangle vertices) or pos_cam")
+        if explicit and window is not None:
+            raise ValueError("window (overscan) needs cameras; an explicit ray map covers the whole image")
         V = rays_d.shape[0] if explicit else c2w.shape[0]
         H, W = view_grid(cfg, resolution)
         Hp, Wp = H // 8, W // 8
@@ -641,20 +647,24 @@ class Engine:
             fov = fov_deg.reshape(-1).to(dev, torch.float32).contiguous()
             pos = ops.positions(st.tri[b], st.mask_u8[b], c2w, self._e((V, Ntp, 9), torch.float32), n=N,
                                 n_reg=cfg.num_register_tokens, rows_out=Ntp, n_views=V)
-            x = self.ray_tokens(V, H, W, fov=fov)
+            x = self.ray_tokens(V, H, W, fov=fov, window=window)
         feats = self.decoder_layers(st, b, x, pos, V, Hp, Wp, taps)
-        return self._dpt(feats, V, Hp, Wp, raw_out=raw_log, out=out)
+        return self._dpt(feats, V, Hp, Wp, raw_out=raw_log, out=out, window=window)
 
-    def ray_tokens(self, V: int, H: int, W: int, fov=None, rays=None):
+    def ray_tokens(self, V: int, H: int, W: int, fov=None, rays=None, window=None):
         """Ray-bundle patch tokens x fp32 [V*(H/8)*(W/8), dv], row-major patch grid: pinhole rays
         (utils/ray_generator.py:13-50) or an explicit ray map -> 8x8 patches -> ray_map_patch_token +
-        RMSNorm(Linear)  (view_transformer.py:104-108)."""
+        RMSNorm(Linear)  (view_transformer.py:104-108).  `window=(h, w, top, left)`: H x W is a canvas and the
+        rays are those of the h x w camera whose image sits at (top, left)."""
         w = self.w
         dv = self.cfg.view_transformer_latent_dim
         rows = V * (H // 8) * (W // 8)
         rt = self._e((rows, 192), torch.float16)
         if rays is not None:
             ops.ray_map_tokens(rays, rt, n_views=V, height=H, width=W)
+        elif window is not None:
+            h, w_, top, left = window
+            ops.ray_tokens_canvas(fov, rt, n_views=V, canvas_h=H, canvas_w=W, height=h, width=w_, top=top, left=left)
         else:
             ops.ray_tokens(fov, rt, n_views=V, height=H, width=W)
         lin = ops.gemm(rt, w["ray.w"], bias=w["ray.b"], out_dtype=torch.float32)
@@ -788,10 +798,11 @@ class Engine:
         o = ops.gemm(o, self.w[name + "out.w"], bias=self.w[name + "out.b"], out=self._e((B * H * W, F_), hf))
         return ops.upsample_bilinear(o, self._e((B * Ho * Wo, F_), hf), B=B, Hi=H, Wi=W, Ho=Ho, Wo=Wo, C_=F_)
 
-    def _dpt(self, feats, V, Hp, Wp, raw_out: bool = False, out: Optional[torch.Tensor] = None):
+    def _dpt(self, feats, V, Hp, Wp, raw_out: bool = False, out: Optional[torch.Tensor] = None, window=None):
         """DPTHead.forward (layers/dpt.py:242-273) on four fp16 feature maps [V*Hp*Wp, dv] -> HDR image fp32
         [V, 8Hp, 8Wp, 3] (the head's ELU and the pipeline's 10^x - 1 are the last conv's epilogue), or with
-        `raw_out` the head's own output before the ELU."""
+        `raw_out` the head's own output before the ELU.  `window=(h, w, top, left)`: the last conv stores only that
+        window of the image, [V, h, w, 3]."""
         cfg, w = self.cfg, self.w
         hf = torch.float16
         C = list(cfg.dpt_out_channels)
@@ -821,9 +832,10 @@ class Engine:
         p1 = self._fusion(1, V, *dims[0], Ho, Wo, p2, lraw[0], lact[0])
         # head (layers/dpt.py:266-271); F.interpolate to (8*Hp, 8*Wp) is the identity here (E2)
         o1 = self._conv(p1, "dpt.oc1", V, Ho, Wo, F_, bias=w["dpt.oc1.b"], out=self._e((V * Ho * Wo, F_ // 2), hf))
-        if out is not None and (tuple(out.shape) != (V, Ho, Wo, 3) or out.dtype != torch.float32 or not out.is_contiguous()):
+        Hs, Ws = (Ho, Wo) if window is None else window[:2]
+        if out is not None and (tuple(out.shape) != (V, Hs, Ws, 3) or out.dtype != torch.float32 or not out.is_contiguous()):
             raise ValueError("out must be a contiguous fp32 [V, H, W, 3] tensor")
-        img = out if out is not None else self._e((V, Ho, Wo, 3), torch.float32)
+        img = out if out is not None else self._e((V, Hs, Ws, 3), torch.float32)
         self._conv(o1, "dpt.oc2", V, Ho, Wo, F_ // 2, bias=w["dpt.oc2.b"], epi=L.EPI_FINAL_RAW if raw_out else L.EPI_FINAL,
-                   w2=w["dpt.oc3.w"], b2=w["dpt.oc3.b"], out=img, ldo=3)
+                   w2=w["dpt.oc3.w"], b2=w["dpt.oc3.b"], out=img, ldo=3, crop=window)
         return img

@@ -4,7 +4,7 @@ These formulas reproduce torch's FlopCounterMode on the reference; the hoisted d
 projections are counted once per scene (the reference pays them per view)."""
 from __future__ import annotations
 
-from .config import RenderFormerConfig
+from .config import RenderFormerConfig, overscan_grid
 
 
 def _patch_grid(resolution):
@@ -43,8 +43,11 @@ def dpt_flops(cfg: RenderFormerConfig, resolution) -> float:
     return fl
 
 
-def view_flops(cfg: RenderFormerConfig, n_tris: int, resolution) -> float:
-    """`resolution`: an int (square) or (H, W)."""
+def view_flops(cfg: RenderFormerConfig, n_tris: int, resolution, overscan: bool = False) -> float:
+    """`resolution`: an int (square) or (H, W).  With `overscan` (any size, `render(..., overscan=True)`) a view
+    costs the FLOPs of its canvas (config.overscan_grid): the model runs on the whole canvas, the crop is free."""
+    if overscan:
+        resolution = overscan_grid(cfg, resolution)[1]
     dv, fv, Lv = cfg.view_transformer_latent_dim, cfg.view_transformer_ffn_hidden_dim, cfg.view_transformer_n_layers
     nt = n_tris + cfg.num_register_tokens
     hp, wp = _patch_grid(resolution)
@@ -54,5 +57,6 @@ def view_flops(cfg: RenderFormerConfig, n_tris: int, resolution) -> float:
     return 2.0 * nr * 192 * dv + Lv * layer + dpt_flops(cfg, resolution)
 
 
-def job_flops(cfg: RenderFormerConfig, n_tris: int, resolution, n_scenes: int, n_views: int) -> float:
-    return n_scenes * (scene_flops(cfg, n_tris) + n_views * view_flops(cfg, n_tris, resolution))
+def job_flops(cfg: RenderFormerConfig, n_tris: int, resolution, n_scenes: int, n_views: int,
+              overscan: bool = False) -> float:
+    return n_scenes * (scene_flops(cfg, n_tris) + n_views * view_flops(cfg, n_tris, resolution, overscan))

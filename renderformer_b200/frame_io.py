@@ -454,19 +454,23 @@ def prefetch(iterable: Iterable, depth: int = 2):
 
 def render_to_files(pipeline, scenes: Iterable[dict], names: Sequence[str], out_dir: str, resolution=512,
                     torch_dtype=None, tone_mapper: str = "none", pad_to: Optional[int] = None,
-                    save_video: bool = False, workers: int = 4, fps: int = 24, sharded: bool = False) -> List[str]:
+                    save_video: bool = False, workers: int = 4, fps: int = 24, sharded: bool = False,
+                    overscan: bool = False) -> List[str]:
     """The batch_infer.py loop (batch_infer.py:122-172) with nothing serialised behind the renderer: `scenes`
     (host tensors, the keys of `render`) go through `pipeline.render_stream` (upload of scene i+1 and download
     of image i-1 overlap the kernels of scene i) and every frame is handed to a `FrameWriter`.  Files are
     named like the reference's: `{name}_view_{v}.exr`, `{name}_view_{v}.png`, `video.mp4`.  `names[i]` belongs
     to the i-th scene (a scene dict holding B > 1 scenes takes B consecutive names).  Returns the frame paths
-    (without extension) this process wrote, in order.  `resolution` is an int or (H, W), as in `render`.
+    (without extension) this process wrote, in order.  `resolution` is an int or (H, W), and `overscan` (any size,
+    rendered on the decoder's grid and cropped), as in `render`.
 
     `sharded=True` (one process per GPU, `torch.distributed` initialised): every rank iterates the SAME scenes
     through `dist.render_stream_sharded` -- scene stage row-sharded, each rank renders and WRITES its own slice
     of the views (no image gather; the view index in the file name is the global one).  The video is then
     assembled by rank 0 from the PNG files after a barrier."""
     kw = {} if torch_dtype is None else {"torch_dtype": torch_dtype}
+    if overscan:
+        kw["overscan"] = True
     names = list(names)
     rank, world = 0, 1
     if sharded:

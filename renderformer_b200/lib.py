@@ -45,6 +45,7 @@ class GemmArgs(C.Structure):
         ("col_mul", C.c_void_p), ("aux_row_map", C.c_void_p),
         ("vt_out", C.c_void_p), ("vt_dtype", C.c_int), ("vt_split", C.c_int), ("vt_rows_per_batch", C.c_int),
         ("vt_ld", C.c_longlong), ("vt_batch_stride", C.c_longlong),
+        ("crop_h", C.c_int), ("crop_w", C.c_int), ("crop_top", C.c_int), ("crop_left", C.c_int),
     ]
 
 
@@ -70,7 +71,7 @@ class AttnArgs(C.Structure):
 SYMBOLS = [
     "rfb_version", "rfb_launch_count", "rfb_gemm", "rfb_attention", "rfb_attention_ws_bytes", "rfb_rmsnorm", "rfb_rowstat", "rfb_qknorm_rope", "rfb_qknorm_rope_table", "rfb_qkv_post",
     "rfb_token_assemble", "rfb_texture_prep", "rfb_texture_const_prep", "rfb_vn_encode", "rfb_ray_tokens", "rfb_ray_map_tokens", "rfb_ray_map", "rfb_ray_tokens_hw",
-    "rfb_ray_map_tokens_hw", "rfb_ray_map_hw", "rfb_positions",
+    "rfb_ray_tokens_canvas", "rfb_ray_map_tokens_hw", "rfb_ray_map_hw", "rfb_positions",
     "rfb_pack_mask", "rfb_cast", "rfb_transpose16", "rfb_pixel_shuffle", "rfb_im2col_s2", "rfb_upsample_bilinear", "rfb_ldr_quantize",
 ]
 
@@ -108,6 +109,7 @@ def load() -> C.CDLL:
         "rfb_ray_map_tokens_hw": [p, p, i, i, i, p],
         "rfb_ray_map_hw": [p, p, p, i, i, i, p],
         "rfb_ray_tokens_hw": [p, p, i, i, i, p],
+        "rfb_ray_tokens_canvas": [p, p, i, i, i, i, i, i, i, p],
         "rfb_positions": [p, p, p, p, i, i, i, i, p],
         "rfb_pack_mask": [p, p, i, i, i, i, p],
         "rfb_cast": [p, p, i, ll, p],

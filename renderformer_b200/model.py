@@ -14,7 +14,7 @@ from typing import Dict, Optional
 import torch
 from torch import nn
 
-from .config import RenderFormerConfig, view_grid
+from .config import RenderFormerConfig, overscan_grid, view_grid
 from . import lib as L
 from .engine import Engine, SceneState
 
@@ -298,26 +298,40 @@ class RenderFormerRenderingPipeline:
             return st
         return eng.encode_scene(triangles, texture, mask, vn, **kw)
 
+    def view_geometry(self, resolution, overscan: bool = False):
+        """(canvas, window, image) of a render: the (H, W) canvas the model runs on, the (h, w, top, left) window of
+        it that is returned (None: the whole canvas) and the (h, w) of the returned images.  Without `overscan`
+        the size must be on the decoder's grid (config.view_grid); with it any size is rendered on the canvas of
+        config.overscan_grid.  Raises ValueError before anything is launched."""
+        if not overscan:
+            hw = view_grid(self.config, resolution)
+            return hw, None, hw
+        hw, canvas, (top, left) = overscan_grid(self.config, resolution)
+        return canvas, (None if canvas == hw else (*hw, top, left)), hw
+
     @torch.no_grad()
-    def render_views(self, state: SceneState, c2w, fov, resolution=512, _eager: bool = False) -> torch.Tensor:
-        """View-dependent stage of `render` on an encoded scene -> HDR [B,V,H,W,3]; `resolution` as in `render`."""
+    def render_views(self, state: SceneState, c2w, fov, resolution=512, overscan: bool = False,
+                     _eager: bool = False) -> torch.Tensor:
+        """View-dependent stage of `render` on an encoded scene -> HDR [B,V,H,W,3]; `resolution` and `overscan` as
+        in `render`."""
         eng = self.model.engine(state.v_all.dtype)  # the operand format the scene state was built in
-        resolution = view_grid(self.config, resolution)
+        canvas, window, hw = self.view_geometry(resolution, overscan)
         if self.cuda_graphs and not _eager and getattr(state, "static", False) and c2w.is_cuda and fov.is_cuda:
             # the graph reads the persistent state in place (no copy of the 300 MB of hoisted K / V)
-            return self._graph_entry(("views", id(eng), id(state), resolution, self.view_chunk) + self._sig((c2w, fov)),
-                                     (c2w, fov), lambda a, b: self.render_views(state, a, b, resolution, _eager=True))
+            return self._graph_entry(("views", id(eng), id(state), canvas, window, self.view_chunk) + self._sig((c2w, fov)),
+                                     (c2w, fov), lambda a, b: self.render_views(state, a, b, hw, overscan, _eager=True))
         B, V = c2w.shape[:2]
         if V == 0:  # a rank whose view slice is empty (fewer views than ranks)
-            return torch.empty((B, 0, *resolution, 3), dtype=torch.float32, device=self.device)
+            return torch.empty((B, 0, *hw, 3), dtype=torch.float32, device=self.device)
         jobs = [(b, v0) for b in range(B) for v0 in range(0, V, self.view_chunk)]
-        # every decoder pass writes its images straight into its slice of the result (no torch.cat afterwards)
-        result = torch.empty((B, V, *resolution, 3), dtype=torch.float32, device=self.device)
+        # every decoder pass writes its images straight into its slice of the result (no torch.cat afterwards); with
+        # overscan its last conv stores only the window, so no canvas-sized image exists
+        result = torch.empty((B, V, *hw, 3), dtype=torch.float32, device=self.device)
         n_str = min(self.view_streams, len(jobs))
         if n_str <= 1:
             for b, v0 in jobs:
-                eng.render_views(state, b, c2w[b, v0:v0 + self.view_chunk], fov[b, v0:v0 + self.view_chunk], resolution,
-                                 out=result[b, v0:v0 + self.view_chunk])
+                eng.render_views(state, b, c2w[b, v0:v0 + self.view_chunk], fov[b, v0:v0 + self.view_chunk], canvas,
+                                 out=result[b, v0:v0 + self.view_chunk], window=window)
             return result
         dev = self.device
         while len(self._side_streams) < n_str:
@@ -330,8 +344,8 @@ class RenderFormerRenderingPipeline:
             if i < n_str:
                 side.wait_event(fork)
             with torch.cuda.stream(side):
-                eng.render_views(state, b, c2w[b, v0:v0 + self.view_chunk], fov[b, v0:v0 + self.view_chunk], resolution,
-                                 out=result[b, v0:v0 + self.view_chunk])
+                eng.render_views(state, b, c2w[b, v0:v0 + self.view_chunk], fov[b, v0:v0 + self.view_chunk], canvas,
+                                 out=result[b, v0:v0 + self.view_chunk], window=window)
         for side in self._side_streams[:n_str]:
             ev = torch.cuda.Event()
             ev.record(side)
@@ -340,7 +354,7 @@ class RenderFormerRenderingPipeline:
 
     @torch.no_grad()
     def render(self, triangles, texture, mask, vn, c2w, fov, resolution=512,
-               torch_dtype: torch.dtype = torch.float16):
+               torch_dtype: torch.dtype = torch.float16, overscan: bool = False):
         """triangles [B,N,3,3], texture [B,N,13,32,32], mask [B,N] bool, vn [B,N,3,3], c2w [B,V,4,4],
         fov [B,V,1] degrees -> HDR [B,V,H,W,3] fp32.
 
@@ -348,6 +362,13 @@ class RenderFormerRenderingPipeline:
         swin models and of 8 for full attention (config.view_grid, checked before any launch).  Camera: pinhole,
         square pixels, principal point at the image centre, `fov` spanning the LONGER image side (Blender's
         "Auto" sensor fit), i.e. f = max(H, W) / 2 / tan(fov / 2); for H = W this is the reference's camera.
+
+        `overscan=True` lifts the size rule: `resolution` may be any positive int or (H, W), e.g. (1080, 1920).  The
+        model then runs on the smallest canvas on the grid that holds the image (config.overscan_grid; 1088 x 1920
+        for 1080p), centred, with the SAME camera as above for the H x W image, and only the H x W window is stored.
+        Every returned pixel is the model's output for a real H x W pinhole image; the border costs the decoder
+        0.7 % more pixels at 1080p and 4K, 6.7 % at 720p.  A size already on the grid renders exactly as without
+        overscan.
 
         `texture` may also be [B,N,13]: per-triangle constants (what scene_processor/to_h5.py:37-66
         expands to the 32x32 texel grid with a fixed triangular mask).  The texture projection then
@@ -360,12 +381,12 @@ class RenderFormerRenderingPipeline:
         softmax, norms and the residual stream are fp32 in every mode and the result is always fp32.
         Unlike the reference (:68) the caller's `texture` is not modified."""
         op = operand_dtype(torch_dtype)
-        resolution = view_grid(self.config, resolution)
+        self.view_geometry(resolution, overscan)  # size errors before any launch
         if self.cuda_graphs and all(t.is_cuda for t in (triangles, texture, mask, vn, c2w, fov)):
-            out = self._render_graphed((triangles, texture, mask, vn, c2w, fov), resolution, op)
+            out = self._render_graphed((triangles, texture, mask, vn, c2w, fov), resolution, op, overscan)
             return out if self.graph_static_outputs else out.clone()
         state = self.encode(triangles, texture, mask, vn, torch_dtype=op)
-        return self.render_views(state, c2w, fov, resolution)
+        return self.render_views(state, c2w, fov, resolution, overscan)
 
     def _graph_entry(self, key, inputs, fn):
         """Capture `fn(*static_inputs)` once per key, replay it with `inputs` copied into the static
@@ -399,12 +420,13 @@ class RenderFormerRenderingPipeline:
     def _sig(tensors):
         return tuple((tuple(t.shape), t.dtype) for t in tensors)
 
-    def _render_graphed(self, inputs, resolution, op: torch.dtype = torch.bfloat16) -> torch.Tensor:
+    def _render_graphed(self, inputs, resolution, op: torch.dtype = torch.bfloat16, overscan: bool = False) -> torch.Tensor:
         eng = self.model.engine(op)
+        canvas, window, _ = self.view_geometry(resolution, overscan)
 
         def run(tri, tex, mask, vn, c2w, fov):
-            return self.render_views(eng.encode_scene(tri, tex, mask, vn), c2w, fov, resolution, _eager=True)
-        return self._graph_entry(("render", id(eng), resolution, self.view_chunk) + self._sig(inputs), inputs, run)
+            return self.render_views(eng.encode_scene(tri, tex, mask, vn), c2w, fov, resolution, overscan, _eager=True)
+        return self._graph_entry(("render", id(eng), canvas, window, self.view_chunk) + self._sig(inputs), inputs, run)
 
     def static_scene_state(self, B: int, N: int, torch_dtype: torch.dtype = torch.float16) -> SceneState:
         """The persistent SceneState of this shape (receive buffer of the NCCL broadcast on ranks that do
@@ -430,11 +452,11 @@ class RenderFormerRenderingPipeline:
 
     @torch.no_grad()
     def render_stream(self, scenes, resolution=512, torch_dtype: torch.dtype = torch.float16,
-                      ldr: Optional[str] = None, pad_to: Optional[int] = None):
+                      ldr: Optional[str] = None, pad_to: Optional[int] = None, overscan: bool = False):
         """Render a sequence of scenes given as HOST tensors (the batch_infer.py use case,
         batch_infer.py:103-143): generator over dicts with the keys of `render` ('triangles', 'texture',
         'mask', 'vn', 'c2w', 'fov'), yielding one pinned-host fp32 HDR tensor [B,V,H,W,3] per scene,
-        in order.  `resolution` is an int or (H, W) as in `render`.
+        in order.  `resolution` is an int or (H, W) and `overscan` as in `render`.
 
         The host->device copy of scene i+1 (218 MB of texture for 4096 triangles) runs on a copy
         stream while scene i is being rendered, and the device->host copy of image i overlaps scene
@@ -467,7 +489,7 @@ class RenderFormerRenderingPipeline:
             pending = upload(nxt) if nxt is not None else None  # overlaps with this scene's kernels
             main.wait_event(ev)
             img = self.render(d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], d["fov"],
-                              resolution=resolution, torch_dtype=torch_dtype)
+                              resolution=resolution, torch_dtype=torch_dtype, overscan=overscan)
             up.release(uslot, main)  # the staging slot may be overwritten once this render has consumed it
             if ldr is not None:
                 img = self.hdr_to_ldr(img, ldr)

@@ -74,9 +74,11 @@ def gemm(A: torch.Tensor, W: torch.Tensor, out: Optional[torch.Tensor] = None, *
          bias=None, res1=None, res2=None, out_act=None, row_map=None, epi=L.EPI_STORE, out_dtype=None,
          conv=None, w2=None, b2=None, lda=None, ldw=None, ldo=None, ldres=None, bn=0,
          in_sumsq=None, in_rscale=None, scale_dim=0, norm_dim=0, norm_eps=1e-6, out_rscale=None, out_sumsq=None,
-         out16=None, col_mul=None, aux_row_map=None, vt_out=None, vt_split=0, vt_rows_per_batch=0) -> torch.Tensor:
+         out16=None, col_mul=None, aux_row_map=None, vt_out=None, vt_split=0, vt_rows_per_batch=0,
+         crop=None) -> torch.Tensor:
     """out[M,N] = A[M,K] @ W[N,K]^T with fused epilogue.  `conv=(B,H,W,Cin)` switches A to NHWC 3x3
-    implicit GEMM.  Shapes default to the tensors' 2-D shapes."""
+    implicit GEMM.  Shapes default to the tensors' 2-D shapes.  `crop=(h, w, top, left)` (conv with a final
+    epilogue): only that window of the conv image is stored, as out [B, h, w, 3]."""
     _need_cuda(A, W)
     lib = L.load()
     a = L.GemmArgs()
@@ -98,7 +100,8 @@ def gemm(A: torch.Tensor, W: torch.Tensor, out: Optional[torch.Tensor] = None, *
     a.epi = epi
     if out is None and out_act is None and out16 is None:
         ncols = N // 2 if epi == L.EPI_SWIGLU else (3 if epi in (L.EPI_FINAL, L.EPI_FINAL_RAW) else N)
-        out = torch.empty((M, ncols), dtype=out_dtype or torch.float32, device=A.device)
+        rows = M if crop is None else conv[0] * crop[0] * crop[1]
+        out = torch.empty((rows, ncols), dtype=out_dtype or torch.float32, device=A.device)
     ref = out if out is not None else out_act
     a.out, a.out_act = _p(out), _p(out_act)
     if ref is not None:
@@ -131,6 +134,8 @@ def gemm(A: torch.Tensor, W: torch.Tensor, out: Optional[torch.Tensor] = None, *
     a.row_map = _p(row_map)
     a.w2, a.b2 = _p(w2), _p(b2)
     a.bn_override = bn
+    if crop is not None:
+        a.crop_h, a.crop_w, a.crop_top, a.crop_left = crop
     tag = f"M={M} N={N} K={K} epi={epi} conv={int(conv is not None)} out={a.out_dtype} res={int(res1 is not None)}"
     L.check(_timed("gemm", 2.0 * M * N * K, lambda: lib.rfb_gemm(C.byref(a), _stream()), tag), "rfb_gemm")
     return out if out is not None else (out_act if out_act is not None else out16)
@@ -273,6 +278,16 @@ def ray_tokens(fov_deg, out, *, n_views, resolution=None, height=None, width=Non
     H, W = _image_hw(resolution, height, width)
     L.check(_timed("ray_tokens", 0.0, lambda: L.load().rfb_ray_tokens_hw(fov_deg.data_ptr(), out.data_ptr(), n_views, H, W,
                                                                           _stream())), "rfb_ray_tokens_hw")
+    return out
+
+
+def ray_tokens_canvas(fov_deg, out, *, n_views, canvas_h, canvas_w, height, width, top, left):
+    """Pinhole ray-bundle patch tokens f16 [V, (canvas_h/8)*(canvas_w/8), 192] of a canvas holding the height x width
+    image at (top, left), with the image's camera (rfb_ray_tokens_canvas)."""
+    _need_cuda(fov_deg, out)
+    L.check(_timed("ray_tokens", 0.0, lambda: L.load().rfb_ray_tokens_canvas(
+        fov_deg.data_ptr(), out.data_ptr(), n_views, canvas_h, canvas_w, height, width, top, left, _stream())),
+        "rfb_ray_tokens_canvas")
     return out
 
 

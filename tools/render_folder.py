@@ -6,7 +6,7 @@ converter's `.h5` files (when h5py is installed); frames are named like the refe
 `<scene>_view_<v>.exr`, `<scene>_view_<v>.png`, `video.mp4`.
 
 usage: python tools/render_folder.py --scene_folder scenes/ --model_id /path/to/checkpoint_dir \
-           [--precision fp16|bf16|fp32] [--resolution 512] [--height H] [--width W] [--padding_length N] [--constant_texture]
+           [--precision fp16|bf16|fp32] [--resolution 512] [--height H] [--width W] [--overscan] [--padding_length N] [--constant_texture]
            [--tone_mapper none|pbr_neutral] [--save_video] [--output_dir out/] [--workers 4]
 
 Multi-GPU: launch with torchrun (`python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1
@@ -16,7 +16,10 @@ tools/render_folder.py ...`): the scene stage is row-sharded, every rank renders
 `--random_init NAME` renders with seeded random weights of a named architecture instead (smoke runs).
 
 `--height` / `--width` render H x W frames (e.g. 576 x 1024 for 16:9 video); either one replaces the matching side of
-the square `--resolution`.  The field of view of a scene spans the longer side."""
+the square `--resolution`.  The field of view of a scene spans the longer side.  Without `--overscan` the sides must be
+multiples of 64 for the swin models (8 for full attention); `--overscan` renders any size, e.g. `--height 1080 --width
+1920`, on the smallest canvas on that grid and writes only the requested frame (same camera, every pixel a real output
+of the model)."""
 import argparse
 import glob
 import os
@@ -42,6 +45,8 @@ def main(argv=None, _pipeline=None) -> int:
     ap.add_argument("--resolution", type=int, default=512)
     ap.add_argument("--height", type=int, default=None, help="image height in pixels (overrides --resolution)")
     ap.add_argument("--width", type=int, default=None, help="image width in pixels (overrides --resolution)")
+    ap.add_argument("--overscan", action="store_true",
+                    help="any frame size: render on the decoder's size grid and crop (e.g. --height 1080 --width 1920)")
     ap.add_argument("--padding_length", type=int, default=None, help="pad every scene to this many triangles on the device: one CUDA graph for all scenes")
     ap.add_argument("--constant_texture", action="store_true", help="upload 13 constants per triangle instead of the 32x32 texel grid")
     ap.add_argument("--tone_mapper", choices=["none", "pbr_neutral"], default="none")
@@ -99,7 +104,8 @@ def main(argv=None, _pipeline=None) -> int:
     # scene files are read / expanded / pinned two scenes ahead on a background thread
     paths = frame_io.render_to_files(pipe, frame_io.prefetch(scenes(), depth=2), names, out_dir, resolution=resolution, torch_dtype=dtype,
                                      tone_mapper=args.tone_mapper, pad_to=args.padding_length if world == 1 else None,
-                                     save_video=args.save_video, workers=args.workers, sharded=world > 1)
+                                     save_video=args.save_video, workers=args.workers, sharded=world > 1,
+                                     overscan=args.overscan)
     dt = time.time() - t0
     print(f"[rank {os.environ.get('RANK', '0')}] {len(paths)} frames of {len(files)} scenes -> {out_dir} in {dt:.2f} s "
           f"({len(paths) / dt:.1f} frames/s incl. file encoding)")
