@@ -254,6 +254,17 @@ int rfb_ray_tokens(const float* fov_deg, void* out, int n_views, int resolution,
  * is the case canvas == image, top = left = 0. */
 int rfb_ray_tokens_canvas(const float* fov_deg, void* out, int n_views, int canvas_h, int canvas_w, int height,
                           int width, int top, int left, rfb_stream_t stream);
+/* the same tokens for per-view pinhole intrinsics intr [V,4] = (fx, fy, cx, cy) on the device, in pixels of the
+ * height x width image the canvas holds at (top, left) (canvas == image: top = left = 0).  The centre of image pixel
+ * (row i, column j) is (j + 0.5, i + 0.5) (OpenCV K: add 0.5 to cx and cy); its ray is
+ * normalize(((u - cx) / fx, -(v - cy) / fy, -1)).  Argument checks as rfb_ray_tokens_canvas. */
+int rfb_ray_tokens_intrinsics(const float* intr, void* out, int n_views, int canvas_h, int canvas_w, int height,
+                              int width, int top, int left, rfb_stream_t stream);
+/* fov in degrees [V] -> intrinsics [V,4] = (f, f, width/2, height/2) of a height x width image, f = side / 2 /
+ * tan(fov / 2) with side = max(height, width) (fit 0, Blender's "Auto"; the focal length rfb_ray_tokens_canvas
+ * uses, bit for bit), width (fit 1, "Horizontal") or height (fit 2, "Vertical"). */
+int rfb_intrinsics_from_fov(const float* fov_deg, float* out, int n_views, int height, int width, int fit,
+                            rfb_stream_t stream);
 
 /* RayGenerator.forward (utils/ray_generator.py:13-50) for callers that want the ray map itself: c2w [V,4,4],
  * fov in RADIANS [V] -> rays_d fp32 [V, H, W, 3] (rotated by R(c2w), L2-normalised). */

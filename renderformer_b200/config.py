@@ -182,3 +182,32 @@ def overscan_grid(cfg: RenderFormerConfig, resolution) -> Tuple[Tuple[int, int],
     m = 64 if cfg.view_transformer_use_swin_attn else cfg.patch_size
     Hc, Wc = -(-H // m) * m, -(-W // m) * m
     return (H, W), (Hc, Wc), ((Hc - H) // 2, (Wc - W) // 2)
+
+
+def view_camera(c2w, fov=None, intrinsics=None):
+    """The camera of a render, as (keyword, tensor): ("fov", fov) or ("intrinsics", intrinsics).
+
+    Exactly one of `fov` (degrees [B, V, 1]) and `intrinsics` must be given.  `intrinsics` is a [B, V, 4] tensor
+    (fx, fy, cx, cy) in pixels of the returned H x W image, B and V matching c2w [B, V, 4, 4].  On the host its
+    values are checked too (all finite, fx and fy > 0); a device tensor is not read back, so that the render path
+    never waits for the device, and its values are the caller's responsibility.  Raises ValueError before anything
+    is launched."""
+    import torch
+    if (fov is None) == (intrinsics is None):
+        raise ValueError("pass exactly one of fov and intrinsics")
+    if intrinsics is None:
+        return "fov", fov
+    if not isinstance(intrinsics, torch.Tensor):
+        raise ValueError(f"intrinsics must be a torch.Tensor, got {type(intrinsics).__name__}")
+    want = (*tuple(c2w.shape[:2]), 4)
+    if tuple(intrinsics.shape) != want:
+        raise ValueError(f"intrinsics must be [B, V, 4] = {list(want)} to match c2w, got {list(intrinsics.shape)}")
+    if not intrinsics.is_floating_point():
+        raise ValueError(f"intrinsics must be a floating-point tensor, got {intrinsics.dtype}")
+    if intrinsics.device.type == "cpu":
+        k = intrinsics.double()
+        if not bool(torch.isfinite(k).all()):
+            raise ValueError("intrinsics must be finite")
+        if not bool((k[..., :2] > 0).all()):
+            raise ValueError("intrinsics: fx and fy must be positive")
+    return "intrinsics", intrinsics

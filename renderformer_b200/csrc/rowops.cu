@@ -496,6 +496,48 @@ __global__ void ray_tokens_kernel(const float* __restrict__ fov_deg, uint16_t* _
   out[t] = *reinterpret_cast<uint16_t*>(&h);
 }
 
+// The same tokens for V cameras with user-set pinhole intrinsics intr [V, 4] = (fx, fy, cx, cy) in pixels of the
+// H x W image the canvas holds at (top, left); pixel (row i, column j) of the image has its centre at (j + 0.5,
+// i + 0.5) and the ray normalize(((u - cx) / fx, -(v - cy) / fy, -1)).  With the intrinsics of rfb_intrinsics_from_fov
+// (auto fit) u - cx and (px + 0.5) - (left + W/2) are the same exact float, so the tokens equal ray_tokens_kernel's.
+// The normalisation repeats ray_tokens_kernel's expressions verbatim: moving them into a shared inline function
+// reschedules that kernel's compiled code.
+__global__ void ray_tokens_intrinsics_kernel(const float* __restrict__ intr, uint16_t* __restrict__ out, int V,
+                                             int Hc, int Wc, int top, int left) {
+  const int P = 8, Tw = Wc / P;
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const long long per_view = (long long)(Hc / P) * Tw * 192;
+  if (t >= V * per_view) return;
+  const int v = t / per_view;
+  const int rem = t % per_view;
+  const int tok = rem / 192, f = rem % 192;
+  const int c = f >> 6, p1 = (f >> 3) & 7, p2 = f & 7;
+  const int py = (tok / Tw) * P + p1, px = (tok % Tw) * P + p2;
+  const float fx = intr[4 * v], fy = intr[4 * v + 1], cx = intr[4 * v + 2], cy = intr[4 * v + 3];
+  const float u = (float)(px - left) + 0.5f, vv = (float)(py - top) + 0.5f;
+  const float dx = (u - cx) / fx;
+  const float dy = -(vv - cy) / fy;
+  const float inv = 1.0f / fmaxf(sqrtf(dx * dx + dy * dy + 1.f), 1e-12f);
+  const float val = (c == 0 ? dx : (c == 1 ? dy : -1.f)) * inv;
+  __half h = __float2half(val);
+  out[t] = *reinterpret_cast<uint16_t*>(&h);
+}
+
+// fov in degrees [V] -> intrinsics [V, 4] = (f, f, W/2, H/2) of an H x W image, the fov spanning the longer side
+// (fit 0, "auto": ray_tokens_kernel's own focal length, bit for bit), the width (1) or the height (2).
+__global__ void intrinsics_from_fov_kernel(const float* __restrict__ fov_deg, float* __restrict__ out, int V, int H,
+                                           int W, int fit) {
+  const int v = blockIdx.x * blockDim.x + threadIdx.x;
+  if (v >= V) return;
+  const float fov = fov_deg[v] / 180.f * 3.14159265358979323846f;
+  const int side = fit == 1 ? W : (fit == 2 ? H : max(H, W));
+  const float fl = pinhole_focal(side, side, fov);
+  out[4 * v] = fl;
+  out[4 * v + 1] = fl;
+  out[4 * v + 2] = W * 0.5f;
+  out[4 * v + 3] = H * 0.5f;
+}
+
 // explicit ray map [V, H, W, 3] fp32 -> patch tokens (same layout as ray_tokens_kernel): the model-level
 // entry RenderFormer.forward(..., rays_d, ...) (models/renderformer.py:171-206) hands the rays in
 __global__ void ray_map_tokens_kernel(const float* __restrict__ rays, uint16_t* __restrict__ out, int V, int H,
@@ -783,6 +825,25 @@ extern "C" int rfb_ray_tokens_canvas(const float* fov_deg, void* out, int n_view
   ray_tokens_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
       fov_deg, (uint16_t*)out, n_views, canvas_h, canvas_w, height, width, cx, cy);
   RFB_LAUNCHED("ray_tokens_kernel");
+}
+
+extern "C" int rfb_ray_tokens_intrinsics(const float* intr, void* out, int n_views, int canvas_h, int canvas_w,
+                                         int height, int width, int top, int left, rfb_stream_t stream) {
+  if (!intr || !out || n_views <= 0 || canvas_h <= 0 || canvas_w <= 0 || canvas_h % 8 || canvas_w % 8 ||
+      height <= 0 || width <= 0 || top < 0 || left < 0 || height > canvas_h - top || width > canvas_w - left)
+    return RFB_ERR_ARG;
+  const long long total = (long long)n_views * (canvas_h / 8) * (canvas_w / 8) * 192;
+  ray_tokens_intrinsics_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      intr, (uint16_t*)out, n_views, canvas_h, canvas_w, top, left);
+  RFB_LAUNCHED("ray_tokens_intrinsics_kernel");
+}
+
+extern "C" int rfb_intrinsics_from_fov(const float* fov_deg, float* out, int n_views, int height, int width, int fit,
+                                       rfb_stream_t stream) {
+  if (!fov_deg || !out || n_views <= 0 || height <= 0 || width <= 0 || fit < 0 || fit > 2) return RFB_ERR_ARG;
+  intrinsics_from_fov_kernel<<<(n_views + 127) / 128, 128, 0, (cudaStream_t)stream>>>(fov_deg, out, n_views, height,
+                                                                                      width, fit);
+  RFB_LAUNCHED("intrinsics_from_fov_kernel");
 }
 
 extern "C" int rfb_ray_tokens_hw(const float* fov_deg, void* out, int n_views, int height, int width,

@@ -24,6 +24,7 @@ import sys
 import torch
 import torch.distributed as dist
 
+from .config import view_camera
 from .engine import RowShard, SceneState
 
 
@@ -194,9 +195,9 @@ def gather_images(img: torch.Tensor, dst: int = 0, sizes: Optional[List[int]] = 
 
 
 @torch.no_grad()
-def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov, resolution=512, dst: Optional[int] = 0,
+def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov=None, resolution=512, dst: Optional[int] = 0,
                    texture_own_rows: bool = False, torch_dtype: torch.dtype = torch.float16, async_gather: bool = False,
-                   overscan: bool = False):
+                   overscan: bool = False, intrinsics=None):
     """`RenderFormerRenderingPipeline.render` on all ranks of the process group: every rank passes the
     SAME scene and the full camera list c2w [B,V,4,4] / fov [B,V,1]; the scene stage is row-sharded, each
     rank renders `view_slice(V)`, and the images are gathered on `dst` (returns [B,V,H,W,3] there and
@@ -205,27 +206,28 @@ def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov, resolution=512,
     CUDA-graph replay.  `async_gather` (one scene per call): the image gather is only enqueued and a
     GatherHandle is returned on every rank -- a caller rendering job after job lets the gather of job k
     travel over NVLink while the scene stage of job k+1 runs, and calls `handle.wait()` before using the
-    images (at the latest before the job after next).  `resolution`: an int or (H, W), and `overscan`, as in
-    `render`."""
+    images (at the latest before the job after next).  `resolution`: an int or (H, W), `overscan`, and the
+    camera (`fov` [B,V,1] or `intrinsics` [B,V,4], full lists, sliced per rank like c2w), as in `render`."""
     canvas, window, _ = pipe.view_geometry(resolution, overscan)
+    kind, cam = view_camera(c2w, fov, intrinsics)
     world, rank = _world()
     V = c2w.shape[1]
     mine = view_slice(V, world, rank)
-    c2w_l, fov_l = c2w[:, mine].contiguous(), fov[:, mine].contiguous()
+    c2w_l, cam_l = c2w[:, mine].contiguous(), cam[:, mine].contiguous()
     sh = row_shard()
     if world == 1:
-        img = pipe.render(triangles, texture, mask, vn, c2w_l, fov_l, resolution=resolution, torch_dtype=torch_dtype,
-                          overscan=overscan)
+        img = pipe.render(triangles, texture, mask, vn, c2w_l, resolution=resolution, torch_dtype=torch_dtype,
+                          overscan=overscan, **{kind: cam_l})
     else:
         from .model import operand_dtype
         eng = pipe.model.engine(operand_dtype(torch_dtype))
-        inputs = (triangles, texture, mask, vn, c2w_l, fov_l)
+        inputs = (triangles, texture, mask, vn, c2w_l, cam_l)
 
-        def run(tri, tex, msk, vnn, cw, fv):
+        def run(tri, tex, msk, vnn, cw, cm):
             st = eng.encode_scene(tri, tex, msk, vnn, shard=sh, texture_own_rows=texture_own_rows)
-            return pipe.render_views(st, cw, fv, resolution, overscan, _eager=True)
+            return pipe.render_views(st, cw, resolution=resolution, overscan=overscan, _eager=True, **{kind: cm})
         if pipe.cuda_graphs and all(t.is_cuda for t in inputs) and mine.stop > mine.start:
-            key = (("render_sharded", id(eng), rank, world, canvas, window, pipe.view_chunk, texture_own_rows) +
+            key = (("render_sharded", id(eng), rank, world, kind, canvas, window, pipe.view_chunk, texture_own_rows) +
                    pipe._sig(inputs))
             img = pipe._graph_entry(key, inputs, run)
         else:
@@ -253,7 +255,8 @@ def render_stream_sharded(pipe, scenes, resolution=512, ldr: Optional[str] = Non
     frames).  Uploads of scene i+1 and downloads of scene i overlap the kernels of the neighbouring scene.
 
     Yields (view_slice, pinned host tensor [B, V_rank, H, W, 3]) per scene; the buffer belongs to a ring of
-    three.  `resolution`: an int or (H, W), and `overscan`, as in `render`."""
+    three.  `resolution`: an int or (H, W), and `overscan`, as in `render`; a scene carries 'fov' or
+    'intrinsics', as in `render_stream`."""
     canvas, window, _ = pipe.view_geometry(resolution, overscan)
     dev = pipe.device
     world, rank = _world()
@@ -265,11 +268,12 @@ def render_stream_sharded(pipe, scenes, resolution=512, ldr: Optional[str] = Non
     up = UploadRing(dev, copy)
 
     def upload(sc):
+        kind, cam = view_camera(sc["c2w"], sc.get("fov"), sc.get("intrinsics"))
         V = sc["c2w"].shape[1]
         mine = view_slice(V, world, rank)
         N = sc["triangles"].shape[1]
         t0, t1 = eng.own_triangles(N, sh) if sh is not None else (0, N)
-        d, ev, slot = up.put({"c2w": sc["c2w"][:, mine], "fov": sc["fov"][:, mine], "triangles": sc["triangles"],
+        d, ev, slot = up.put({"c2w": sc["c2w"][:, mine], kind: cam[:, mine], "triangles": sc["triangles"],
                               "mask": sc["mask"], "vn": sc["vn"],
                               "texture": sc["texture"][:, t0:t1]})  # only this rank's rows of the texture
         return d, ev, mine, slot
@@ -289,18 +293,19 @@ def render_stream_sharded(pipe, scenes, resolution=512, ldr: Optional[str] = Non
         pending = upload(nxt) if nxt is not None else None
         t_1 = time.perf_counter()
         main.wait_event(ev)
+        kind = "intrinsics" if "intrinsics" in d else "fov"
         if sh is None:
-            img = pipe.render(d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], d["fov"], resolution=resolution,
-                              torch_dtype=torch_dtype, overscan=overscan)
+            img = pipe.render(d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], resolution=resolution,
+                              torch_dtype=torch_dtype, overscan=overscan, **{kind: d[kind]})
         else:
             # full camera list is not needed here: the slice was taken on the host
-            inputs = (d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], d["fov"])
+            inputs = (d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], d[kind])
 
-            def run(tri, tex, msk, vnn, cw, fv):
+            def run(tri, tex, msk, vnn, cw, cm):
                 st = eng.encode_scene(tri, tex, msk, vnn, shard=sh, texture_own_rows=True)
-                return pipe.render_views(st, cw, fv, resolution, overscan, _eager=True)
+                return pipe.render_views(st, cw, resolution=resolution, overscan=overscan, _eager=True, **{kind: cm})
             if pipe.cuda_graphs and mine.stop > mine.start:
-                key = ("stream_sharded", id(eng), rank, world, canvas, window, pipe.view_chunk) + pipe._sig(inputs)
+                key = ("stream_sharded", id(eng), rank, world, kind, canvas, window, pipe.view_chunk) + pipe._sig(inputs)
                 img = pipe._graph_entry(key, inputs, run)
             else:
                 img = run(*inputs)

@@ -605,7 +605,7 @@ class Engine:
                      resolution, taps: Optional[dict] = None, rays_d: Optional[torch.Tensor] = None,
                      tri_cam: Optional[torch.Tensor] = None, pos_cam: Optional[torch.Tensor] = None,
                      raw_log: bool = False, out: Optional[torch.Tensor] = None,
-                     window: Optional[tuple] = None) -> torch.Tensor:
+                     window: Optional[tuple] = None, intrinsics: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Render V views of scene `b` -> HDR fp32 [V,H,W,3]; `resolution` is an int (square) or (H, W)
         (config.view_grid).  Either cameras (c2w [V,4,4], fov_deg [V] or [V,1]; rays and camera-space triangles
         are derived on the device, fov spanning the longer image side) or, for the model-level entry
@@ -617,7 +617,9 @@ class Engine:
         writes the image into (a slice of the caller's result tensor: no concatenation afterwards).
         `window=(h, w, top, left)` (cameras only, config.overscan_grid): `resolution` is the canvas the model runs
         on, the cameras are those of the h x w image it holds at canvas pixel (top, left), and only that window is
-        stored: the result (and `out`) is [V, h, w, 3]."""
+        stored: the result (and `out`) is [V, h, w, 3].
+        `intrinsics` [V, 4] (fx, fy, cx, cy) in pixels of the returned image (the window, or the whole image) takes
+        the place of `fov_deg`: a pinhole camera with those focal lengths and that principal point."""
         cfg, dev = self.cfg, self.device
         explicit = rays_d is not None
         if explicit and tri_cam is None and pos_cam is None:
@@ -644,24 +646,32 @@ class Engine:
             x = self.ray_tokens(V, H, W, rays=rays)
         else:
             c2w = c2w.to(dev, torch.float32).contiguous()
-            fov = fov_deg.reshape(-1).to(dev, torch.float32).contiguous()
+            if intrinsics is not None:
+                fov, intr = None, intrinsics.reshape(V, 4).to(dev, torch.float32).contiguous()
+            else:
+                fov, intr = fov_deg.reshape(-1).to(dev, torch.float32).contiguous(), None
             pos = ops.positions(st.tri[b], st.mask_u8[b], c2w, self._e((V, Ntp, 9), torch.float32), n=N,
                                 n_reg=cfg.num_register_tokens, rows_out=Ntp, n_views=V)
-            x = self.ray_tokens(V, H, W, fov=fov, window=window)
+            x = self.ray_tokens(V, H, W, fov=fov, window=window, intrinsics=intr)
         feats = self.decoder_layers(st, b, x, pos, V, Hp, Wp, taps)
         return self._dpt(feats, V, Hp, Wp, raw_out=raw_log, out=out, window=window)
 
-    def ray_tokens(self, V: int, H: int, W: int, fov=None, rays=None, window=None):
+    def ray_tokens(self, V: int, H: int, W: int, fov=None, rays=None, window=None, intrinsics=None):
         """Ray-bundle patch tokens x fp32 [V*(H/8)*(W/8), dv], row-major patch grid: pinhole rays
         (utils/ray_generator.py:13-50) or an explicit ray map -> 8x8 patches -> ray_map_patch_token +
         RMSNorm(Linear)  (view_transformer.py:104-108).  `window=(h, w, top, left)`: H x W is a canvas and the
-        rays are those of the h x w camera whose image sits at (top, left)."""
+        rays are those of the h x w camera whose image sits at (top, left).  `intrinsics` fp32 [V, 4] (fx, fy, cx,
+        cy) in pixels of that image replaces `fov`."""
         w = self.w
         dv = self.cfg.view_transformer_latent_dim
         rows = V * (H // 8) * (W // 8)
         rt = self._e((rows, 192), torch.float16)
         if rays is not None:
             ops.ray_map_tokens(rays, rt, n_views=V, height=H, width=W)
+        elif intrinsics is not None:
+            h, w_, top, left = (H, W, 0, 0) if window is None else window
+            ops.ray_tokens_intrinsics(intrinsics, rt, n_views=V, canvas_h=H, canvas_w=W, height=h, width=w_, top=top,
+                                      left=left)
         elif window is not None:
             h, w_, top, left = window
             ops.ray_tokens_canvas(fov, rt, n_views=V, canvas_h=H, canvas_w=W, height=h, width=w_, top=top, left=left)

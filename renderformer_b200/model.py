@@ -14,7 +14,7 @@ from typing import Dict, Optional
 import torch
 from torch import nn
 
-from .config import RenderFormerConfig, overscan_grid, view_grid
+from .config import RenderFormerConfig, _size_pair, overscan_grid, view_camera, view_grid
 from . import lib as L
 from .engine import Engine, SceneState
 
@@ -310,16 +310,40 @@ class RenderFormerRenderingPipeline:
         return canvas, (None if canvas == hw else (*hw, top, left)), hw
 
     @torch.no_grad()
-    def render_views(self, state: SceneState, c2w, fov, resolution=512, overscan: bool = False,
-                     _eager: bool = False) -> torch.Tensor:
-        """View-dependent stage of `render` on an encoded scene -> HDR [B,V,H,W,3]; `resolution` and `overscan` as
-        in `render`."""
+    def intrinsics_from_fov(self, fov, resolution, fit: str = "auto") -> torch.Tensor:
+        """Pinhole intrinsics fp32 [B, V, 4] = (f, f, W/2, H/2) on the device for `render(..., intrinsics=...)`, from
+        fov [B, V, 1] (or [B, V]) in degrees and the H x W size of the RETURNED image (`resolution`: an int or
+        (H, W), any positive size).  `fit` is the side the fov spans, as Blender's camera sensor fit: "auto" (the
+        longer side: the camera `render(..., fov=...)` uses, to the bit), "horizontal" (the width) or "vertical"
+        (the height): f = side / 2 / tan(fov / 2)."""
+        from . import ops
+        H, W = _size_pair(resolution)
+        if fit not in ops.FITS:
+            raise ValueError(f"fit must be one of {sorted(ops.FITS)}, got {fit!r}")
+        if fov.dim() == 3 and fov.shape[-1] == 1:
+            fov = fov[..., 0]
+        if fov.dim() != 2:
+            raise ValueError(f"fov must be [B, V, 1] or [B, V], got {list(fov.shape)}")
+        f = fov.to(self.device, torch.float32).contiguous()
+        out = torch.empty((*f.shape, 4), dtype=torch.float32, device=self.device)
+        if f.numel():
+            ops.intrinsics_from_fov(f, out, n_views=f.numel(), height=H, width=W, fit=fit)
+        return out
+
+    @torch.no_grad()
+    def render_views(self, state: SceneState, c2w, fov=None, resolution=512, overscan: bool = False,
+                     intrinsics=None, _eager: bool = False) -> torch.Tensor:
+        """View-dependent stage of `render` on an encoded scene -> HDR [B,V,H,W,3]; `resolution`, `overscan` and the
+        camera (`fov` or `intrinsics`) as in `render`."""
         eng = self.model.engine(state.v_all.dtype)  # the operand format the scene state was built in
         canvas, window, hw = self.view_geometry(resolution, overscan)
-        if self.cuda_graphs and not _eager and getattr(state, "static", False) and c2w.is_cuda and fov.is_cuda:
+        kind, cam = view_camera(c2w, fov, intrinsics)
+        if self.cuda_graphs and not _eager and getattr(state, "static", False) and c2w.is_cuda and cam.is_cuda:
             # the graph reads the persistent state in place (no copy of the 300 MB of hoisted K / V)
-            return self._graph_entry(("views", id(eng), id(state), canvas, window, self.view_chunk) + self._sig((c2w, fov)),
-                                     (c2w, fov), lambda a, b: self.render_views(state, a, b, hw, overscan, _eager=True))
+            return self._graph_entry(("views", id(eng), id(state), kind, canvas, window, self.view_chunk) +
+                                     self._sig((c2w, cam)), (c2w, cam),
+                                     lambda a, k: self.render_views(state, a, resolution=hw, overscan=overscan,
+                                                                    _eager=True, **{kind: k}))
         B, V = c2w.shape[:2]
         if V == 0:  # a rank whose view slice is empty (fewer views than ranks)
             return torch.empty((B, 0, *hw, 3), dtype=torch.float32, device=self.device)
@@ -327,11 +351,15 @@ class RenderFormerRenderingPipeline:
         # every decoder pass writes its images straight into its slice of the result (no torch.cat afterwards); with
         # overscan its last conv stores only the window, so no canvas-sized image exists
         result = torch.empty((B, V, *hw, 3), dtype=torch.float32, device=self.device)
+
+        def job(b, v0):
+            s = slice(v0, v0 + self.view_chunk)
+            eng.render_views(state, b, c2w[b, s], None if fov is None else fov[b, s], canvas, out=result[b, s],
+                             window=window, intrinsics=None if intrinsics is None else intrinsics[b, s])
         n_str = min(self.view_streams, len(jobs))
         if n_str <= 1:
             for b, v0 in jobs:
-                eng.render_views(state, b, c2w[b, v0:v0 + self.view_chunk], fov[b, v0:v0 + self.view_chunk], canvas,
-                                 out=result[b, v0:v0 + self.view_chunk], window=window)
+                job(b, v0)
             return result
         dev = self.device
         while len(self._side_streams) < n_str:
@@ -344,8 +372,7 @@ class RenderFormerRenderingPipeline:
             if i < n_str:
                 side.wait_event(fork)
             with torch.cuda.stream(side):
-                eng.render_views(state, b, c2w[b, v0:v0 + self.view_chunk], fov[b, v0:v0 + self.view_chunk], canvas,
-                                 out=result[b, v0:v0 + self.view_chunk], window=window)
+                job(b, v0)
         for side in self._side_streams[:n_str]:
             ev = torch.cuda.Event()
             ev.record(side)
@@ -353,10 +380,10 @@ class RenderFormerRenderingPipeline:
         return result
 
     @torch.no_grad()
-    def render(self, triangles, texture, mask, vn, c2w, fov, resolution=512,
-               torch_dtype: torch.dtype = torch.float16, overscan: bool = False):
+    def render(self, triangles, texture, mask, vn, c2w, fov=None, resolution=512,
+               torch_dtype: torch.dtype = torch.float16, overscan: bool = False, intrinsics=None):
         """triangles [B,N,3,3], texture [B,N,13,32,32], mask [B,N] bool, vn [B,N,3,3], c2w [B,V,4,4],
-        fov [B,V,1] degrees -> HDR [B,V,H,W,3] fp32.
+        fov [B,V,1] degrees or intrinsics [B,V,4] -> HDR [B,V,H,W,3] fp32.
 
         `resolution` is an int (square H = W) or a (height, width) pair; sides must be multiples of 64 for the
         swin models and of 8 for full attention (config.view_grid, checked before any launch).  Camera: pinhole,
@@ -370,6 +397,16 @@ class RenderFormerRenderingPipeline:
         0.7 % more pixels at 1080p and 4K, 6.7 % at 720p.  A size already on the grid renders exactly as without
         overscan.
 
+        `intrinsics` [B,V,4] = (fx, fy, cx, cy) per view, in place of `fov`, renders calibrated or off-axis pinhole
+        cameras: separate focal lengths and any principal point, in pixels of the RETURNED H x W image (with
+        overscan too: the window, not the canvas).  The centre of pixel (row i, column j) is (j + 0.5, i + 0.5),
+        as in COLMAP; with an OpenCV K add 0.5 to cx and cy.  The ray of a pixel at (u, v) is
+        normalize(((u - cx) / fx, -(v - cy) / fy, -1)) in camera space (x right, y up, looking down -z), and the
+        `fov` camera is fx = fy = max(H, W) / 2 / tan(fov / 2), cx = W / 2, cy = H / 2
+        (`intrinsics_from_fov`; the render is then bit-identical to the `fov` one).  Exactly one of `fov` and
+        `intrinsics` is given (config.view_camera).  Intrinsics on the host are checked (finite, fx, fy > 0);
+        on the device they are used as they are, without a synchronising read-back.
+
         `texture` may also be [B,N,13]: per-triangle constants (what scene_processor/to_h5.py:37-66
         expands to the 32x32 texel grid with a fixed triangular mask).  The texture projection then
         uses texel-summed weights -- no 218 MB texel grid has to exist or be uploaded
@@ -382,11 +419,13 @@ class RenderFormerRenderingPipeline:
         Unlike the reference (:68) the caller's `texture` is not modified."""
         op = operand_dtype(torch_dtype)
         self.view_geometry(resolution, overscan)  # size errors before any launch
-        if self.cuda_graphs and all(t.is_cuda for t in (triangles, texture, mask, vn, c2w, fov)):
-            out = self._render_graphed((triangles, texture, mask, vn, c2w, fov), resolution, op, overscan)
+        kind, cam = view_camera(c2w, fov, intrinsics)
+        inputs = (triangles, texture, mask, vn, c2w, cam)
+        if self.cuda_graphs and all(t.is_cuda for t in inputs):
+            out = self._render_graphed(inputs, resolution, op, overscan, kind)
             return out if self.graph_static_outputs else out.clone()
         state = self.encode(triangles, texture, mask, vn, torch_dtype=op)
-        return self.render_views(state, c2w, fov, resolution, overscan)
+        return self.render_views(state, c2w, fov, resolution, overscan, intrinsics)
 
     def _graph_entry(self, key, inputs, fn):
         """Capture `fn(*static_inputs)` once per key, replay it with `inputs` copied into the static
@@ -420,13 +459,18 @@ class RenderFormerRenderingPipeline:
     def _sig(tensors):
         return tuple((tuple(t.shape), t.dtype) for t in tensors)
 
-    def _render_graphed(self, inputs, resolution, op: torch.dtype = torch.bfloat16, overscan: bool = False) -> torch.Tensor:
+    def _render_graphed(self, inputs, resolution, op: torch.dtype = torch.bfloat16, overscan: bool = False,
+                        camera: str = "fov") -> torch.Tensor:
+        """`inputs` = (triangles, texture, mask, vn, c2w, camera tensor); `camera` names the last: "fov" or
+        "intrinsics" (a static input of the graph either way, and part of its key)."""
         eng = self.model.engine(op)
         canvas, window, _ = self.view_geometry(resolution, overscan)
 
-        def run(tri, tex, mask, vn, c2w, fov):
-            return self.render_views(eng.encode_scene(tri, tex, mask, vn), c2w, fov, resolution, overscan, _eager=True)
-        return self._graph_entry(("render", id(eng), canvas, window, self.view_chunk) + self._sig(inputs), inputs, run)
+        def run(tri, tex, mask, vn, c2w, cam):
+            return self.render_views(eng.encode_scene(tri, tex, mask, vn), c2w, resolution=resolution,
+                                     overscan=overscan, _eager=True, **{camera: cam})
+        return self._graph_entry(("render", id(eng), camera, canvas, window, self.view_chunk) + self._sig(inputs),
+                                 inputs, run)
 
     def static_scene_state(self, B: int, N: int, torch_dtype: torch.dtype = torch.float16) -> SceneState:
         """The persistent SceneState of this shape (receive buffer of the NCCL broadcast on ranks that do
@@ -455,8 +499,8 @@ class RenderFormerRenderingPipeline:
                       ldr: Optional[str] = None, pad_to: Optional[int] = None, overscan: bool = False):
         """Render a sequence of scenes given as HOST tensors (the batch_infer.py use case,
         batch_infer.py:103-143): generator over dicts with the keys of `render` ('triangles', 'texture',
-        'mask', 'vn', 'c2w', 'fov'), yielding one pinned-host fp32 HDR tensor [B,V,H,W,3] per scene,
-        in order.  `resolution` is an int or (H, W) and `overscan` as in `render`.
+        'mask', 'vn', 'c2w', and 'fov' or 'intrinsics'), yielding one pinned-host fp32 HDR tensor [B,V,H,W,3] per
+        scene, in order.  `resolution` is an int or (H, W) and `overscan` as in `render`.
 
         The host->device copy of scene i+1 (218 MB of texture for 4096 triangles) runs on a copy
         stream while scene i is being rendered, and the device->host copy of image i overlaps scene
@@ -471,13 +515,14 @@ class RenderFormerRenderingPipeline:
         dev = self.device
         if dev.type != "cuda":
             raise L.RfbError("render_stream needs a CUDA device (there is no CPU fallback)")
-        keys = ("triangles", "texture", "mask", "vn", "c2w", "fov")
+        keys = ("triangles", "texture", "mask", "vn", "c2w")
         main = torch.cuda.current_stream(dev)
         copy = torch.cuda.Stream(dev)
         up = UploadRing(dev, copy)
 
         def upload(sc):
-            return up.put({k: sc[k] for k in keys}, pad_to=pad_to)
+            kind, _ = view_camera(sc["c2w"], sc.get("fov"), sc.get("intrinsics"))  # host checks before the copy
+            return up.put({k: sc[k] for k in keys + (kind,)}, pad_to=pad_to)
 
         it = iter(scenes)
         first = next(it, None)
@@ -488,8 +533,9 @@ class RenderFormerRenderingPipeline:
             nxt = next(it, None)
             pending = upload(nxt) if nxt is not None else None  # overlaps with this scene's kernels
             main.wait_event(ev)
-            img = self.render(d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], d["fov"],
-                              resolution=resolution, torch_dtype=torch_dtype, overscan=overscan)
+            img = self.render(d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], d.get("fov"),
+                              resolution=resolution, torch_dtype=torch_dtype, overscan=overscan,
+                              intrinsics=d.get("intrinsics"))
             up.release(uslot, main)  # the staging slot may be overwritten once this render has consumed it
             if ldr is not None:
                 img = self.hdr_to_ldr(img, ldr)

@@ -291,6 +291,31 @@ def ray_tokens_canvas(fov_deg, out, *, n_views, canvas_h, canvas_w, height, widt
     return out
 
 
+def ray_tokens_intrinsics(intr, out, *, n_views, canvas_h, canvas_w, height, width, top=0, left=0):
+    """Pinhole ray-bundle patch tokens f16 [V, (canvas_h/8)*(canvas_w/8), 192] from per-view intrinsics fp32 [V, 4] =
+    (fx, fy, cx, cy) in pixels of the height x width image the canvas holds at (top, left)
+    (rfb_ray_tokens_intrinsics)."""
+    _need_cuda(intr, out)
+    L.check(_timed("ray_tokens", 0.0, lambda: L.load().rfb_ray_tokens_intrinsics(
+        intr.data_ptr(), out.data_ptr(), n_views, canvas_h, canvas_w, height, width, top, left, _stream())),
+        "rfb_ray_tokens_intrinsics")
+    return out
+
+
+FITS = {"auto": 0, "horizontal": 1, "vertical": 2}
+
+
+def intrinsics_from_fov(fov_deg, out, *, n_views, height, width, fit="auto"):
+    """fov in degrees fp32 [V] -> intrinsics fp32 [V, 4] = (f, f, width/2, height/2), the fov spanning the longer side
+    ("auto"), the width ("horizontal") or the height ("vertical") (rfb_intrinsics_from_fov)."""
+    if fit not in FITS:
+        raise ValueError(f"fit must be one of {sorted(FITS)}, got {fit!r}")
+    _need_cuda(fov_deg, out)
+    L.check(_timed("intrinsics_from_fov", 0.0, lambda: L.load().rfb_intrinsics_from_fov(
+        fov_deg.data_ptr(), out.data_ptr(), n_views, height, width, FITS[fit], _stream())), "rfb_intrinsics_from_fov")
+    return out
+
+
 def ray_map_tokens(rays_d, out, *, n_views, resolution=None, height=None, width=None):
     """Explicit ray map fp32 [V, H, W, 3] -> patch tokens f16 [V, (H/8)*(W/8), 192] (rfb_ray_map_tokens_hw)."""
     _need_cuda(rays_d, out)
