@@ -260,6 +260,14 @@ int rfb_ray_tokens_canvas(const float* fov_deg, void* out, int n_views, int canv
  * normalize(((u - cx) / fx, -(v - cy) / fy, -1)).  Argument checks as rfb_ray_tokens_canvas. */
 int rfb_ray_tokens_intrinsics(const float* intr, void* out, int n_views, int canvas_h, int canvas_w, int height,
                               int width, int top, int left, rfb_stream_t stream);
+/* the same tokens for lens-distorted cameras: intrinsics as rfb_ray_tokens_intrinsics, and per view lens coefficients
+ * on the device, dist [V,8] = (k1, k2, p1, p2, k3, k4, k5, k6) for lens 0 (OpenCV, COLMAP FULL_OPENCV) or dist [V,4]
+ * = (k1, k2, k3, k4) for lens 1 (OpenCV fisheye, COLMAP OPENCV_FISHEYE).  Each pixel's distorted normalized
+ * coordinates ((u - cx) / fx, (v - cy) / fy) are undistorted by Newton's method; the ray is normalize((x, -y, -1))
+ * (lens 0) or (sin t * xd / rd, -sin t * yd / rd, -cos t) (lens 1).  Coefficients that do not invert give finite
+ * tokens, not correct ones.  Argument checks as rfb_ray_tokens_intrinsics, and lens must be 0 or 1. */
+int rfb_ray_tokens_lens(const float* intr, const float* dist, int lens, void* out, int n_views, int canvas_h,
+                        int canvas_w, int height, int width, int top, int left, rfb_stream_t stream);
 /* fov in degrees [V] -> intrinsics [V,4] = (f, f, width/2, height/2) of a height x width image, f = side / 2 /
  * tan(fov / 2) with side = max(height, width) (fit 0, Blender's "Auto"; the focal length rfb_ray_tokens_canvas
  * uses, bit for bit), width (fit 1, "Horizontal") or height (fit 2, "Vertical"). */

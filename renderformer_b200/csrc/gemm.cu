@@ -1309,5 +1309,5 @@ extern "C" int rfb_gemm(const rfb_gemm_args* a, rfb_stream_t stream_) {
   }
 }
 
-extern "C" int rfb_version(void) { return 101; }
+extern "C" int rfb_version(void) { return 102; }
 extern "C" long long rfb_launch_count(void) { return g_launch_count.load(); }

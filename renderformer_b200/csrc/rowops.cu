@@ -523,6 +523,108 @@ __global__ void ray_tokens_intrinsics_kernel(const float* __restrict__ intr, uin
   out[t] = *reinterpret_cast<uint16_t*>(&h);
 }
 
+// The same tokens for V lens-distorted cameras: intrinsics intr [V, 4] as ray_tokens_intrinsics_kernel, and per view
+// dist [V, 8] = (k1, k2, p1, p2, k3, k4, k5, k6) (lens 0, OpenCV / COLMAP FULL_OPENCV) or dist [V, 4] = (k1, k2, k3,
+// k4) (lens 1, OpenCV fisheye / COLMAP OPENCV_FISHEYE).  A pixel's distorted normalized coordinates are
+// (xd, yd) = ((u - cx) / fx, (v - cy) / fy) in COLMAP's axes (y down).
+//   lens 0: Newton's method with the analytic 2x2 Jacobian, from (xd, yd), solves
+//           xd = x g + 2 p1 x y + p2 (r2 + 2 x^2),  yd = y g + p1 (r2 + 2 y^2) + 2 p2 x y,
+//           g = (1 + k1 r2 + k2 r2^2 + k3 r2^3) / (1 + k4 r2 + k5 r2^2 + k6 r2^3),  r2 = x^2 + y^2,
+//           and the ray is normalize((x, -y, -1)).
+//   lens 1: 1-D Newton in fp64 from theta = rd = |(xd, yd)| solves rd = theta (1 + k1 t2 + k2 t2^2 + k3 t2^3 + k4 t2^4),
+//           t2 = theta^2, and the ray is (sin theta xd / rd, -sin theta yd / rd, -cos theta) ((0, 0, -1) at rd = 0).
+// One thread per pixel: the solve is ~20x the pinhole's arithmetic, so it runs once and writes the three channels.
+// Threads are ordered (view, token, p1, p2) so that a warp stores 64 contiguous bytes per channel.  With all
+// coefficients zero the first residual is exactly 0, so (x, -y) are ray_tokens_intrinsics_kernel's (dx, dy) and the
+// normalisation below repeats its expressions, with the contraction its SASS shows (fma(dx, dx, dy * dy) + 1) pinned:
+// the tokens are that kernel's, bit for bit.  A pixel that does not converge keeps its last iterate; a non-finite one
+// (coefficients that fold or a vanishing denominator, which the host checks only for host tensors) falls back to the
+// pinhole ray normalize((xd, -yd, -1)), so no token is ever non-finite for finite intrinsics.
+__global__ void ray_tokens_lens_kernel(const float* __restrict__ intr, const float* __restrict__ dist, int lens,
+                                       uint16_t* __restrict__ out, int V, int Hc, int Wc, int top, int left) {
+  const int P = 8, Tw = Wc / P;
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const long long per_view = (long long)Hc * Wc;
+  if (t >= V * per_view) return;
+  const int v = t / per_view;
+  const int rem = t % per_view;
+  const int tok = rem / 64, p1 = (rem >> 3) & 7, p2 = rem & 7;
+  const int py = (tok / Tw) * P + p1, px = (tok % Tw) * P + p2;
+  const float fx = intr[4 * v], fy = intr[4 * v + 1], cx = intr[4 * v + 2], cy = intr[4 * v + 3];
+  const float u = (float)(px - left) + 0.5f, vv = (float)(py - top) + 0.5f;
+  const float xd = (u - cx) / fx;
+  const float yd = (vv - cy) / fy;
+  float o0, o1, o2;
+  bool pinhole = true;
+  if (lens == 0) {
+    const float* k = dist + 8 * v;
+    const float k1 = k[0], k2 = k[1], q1 = k[2], q2 = k[3], k3 = k[4], k4 = k[5], k5 = k[6], k6 = k[7];
+    float x = xd, y = yd;
+    for (int it = 0; it < 20; ++it) {
+      const float x2 = x * x, y2 = y * y, xy = x * y, r2 = x2 + y2;
+      const float num = 1.f + r2 * (k1 + r2 * (k2 + r2 * k3));
+      const float den = 1.f + r2 * (k4 + r2 * (k5 + r2 * k6));
+      const float g = num / den;
+      const float gp = ((k1 + r2 * (2.f * k2 + r2 * 3.f * k3)) * den - num * (k4 + r2 * (2.f * k5 + r2 * 3.f * k6))) /
+                       (den * den);  // dg / dr2
+      const float ex = x * g + 2.f * q1 * xy + q2 * (r2 + 2.f * x2) - xd;
+      const float ey = y * g + q1 * (r2 + 2.f * y2) + 2.f * q2 * xy - yd;
+      const float jxx = g + 2.f * x2 * gp + 2.f * q1 * y + 6.f * q2 * x;
+      const float jyy = g + 2.f * y2 * gp + 6.f * q1 * y + 2.f * q2 * x;
+      const float jxy = 2.f * xy * gp + 2.f * q1 * x + 2.f * q2 * y;
+      const float det = jxx * jyy - jxy * jxy;
+      const float sx = (jyy * ex - jxy * ey) / det, sy = (jxx * ey - jxy * ex) / det;
+      x -= sx;
+      y -= sy;
+      if (!(fabsf(sx) + fabsf(sy) > 1e-7f * (1.f + fabsf(x) + fabsf(y)))) break;  // converged, or NaN
+    }
+    if (isfinite(x) && isfinite(y)) {
+      const float dx = x;
+      const float dy = -y;
+      const float inv = 1.0f / fmaxf(sqrtf(__fadd_rn(__fmaf_rn(dx, dx, __fmul_rn(dy, dy)), 1.f)), 1e-12f);
+      o0 = dx * inv;
+      o1 = dy * inv;
+      o2 = -1.f * inv;
+      pinhole = false;
+    }
+  } else {
+    // in fp64: -cos theta crosses zero at 90 degrees, and near there an fp32 theta (or fp32 (xd, yd)) cannot resolve it
+    // to an fp16 ulp of the token
+    const float* k = dist + 4 * v;
+    const double k1 = k[0], k2 = k[1], k3 = k[2], k4 = k[3];
+    const double x = ((double)u - cx) / fx, y = ((double)vv - cy) / fy;
+    const double rd = sqrt(x * x + y * y);
+    double th = rd;
+    for (int it = 0; it < 20; ++it) {
+      const double t2 = th * th;
+      const double poly = 1.0 + t2 * (k1 + t2 * (k2 + t2 * (k3 + t2 * k4)));
+      const double dpoly = 1.0 + t2 * (3.0 * k1 + t2 * (5.0 * k2 + t2 * (7.0 * k3 + t2 * 9.0 * k4)));
+      const double s = (th * poly - rd) / dpoly;
+      th -= s;
+      if (!(fabs(s) > 1e-12 * (1.0 + th))) break;  // converged (the next step would be ~1e-24), or NaN
+    }
+    if (isfinite(th)) {
+      double sn, cs;
+      sincos(th, &sn, &cs);
+      const double q = rd > 0.0 ? sn / rd : 0.0;
+      o0 = (float)(q * x);
+      o1 = (float)(-q * y);
+      o2 = rd > 0.0 ? (float)-cs : -1.f;
+      pinhole = false;
+    }
+  }
+  if (pinhole) {
+    const float inv = 1.0f / fmaxf(sqrtf(xd * xd + yd * yd + 1.f), 1e-12f);
+    o0 = xd * inv;
+    o1 = -yd * inv;
+    o2 = -inv;
+  }
+  uint16_t* o = out + ((long long)v * (Hc / P) * Tw + tok) * 192 + p1 * 8 + p2;
+  o[0] = __half_as_ushort(__float2half(o0));
+  o[64] = __half_as_ushort(__float2half(o1));
+  o[128] = __half_as_ushort(__float2half(o2));
+}
+
 // fov in degrees [V] -> intrinsics [V, 4] = (f, f, W/2, H/2) of an H x W image, the fov spanning the longer side
 // (fit 0, "auto": ray_tokens_kernel's own focal length, bit for bit), the width (1) or the height (2).
 __global__ void intrinsics_from_fov_kernel(const float* __restrict__ fov_deg, float* __restrict__ out, int V, int H,
@@ -836,6 +938,19 @@ extern "C" int rfb_ray_tokens_intrinsics(const float* intr, void* out, int n_vie
   ray_tokens_intrinsics_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
       intr, (uint16_t*)out, n_views, canvas_h, canvas_w, top, left);
   RFB_LAUNCHED("ray_tokens_intrinsics_kernel");
+}
+
+extern "C" int rfb_ray_tokens_lens(const float* intr, const float* dist, int lens, void* out, int n_views,
+                                   int canvas_h, int canvas_w, int height, int width, int top, int left,
+                                   rfb_stream_t stream) {
+  if (!intr || !dist || !out || lens < 0 || lens > 1 || n_views <= 0 || canvas_h <= 0 || canvas_w <= 0 ||
+      canvas_h % 8 || canvas_w % 8 || height <= 0 || width <= 0 || top < 0 || left < 0 || height > canvas_h - top ||
+      width > canvas_w - left)
+    return RFB_ERR_ARG;
+  const long long total = (long long)n_views * canvas_h * canvas_w;  // one thread per pixel
+  ray_tokens_lens_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      intr, dist, lens, (uint16_t*)out, n_views, canvas_h, canvas_w, top, left);
+  RFB_LAUNCHED("ray_tokens_lens_kernel");
 }
 
 extern "C" int rfb_intrinsics_from_fov(const float* fov_deg, float* out, int n_views, int height, int width, int fit,

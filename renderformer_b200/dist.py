@@ -24,7 +24,7 @@ import sys
 import torch
 import torch.distributed as dist
 
-from .config import view_camera
+from .config import camera_kwargs, view_camera
 from .engine import RowShard, SceneState
 
 
@@ -197,7 +197,7 @@ def gather_images(img: torch.Tensor, dst: int = 0, sizes: Optional[List[int]] = 
 @torch.no_grad()
 def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov=None, resolution=512, dst: Optional[int] = 0,
                    texture_own_rows: bool = False, torch_dtype: torch.dtype = torch.float16, async_gather: bool = False,
-                   overscan: bool = False, intrinsics=None):
+                   overscan: bool = False, intrinsics=None, distortion=None, lens: str = "opencv"):
     """`RenderFormerRenderingPipeline.render` on all ranks of the process group: every rank passes the
     SAME scene and the full camera list c2w [B,V,4,4] / fov [B,V,1]; the scene stage is row-sharded, each
     rank renders `view_slice(V)`, and the images are gathered on `dst` (returns [B,V,H,W,3] there and
@@ -207,9 +207,10 @@ def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov=None, resolution
     GatherHandle is returned on every rank -- a caller rendering job after job lets the gather of job k
     travel over NVLink while the scene stage of job k+1 runs, and calls `handle.wait()` before using the
     images (at the latest before the job after next).  `resolution`: an int or (H, W), `overscan`, and the
-    camera (`fov` [B,V,1] or `intrinsics` [B,V,4], full lists, sliced per rank like c2w), as in `render`."""
+    camera (`fov` [B,V,1] or `intrinsics` [B,V,4] with the optional `distortion` [B,V,n] of `lens`, full lists,
+    sliced per rank like c2w), as in `render`."""
     canvas, window, _ = pipe.view_geometry(resolution, overscan)
-    kind, cam = view_camera(c2w, fov, intrinsics)
+    kind, cam = view_camera(c2w, fov, intrinsics, distortion, lens, canvas, window)
     world, rank = _world()
     V = c2w.shape[1]
     mine = view_slice(V, world, rank)
@@ -217,7 +218,7 @@ def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov=None, resolution
     sh = row_shard()
     if world == 1:
         img = pipe.render(triangles, texture, mask, vn, c2w_l, resolution=resolution, torch_dtype=torch_dtype,
-                          overscan=overscan, **{kind: cam_l})
+                          overscan=overscan, **camera_kwargs(kind, cam_l))
     else:
         from .model import operand_dtype
         eng = pipe.model.engine(operand_dtype(torch_dtype))
@@ -225,7 +226,8 @@ def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov=None, resolution
 
         def run(tri, tex, msk, vnn, cw, cm):
             st = eng.encode_scene(tri, tex, msk, vnn, shard=sh, texture_own_rows=texture_own_rows)
-            return pipe.render_views(st, cw, resolution=resolution, overscan=overscan, _eager=True, **{kind: cm})
+            return pipe.render_views(st, cw, resolution=resolution, overscan=overscan, _eager=True,
+                                     **camera_kwargs(kind, cm))
         if pipe.cuda_graphs and all(t.is_cuda for t in inputs) and mine.stop > mine.start:
             key = (("render_sharded", id(eng), rank, world, kind, canvas, window, pipe.view_chunk, texture_own_rows) +
                    pipe._sig(inputs))
@@ -247,7 +249,7 @@ def render_sharded(pipe, triangles, texture, mask, vn, c2w, fov=None, resolution
 
 @torch.no_grad()
 def render_stream_sharded(pipe, scenes, resolution=512, ldr: Optional[str] = None,
-                          torch_dtype: torch.dtype = torch.float16, overscan: bool = False):
+                          torch_dtype: torch.dtype = torch.float16, overscan: bool = False, lens: str = "opencv"):
     """Multi-GPU counterpart of `RenderFormerRenderingPipeline.render_stream`: every rank iterates the SAME
     sequence of host scene dicts (keys of `render`).  Each rank uploads the geometry and only ITS OWN
     rows of the texture (1/world of the 218 MB), the scene stage runs row-sharded, each rank renders its
@@ -256,7 +258,7 @@ def render_stream_sharded(pipe, scenes, resolution=512, ldr: Optional[str] = Non
 
     Yields (view_slice, pinned host tensor [B, V_rank, H, W, 3]) per scene; the buffer belongs to a ring of
     three.  `resolution`: an int or (H, W), and `overscan`, as in `render`; a scene carries 'fov' or
-    'intrinsics', as in `render_stream`."""
+    'intrinsics' (and optionally 'distortion' of the model `lens`), as in `render_stream`."""
     canvas, window, _ = pipe.view_geometry(resolution, overscan)
     dev = pipe.device
     world, rank = _world()
@@ -268,7 +270,8 @@ def render_stream_sharded(pipe, scenes, resolution=512, ldr: Optional[str] = Non
     up = UploadRing(dev, copy)
 
     def upload(sc):
-        kind, cam = view_camera(sc["c2w"], sc.get("fov"), sc.get("intrinsics"))
+        kind, cam = view_camera(sc["c2w"], sc.get("fov"), sc.get("intrinsics"), sc.get("distortion"), lens, canvas,
+                                window)
         V = sc["c2w"].shape[1]
         mine = view_slice(V, world, rank)
         N = sc["triangles"].shape[1]
@@ -276,7 +279,7 @@ def render_stream_sharded(pipe, scenes, resolution=512, ldr: Optional[str] = Non
         d, ev, slot = up.put({"c2w": sc["c2w"][:, mine], kind: cam[:, mine], "triangles": sc["triangles"],
                               "mask": sc["mask"], "vn": sc["vn"],
                               "texture": sc["texture"][:, t0:t1]})  # only this rank's rows of the texture
-        return d, ev, mine, slot
+        return kind, d, ev, mine, slot
 
     import os
     import sys
@@ -288,22 +291,22 @@ def render_stream_sharded(pipe, scenes, resolution=512, ldr: Optional[str] = Non
     ring, rslot, prev = [None, None, None], 0, None
     while pending is not None:
         t_0 = time.perf_counter()
-        d, ev, mine, slot = pending
+        kind, d, ev, mine, slot = pending
         nxt = next(it, None)
         pending = upload(nxt) if nxt is not None else None
         t_1 = time.perf_counter()
         main.wait_event(ev)
-        kind = "intrinsics" if "intrinsics" in d else "fov"
         if sh is None:
             img = pipe.render(d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], resolution=resolution,
-                              torch_dtype=torch_dtype, overscan=overscan, **{kind: d[kind]})
+                              torch_dtype=torch_dtype, overscan=overscan, **camera_kwargs(kind, d[kind]))
         else:
             # full camera list is not needed here: the slice was taken on the host
             inputs = (d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], d[kind])
 
             def run(tri, tex, msk, vnn, cw, cm):
                 st = eng.encode_scene(tri, tex, msk, vnn, shard=sh, texture_own_rows=True)
-                return pipe.render_views(st, cw, resolution=resolution, overscan=overscan, _eager=True, **{kind: cm})
+                return pipe.render_views(st, cw, resolution=resolution, overscan=overscan, _eager=True,
+                                         **camera_kwargs(kind, cm))
             if pipe.cuda_graphs and mine.stop > mine.start:
                 key = ("stream_sharded", id(eng), rank, world, kind, canvas, window, pipe.view_chunk) + pipe._sig(inputs)
                 img = pipe._graph_entry(key, inputs, run)

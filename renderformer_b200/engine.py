@@ -605,7 +605,8 @@ class Engine:
                      resolution, taps: Optional[dict] = None, rays_d: Optional[torch.Tensor] = None,
                      tri_cam: Optional[torch.Tensor] = None, pos_cam: Optional[torch.Tensor] = None,
                      raw_log: bool = False, out: Optional[torch.Tensor] = None,
-                     window: Optional[tuple] = None, intrinsics: Optional[torch.Tensor] = None) -> torch.Tensor:
+                     window: Optional[tuple] = None, intrinsics: Optional[torch.Tensor] = None,
+                     distortion: Optional[torch.Tensor] = None, lens: str = "opencv") -> torch.Tensor:
         """Render V views of scene `b` -> HDR fp32 [V,H,W,3]; `resolution` is an int (square) or (H, W)
         (config.view_grid).  Either cameras (c2w [V,4,4], fov_deg [V] or [V,1]; rays and camera-space triangles
         are derived on the device, fov spanning the longer image side) or, for the model-level entry
@@ -619,7 +620,9 @@ class Engine:
         on, the cameras are those of the h x w image it holds at canvas pixel (top, left), and only that window is
         stored: the result (and `out`) is [V, h, w, 3].
         `intrinsics` [V, 4] (fx, fy, cx, cy) in pixels of the returned image (the window, or the whole image) takes
-        the place of `fov_deg`: a pinhole camera with those focal lengths and that principal point."""
+        the place of `fov_deg`: a pinhole camera with those focal lengths and that principal point.  `distortion` (with
+        `intrinsics`) makes it a lens-distorted camera: [V, 8] coefficients of lens "opencv" or [V, 4] of "fisheye"
+        (config.view_camera's padded form)."""
         cfg, dev = self.cfg, self.device
         explicit = rays_d is not None
         if explicit and tri_cam is None and pos_cam is None:
@@ -650,18 +653,22 @@ class Engine:
                 fov, intr = None, intrinsics.reshape(V, 4).to(dev, torch.float32).contiguous()
             else:
                 fov, intr = fov_deg.reshape(-1).to(dev, torch.float32).contiguous(), None
+            if distortion is not None:
+                distortion = distortion.reshape(V, -1).to(dev, torch.float32).contiguous()
             pos = ops.positions(st.tri[b], st.mask_u8[b], c2w, self._e((V, Ntp, 9), torch.float32), n=N,
                                 n_reg=cfg.num_register_tokens, rows_out=Ntp, n_views=V)
-            x = self.ray_tokens(V, H, W, fov=fov, window=window, intrinsics=intr)
+            x = self.ray_tokens(V, H, W, fov=fov, window=window, intrinsics=intr, distortion=distortion, lens=lens)
         feats = self.decoder_layers(st, b, x, pos, V, Hp, Wp, taps)
         return self._dpt(feats, V, Hp, Wp, raw_out=raw_log, out=out, window=window)
 
-    def ray_tokens(self, V: int, H: int, W: int, fov=None, rays=None, window=None, intrinsics=None):
+    def ray_tokens(self, V: int, H: int, W: int, fov=None, rays=None, window=None, intrinsics=None, distortion=None,
+                   lens: str = "opencv"):
         """Ray-bundle patch tokens x fp32 [V*(H/8)*(W/8), dv], row-major patch grid: pinhole rays
         (utils/ray_generator.py:13-50) or an explicit ray map -> 8x8 patches -> ray_map_patch_token +
         RMSNorm(Linear)  (view_transformer.py:104-108).  `window=(h, w, top, left)`: H x W is a canvas and the
         rays are those of the h x w camera whose image sits at (top, left).  `intrinsics` fp32 [V, 4] (fx, fy, cx,
-        cy) in pixels of that image replaces `fov`."""
+        cy) in pixels of that image replaces `fov`, and `distortion` fp32 [V, 8] ("opencv") or [V, 4] ("fisheye") adds
+        the `lens` model to it."""
         w = self.w
         dv = self.cfg.view_transformer_latent_dim
         rows = V * (H // 8) * (W // 8)
@@ -670,8 +677,12 @@ class Engine:
             ops.ray_map_tokens(rays, rt, n_views=V, height=H, width=W)
         elif intrinsics is not None:
             h, w_, top, left = (H, W, 0, 0) if window is None else window
-            ops.ray_tokens_intrinsics(intrinsics, rt, n_views=V, canvas_h=H, canvas_w=W, height=h, width=w_, top=top,
-                                      left=left)
+            if distortion is not None:
+                ops.ray_tokens_lens(intrinsics, distortion, rt, lens=lens, n_views=V, canvas_h=H, canvas_w=W, height=h,
+                                    width=w_, top=top, left=left)
+            else:
+                ops.ray_tokens_intrinsics(intrinsics, rt, n_views=V, canvas_h=H, canvas_w=W, height=h, width=w_,
+                                          top=top, left=left)
         elif window is not None:
             h, w_, top, left = window
             ops.ray_tokens_canvas(fov, rt, n_views=V, canvas_h=H, canvas_w=W, height=h, width=w_, top=top, left=left)

@@ -455,14 +455,14 @@ def prefetch(iterable: Iterable, depth: int = 2):
 def render_to_files(pipeline, scenes: Iterable[dict], names: Sequence[str], out_dir: str, resolution=512,
                     torch_dtype=None, tone_mapper: str = "none", pad_to: Optional[int] = None,
                     save_video: bool = False, workers: int = 4, fps: int = 24, sharded: bool = False,
-                    overscan: bool = False) -> List[str]:
+                    overscan: bool = False, lens: str = "opencv") -> List[str]:
     """The batch_infer.py loop (batch_infer.py:122-172) with nothing serialised behind the renderer: `scenes`
     (host tensors, the keys of `render`) go through `pipeline.render_stream` (upload of scene i+1 and download
     of image i-1 overlap the kernels of scene i) and every frame is handed to a `FrameWriter`.  Files are
     named like the reference's: `{name}_view_{v}.exr`, `{name}_view_{v}.png`, `video.mp4`.  `names[i]` belongs
     to the i-th scene (a scene dict holding B > 1 scenes takes B consecutive names).  Returns the frame paths
-    (without extension) this process wrote, in order.  `resolution` is an int or (H, W), and `overscan` (any size,
-    rendered on the decoder's grid and cropped), as in `render`.
+    (without extension) this process wrote, in order.  `resolution` is an int or (H, W), `overscan` (any size,
+    rendered on the decoder's grid and cropped), and `lens` (the model of the scenes' 'distortion'), as in `render`.
 
     `sharded=True` (one process per GPU, `torch.distributed` initialised): every rank iterates the SAME scenes
     through `dist.render_stream_sharded` -- scene stage row-sharded, each rank renders and WRITES its own slice
@@ -471,6 +471,8 @@ def render_to_files(pipeline, scenes: Iterable[dict], names: Sequence[str], out_
     kw = {} if torch_dtype is None else {"torch_dtype": torch_dtype}
     if overscan:
         kw["overscan"] = True
+    if lens != "opencv":
+        kw["lens"] = lens
     names = list(names)
     rank, world = 0, 1
     if sharded:

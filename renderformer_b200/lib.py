@@ -71,7 +71,7 @@ class AttnArgs(C.Structure):
 SYMBOLS = [
     "rfb_version", "rfb_launch_count", "rfb_gemm", "rfb_attention", "rfb_attention_ws_bytes", "rfb_rmsnorm", "rfb_rowstat", "rfb_qknorm_rope", "rfb_qknorm_rope_table", "rfb_qkv_post",
     "rfb_token_assemble", "rfb_texture_prep", "rfb_texture_const_prep", "rfb_vn_encode", "rfb_ray_tokens", "rfb_ray_map_tokens", "rfb_ray_map", "rfb_ray_tokens_hw",
-    "rfb_ray_tokens_canvas", "rfb_ray_tokens_intrinsics", "rfb_intrinsics_from_fov", "rfb_ray_map_tokens_hw", "rfb_ray_map_hw", "rfb_positions",
+    "rfb_ray_tokens_canvas", "rfb_ray_tokens_intrinsics", "rfb_ray_tokens_lens", "rfb_intrinsics_from_fov", "rfb_ray_map_tokens_hw", "rfb_ray_map_hw", "rfb_positions",
     "rfb_pack_mask", "rfb_cast", "rfb_transpose16", "rfb_pixel_shuffle", "rfb_im2col_s2", "rfb_upsample_bilinear", "rfb_ldr_quantize",
 ]
 
@@ -111,6 +111,7 @@ def load() -> C.CDLL:
         "rfb_ray_tokens_hw": [p, p, i, i, i, p],
         "rfb_ray_tokens_canvas": [p, p, i, i, i, i, i, i, i, p],
         "rfb_ray_tokens_intrinsics": [p, p, i, i, i, i, i, i, i, p],
+        "rfb_ray_tokens_lens": [p, p, i, p, i, i, i, i, i, i, i, p],
         "rfb_intrinsics_from_fov": [p, p, i, i, i, i, p],
         "rfb_positions": [p, p, p, p, i, i, i, i, p],
         "rfb_pack_mask": [p, p, i, i, i, i, p],

@@ -14,7 +14,7 @@ from typing import Dict, Optional
 import torch
 from torch import nn
 
-from .config import RenderFormerConfig, _size_pair, overscan_grid, view_camera, view_grid
+from .config import RenderFormerConfig, _size_pair, camera_kwargs, overscan_grid, view_camera, view_grid
 from . import lib as L
 from .engine import Engine, SceneState
 
@@ -332,18 +332,18 @@ class RenderFormerRenderingPipeline:
 
     @torch.no_grad()
     def render_views(self, state: SceneState, c2w, fov=None, resolution=512, overscan: bool = False,
-                     intrinsics=None, _eager: bool = False) -> torch.Tensor:
+                     intrinsics=None, distortion=None, lens: str = "opencv", _eager: bool = False) -> torch.Tensor:
         """View-dependent stage of `render` on an encoded scene -> HDR [B,V,H,W,3]; `resolution`, `overscan` and the
-        camera (`fov` or `intrinsics`) as in `render`."""
+        camera (`fov` or `intrinsics`, with `distortion` and `lens`) as in `render`."""
         eng = self.model.engine(state.v_all.dtype)  # the operand format the scene state was built in
         canvas, window, hw = self.view_geometry(resolution, overscan)
-        kind, cam = view_camera(c2w, fov, intrinsics)
+        kind, cam = view_camera(c2w, fov, intrinsics, distortion, lens, canvas, window)
         if self.cuda_graphs and not _eager and getattr(state, "static", False) and c2w.is_cuda and cam.is_cuda:
             # the graph reads the persistent state in place (no copy of the 300 MB of hoisted K / V)
             return self._graph_entry(("views", id(eng), id(state), kind, canvas, window, self.view_chunk) +
                                      self._sig((c2w, cam)), (c2w, cam),
                                      lambda a, k: self.render_views(state, a, resolution=hw, overscan=overscan,
-                                                                    _eager=True, **{kind: k}))
+                                                                    _eager=True, **camera_kwargs(kind, k)))
         B, V = c2w.shape[:2]
         if V == 0:  # a rank whose view slice is empty (fewer views than ranks)
             return torch.empty((B, 0, *hw, 3), dtype=torch.float32, device=self.device)
@@ -351,11 +351,14 @@ class RenderFormerRenderingPipeline:
         # every decoder pass writes its images straight into its slice of the result (no torch.cat afterwards); with
         # overscan its last conv stores only the window, so no canvas-sized image exists
         result = torch.empty((B, V, *hw, 3), dtype=torch.float32, device=self.device)
+        cam_kw = camera_kwargs(kind, cam)
+        fov = cam_kw.pop("fov", None)
 
         def job(b, v0):
             s = slice(v0, v0 + self.view_chunk)
             eng.render_views(state, b, c2w[b, s], None if fov is None else fov[b, s], canvas, out=result[b, s],
-                             window=window, intrinsics=None if intrinsics is None else intrinsics[b, s])
+                             window=window, **{k: t[b, s] if isinstance(t, torch.Tensor) else t
+                                               for k, t in cam_kw.items()})
         n_str = min(self.view_streams, len(jobs))
         if n_str <= 1:
             for b, v0 in jobs:
@@ -381,7 +384,8 @@ class RenderFormerRenderingPipeline:
 
     @torch.no_grad()
     def render(self, triangles, texture, mask, vn, c2w, fov=None, resolution=512,
-               torch_dtype: torch.dtype = torch.float16, overscan: bool = False, intrinsics=None):
+               torch_dtype: torch.dtype = torch.float16, overscan: bool = False, intrinsics=None, distortion=None,
+               lens: str = "opencv"):
         """triangles [B,N,3,3], texture [B,N,13,32,32], mask [B,N] bool, vn [B,N,3,3], c2w [B,V,4,4],
         fov [B,V,1] degrees or intrinsics [B,V,4] -> HDR [B,V,H,W,3] fp32.
 
@@ -407,6 +411,20 @@ class RenderFormerRenderingPipeline:
         `intrinsics` is given (config.view_camera).  Intrinsics on the host are checked (finite, fx, fy > 0);
         on the device they are used as they are, without a synchronising read-back.
 
+        `distortion` (with `intrinsics`) renders through a lens-distorted camera; `lens` names its model, as OpenCV
+        and COLMAP define them.  "opencv": [B,V,8] = (k1, k2, p1, p2, k3, k4, k5, k6), OpenCV's distCoeffs order and
+        COLMAP's FULL_OPENCV ([B,V,4] and [B,V,5] too: the missing coefficients are zero).  A pixel at (u, v) has the
+        distorted coordinates xd = (u - cx) / fx, yd = (v - cy) / fy, and with r2 = x^2 + y^2 and
+        g = (1 + k1 r2 + k2 r2^2 + k3 r2^3) / (1 + k4 r2 + k5 r2^2 + k6 r2^3) the lens maps (x, y) to
+        xd = x g + 2 p1 x y + p2 (r2 + 2 x^2), yd = y g + p1 (r2 + 2 y^2) + 2 p2 x y; the ray is normalize((x, -y, -1)).
+        "fisheye": [B,V,4] = (k1, k2, k3, k4) of OpenCV's fisheye model and COLMAP's OPENCV_FISHEYE: the ray at
+        angle theta from the axis lands at rd = |(xd, yd)| = theta (1 + k1 theta^2 + k2 theta^4 + k3 theta^6 +
+        k4 theta^8), so rays at 90 degrees and more are rendered too; all-zero coefficients are the equidistant fisheye.
+        The ray kernel inverts the lens per pixel by Newton's method.  Coefficients on the host are checked
+        (config.lens_check): the lens must invert on the whole canvas, overscan border included; on the device they
+        are used as they are.  `lens="opencv"` with all coefficients zero renders bit-identically to `intrinsics`
+        alone.  `scene_io.read_colmap_cameras` reads COLMAP cameras into these arguments.
+
         `texture` may also be [B,N,13]: per-triangle constants (what scene_processor/to_h5.py:37-66
         expands to the 32x32 texel grid with a fixed triangular mask).  The texture projection then
         uses texel-summed weights -- no 218 MB texel grid has to exist or be uploaded
@@ -418,14 +436,14 @@ class RenderFormerRenderingPipeline:
         softmax, norms and the residual stream are fp32 in every mode and the result is always fp32.
         Unlike the reference (:68) the caller's `texture` is not modified."""
         op = operand_dtype(torch_dtype)
-        self.view_geometry(resolution, overscan)  # size errors before any launch
-        kind, cam = view_camera(c2w, fov, intrinsics)
+        canvas, window, _ = self.view_geometry(resolution, overscan)  # size errors before any launch
+        kind, cam = view_camera(c2w, fov, intrinsics, distortion, lens, canvas, window)
         inputs = (triangles, texture, mask, vn, c2w, cam)
         if self.cuda_graphs and all(t.is_cuda for t in inputs):
             out = self._render_graphed(inputs, resolution, op, overscan, kind)
             return out if self.graph_static_outputs else out.clone()
         state = self.encode(triangles, texture, mask, vn, torch_dtype=op)
-        return self.render_views(state, c2w, fov, resolution, overscan, intrinsics)
+        return self.render_views(state, c2w, fov, resolution, overscan, intrinsics, distortion, lens)
 
     def _graph_entry(self, key, inputs, fn):
         """Capture `fn(*static_inputs)` once per key, replay it with `inputs` copied into the static
@@ -461,14 +479,15 @@ class RenderFormerRenderingPipeline:
 
     def _render_graphed(self, inputs, resolution, op: torch.dtype = torch.bfloat16, overscan: bool = False,
                         camera: str = "fov") -> torch.Tensor:
-        """`inputs` = (triangles, texture, mask, vn, c2w, camera tensor); `camera` names the last: "fov" or
-        "intrinsics" (a static input of the graph either way, and part of its key)."""
+        """`inputs` = (triangles, texture, mask, vn, c2w, camera tensor); `camera` names the last as
+        config.view_camera does: "fov", "intrinsics", "opencv" or "fisheye" (a static input of the graph either way,
+        and part of its key)."""
         eng = self.model.engine(op)
         canvas, window, _ = self.view_geometry(resolution, overscan)
 
         def run(tri, tex, mask, vn, c2w, cam):
             return self.render_views(eng.encode_scene(tri, tex, mask, vn), c2w, resolution=resolution,
-                                     overscan=overscan, _eager=True, **{camera: cam})
+                                     overscan=overscan, _eager=True, **camera_kwargs(camera, cam))
         return self._graph_entry(("render", id(eng), camera, canvas, window, self.view_chunk) + self._sig(inputs),
                                  inputs, run)
 
@@ -496,11 +515,13 @@ class RenderFormerRenderingPipeline:
 
     @torch.no_grad()
     def render_stream(self, scenes, resolution=512, torch_dtype: torch.dtype = torch.float16,
-                      ldr: Optional[str] = None, pad_to: Optional[int] = None, overscan: bool = False):
+                      ldr: Optional[str] = None, pad_to: Optional[int] = None, overscan: bool = False,
+                      lens: str = "opencv"):
         """Render a sequence of scenes given as HOST tensors (the batch_infer.py use case,
         batch_infer.py:103-143): generator over dicts with the keys of `render` ('triangles', 'texture',
-        'mask', 'vn', 'c2w', and 'fov' or 'intrinsics'), yielding one pinned-host fp32 HDR tensor [B,V,H,W,3] per
-        scene, in order.  `resolution` is an int or (H, W) and `overscan` as in `render`.
+        'mask', 'vn', 'c2w', and 'fov' or 'intrinsics', the latter optionally with 'distortion'), yielding one
+        pinned-host fp32 HDR tensor [B,V,H,W,3] per scene, in order.  `resolution` is an int or (H, W), and
+        `overscan` and `lens` (the model of every scene's 'distortion') as in `render`.
 
         The host->device copy of scene i+1 (218 MB of texture for 4096 triangles) runs on a copy
         stream while scene i is being rendered, and the device->host copy of image i overlaps scene
@@ -516,26 +537,27 @@ class RenderFormerRenderingPipeline:
         if dev.type != "cuda":
             raise L.RfbError("render_stream needs a CUDA device (there is no CPU fallback)")
         keys = ("triangles", "texture", "mask", "vn", "c2w")
+        canvas, window, _ = self.view_geometry(resolution, overscan)
         main = torch.cuda.current_stream(dev)
         copy = torch.cuda.Stream(dev)
         up = UploadRing(dev, copy)
 
         def upload(sc):
-            kind, _ = view_camera(sc["c2w"], sc.get("fov"), sc.get("intrinsics"))  # host checks before the copy
-            return up.put({k: sc[k] for k in keys + (kind,)}, pad_to=pad_to)
+            kind, cam = view_camera(sc["c2w"], sc.get("fov"), sc.get("intrinsics"), sc.get("distortion"), lens, canvas,
+                                    window)  # host checks before the copy
+            return (kind, *up.put({**{k: sc[k] for k in keys}, kind: cam}, pad_to=pad_to))
 
         it = iter(scenes)
         first = next(it, None)
         pending = upload(first) if first is not None else None
         ring, slot, prev = [None, None, None], 0, None
         while pending is not None:
-            d, ev, uslot = pending
+            kind, d, ev, uslot = pending
             nxt = next(it, None)
             pending = upload(nxt) if nxt is not None else None  # overlaps with this scene's kernels
             main.wait_event(ev)
-            img = self.render(d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], d.get("fov"),
-                              resolution=resolution, torch_dtype=torch_dtype, overscan=overscan,
-                              intrinsics=d.get("intrinsics"))
+            img = self.render(d["triangles"], d["texture"], d["mask"], d["vn"], d["c2w"], resolution=resolution,
+                              torch_dtype=torch_dtype, overscan=overscan, **camera_kwargs(kind, d[kind]))
             up.release(uslot, main)  # the staging slot may be overwritten once this render has consumed it
             if ldr is not None:
                 img = self.hdr_to_ldr(img, ldr)

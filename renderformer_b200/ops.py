@@ -302,6 +302,25 @@ def ray_tokens_intrinsics(intr, out, *, n_views, canvas_h, canvas_w, height, wid
     return out
 
 
+LENSES = {"opencv": 0, "fisheye": 1}
+
+
+def ray_tokens_lens(intr, dist, out, *, lens, n_views, canvas_h, canvas_w, height, width, top=0, left=0):
+    """Ray-bundle patch tokens f16 [V, (canvas_h/8)*(canvas_w/8), 192] of lens-distorted cameras: intrinsics fp32 [V, 4]
+    as `ray_tokens_intrinsics` and coefficients fp32 dist [V, 8] (lens "opencv") or [V, 4] (lens "fisheye")
+    (rfb_ray_tokens_lens)."""
+    if lens not in LENSES:
+        raise ValueError(f"lens must be one of {sorted(LENSES)}, got {lens!r}")
+    if dist.numel() != n_views * (8 if lens == "opencv" else 4):
+        raise ValueError(f"lens {lens!r} reads {8 if lens == 'opencv' else 4} coefficients per view: dist must have "
+                         f"{n_views} x that many values, got {list(dist.shape)}")
+    _need_cuda(intr, dist, out)
+    L.check(_timed("ray_tokens", 0.0, lambda: L.load().rfb_ray_tokens_lens(
+        intr.data_ptr(), dist.data_ptr(), LENSES[lens], out.data_ptr(), n_views, canvas_h, canvas_w, height, width, top,
+        left, _stream())), "rfb_ray_tokens_lens")
+    return out
+
+
 FITS = {"auto": 0, "horizontal": 1, "vertical": 2}
 
 

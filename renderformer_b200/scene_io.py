@@ -324,3 +324,83 @@ def load_scene_file(path: str) -> Dict[str, np.ndarray]:
     if ext == ".json":
         return load_scene(path)
     raise ValueError(f"{path}: unknown scene file type")
+
+
+# ------------------------------------------------------------------------------------------- COLMAP cameras
+# COLMAP camera model -> (lens, intrinsics from the parameters, distortion from the parameters).  The fisheye models
+# share one theta polynomial: SIMPLE_RADIAL_FISHEYE and RADIAL_FISHEYE are OPENCV_FISHEYE with k2.. or k3.. zero.
+_COLMAP_MODELS = {
+    "SIMPLE_PINHOLE": ("opencv", lambda p: (p[0], p[0], p[1], p[2]), None),
+    "PINHOLE": ("opencv", lambda p: p[:4], None),
+    "SIMPLE_RADIAL": ("opencv", lambda p: (p[0], p[0], p[1], p[2]), lambda p: (p[3], 0, 0, 0, 0, 0, 0, 0)),
+    "RADIAL": ("opencv", lambda p: (p[0], p[0], p[1], p[2]), lambda p: (p[3], p[4], 0, 0, 0, 0, 0, 0)),
+    "OPENCV": ("opencv", lambda p: p[:4], lambda p: (*p[4:8], 0, 0, 0, 0)),
+    "FULL_OPENCV": ("opencv", lambda p: p[:4], lambda p: p[4:12]),
+    "SIMPLE_RADIAL_FISHEYE": ("fisheye", lambda p: (p[0], p[0], p[1], p[2]), lambda p: (p[3], 0, 0, 0)),
+    "RADIAL_FISHEYE": ("fisheye", lambda p: (p[0], p[0], p[1], p[2]), lambda p: (p[3], p[4], 0, 0)),
+    "OPENCV_FISHEYE": ("fisheye", lambda p: p[:4], lambda p: p[4:8]),
+}
+_COLMAP_NPARAMS = {"SIMPLE_PINHOLE": 3, "PINHOLE": 4, "SIMPLE_RADIAL": 4, "RADIAL": 5, "OPENCV": 8, "FULL_OPENCV": 12,
+                   "SIMPLE_RADIAL_FISHEYE": 4, "RADIAL_FISHEYE": 5, "OPENCV_FISHEYE": 8}
+
+
+def _colmap_lines(path: str) -> List[str]:
+    with open(path) as f:
+        return [line.rstrip("\n") for line in f]
+
+
+def _quat_to_rot(q) -> np.ndarray:
+    """Rotation matrix [3,3] of a quaternion (w, x, y, z) (normalised first), COLMAP's convention."""
+    w, x, y, z = np.asarray(q, dtype=np.float64) / np.linalg.norm(q)
+    return np.array([[1 - 2 * (y * y + z * z), 2 * (x * y - w * z), 2 * (x * z + w * y)],
+                     [2 * (x * y + w * z), 1 - 2 * (x * x + z * z), 2 * (y * z - w * x)],
+                     [2 * (x * z - w * y), 2 * (y * z + w * x), 1 - 2 * (x * x + y * y)]])
+
+
+def read_colmap_cameras(sparse_dir: str) -> List[dict]:
+    """The cameras of a COLMAP reconstruction in the TEXT model format (`cameras.txt` and `images.txt` in
+    `sparse_dir`; `colmap model_converter --output_type TXT` writes them from the binary format).
+
+    Returns one record per image, in the order of images.txt: 'name', 'resolution' (height, width), 'intrinsics'
+    float64 [4] = (fx, fy, cx, cy), 'distortion' float64 [8] (lens 'opencv': k1, k2, p1, p2, k3, k4, k5, k6) or [4]
+    (lens 'fisheye': k1, k2, k3, k4) or None (the pinhole models), 'lens' ('opencv' for the pinhole models) and
+    'c2w' float64 [4,4] in this project's camera axes (x right, y up, looking down -z): inv([R(q) | t]) @
+    diag(1, -1, -1, 1) of COLMAP's world-to-camera pose.  These are `render`'s camera arguments as they are: COLMAP's
+    pixel centres are at j + 0.5 and its principal point is in pixels of the image, as `intrinsics` expects.
+    Models: SIMPLE_PINHOLE, PINHOLE (no distortion); SIMPLE_RADIAL, RADIAL, OPENCV, FULL_OPENCV (opencv);
+    SIMPLE_RADIAL_FISHEYE, RADIAL_FISHEYE, OPENCV_FISHEYE (fisheye).  Any other (FOV, the thin-prism models, ...)
+    raises NotImplementedError naming it."""
+    cams = {}
+    for line in _colmap_lines(os.path.join(sparse_dir, "cameras.txt")):
+        el = line.split()
+        if not el or el[0].startswith("#"):
+            continue
+        cam_id, model, width, height = int(el[0]), el[1], int(el[2]), int(el[3])
+        if model not in _COLMAP_MODELS:
+            raise NotImplementedError(f"COLMAP camera model {model} (camera {cam_id}) is not supported; supported: "
+                                      f"{', '.join(_COLMAP_MODELS)}")
+        p = [float(v) for v in el[4:]]
+        if len(p) != _COLMAP_NPARAMS[model]:
+            raise ValueError(f"COLMAP camera {cam_id}: model {model} has {_COLMAP_NPARAMS[model]} parameters, "
+                             f"got {len(p)}")
+        lens, intr, dist = _COLMAP_MODELS[model]
+        cams[cam_id] = dict(resolution=(height, width), intrinsics=np.array(intr(p), dtype=np.float64),
+                            distortion=None if dist is None else np.array(dist(p), dtype=np.float64), lens=lens)
+    out = []
+    lines = iter(_colmap_lines(os.path.join(sparse_dir, "images.txt")))
+    flip = np.diag([1.0, -1.0, -1.0, 1.0])  # COLMAP's camera axes (x right, y down, z forward) -> this project's
+    for line in lines:
+        el = line.split()
+        if not el or el[0].startswith("#"):
+            continue
+        next(lines, None)  # the image's POINTS2D line (possibly empty)
+        q, t = [float(v) for v in el[1:5]], np.array([float(v) for v in el[5:8]])
+        cam_id, name = int(el[8]), " ".join(el[9:])
+        if cam_id not in cams:
+            raise ValueError(f"COLMAP image {name}: camera {cam_id} is not in cameras.txt")
+        R = _quat_to_rot(q)
+        c2w = np.eye(4)
+        c2w[:3, :3], c2w[:3, 3] = R.T, -R.T @ t
+        out.append(dict(name=name, c2w=c2w @ flip, **{k: (v.copy() if isinstance(v, np.ndarray) else v)
+                                                      for k, v in cams[cam_id].items()}))
+    return out
